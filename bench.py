@@ -6,7 +6,10 @@ the whole default simulated trajectory (mandala0_mono, 140 camera frames, 10 IMU
 1390 x Filter.propagate + 139 x Filter.update) inside ONE persistent kernel launch.  One *filter-step*
 (the metric's unit) = one Filter.propagate on one filter.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--filters F] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--filters F] [--impl ours|reference] [--dump-outputs DIR]
+
+--dump-outputs DIR writes what the last timed pass computed (per-filter statistics, the reduced statistics vector, final
+state x and covariance P) as DIR/<name>.npy, so that two builds can be compared output for output on identical inputs.
 
 N > 1 is launched by torchrun (one rank per GPU); every rank runs its own shard of the Monte-Carlo batch
 (weak scaling: --filters is per GPU; Philox noise is keyed by the GLOBAL filter id) and the only
@@ -234,6 +237,35 @@ def ncu_traffic():
             except Exception:
                 pass
     return None
+
+
+DUMP_BYTES = 64 << 20
+DUMP_SEED = 20240
+
+
+def dump_rows(n, bytes_per_row, budget):
+    """Rows of the per-filter outputs that --dump-outputs writes: all of them if they fit the budget, else a fixed seeded
+    sample (sorted), the same from run to run for the same n."""
+    cap = budget // bytes_per_row
+    if n <= cap:
+        return None
+    return np.sort(np.random.default_rng(DUMP_SEED).choice(n, size=cap, replace=False))
+
+
+def last_pass_outputs(bf, st, sm, budget):
+    """The arrays a caller of the timed pass receives: per-filter statistics [N,16] and the reduced vector [16] from run(),
+    the final state x [N,26] and covariance P [N,24,24] from get_state(); a seeded row sample above `budget` bytes."""
+    import torch
+
+    x, P, _, _, _ = bf.get_state(device=True)
+    rows = dump_rows(bf.n, (st.shape[1] + x.shape[1] + P.shape[1] * P.shape[2]) * 8, budget - sm.numel() * 8)
+    per = {"stats": st, "x": x, "P": P}
+    if rows is not None:
+        idx = torch.from_numpy(rows).to(st.device)
+        per = {k: v.index_select(0, idx) for k, v in per.items()}
+    out = {k: v.cpu().numpy() for k, v in per.items()}
+    out["stats_sum"] = sm.cpu().numpy()
+    return out
 
 
 def _guard(launch, dev):
@@ -539,6 +571,8 @@ def run_ours(a):
     # keep the hardware busy for the clock sampler a little longer on very short runs
     clocks = sampler.stop() if rank == 0 else None
     stats_sum = sm.cpu().numpy()
+    # read out before the end-to-end passes below overwrite the filters' state
+    dumped = last_pass_outputs(bf, st, sm, DUMP_BYTES // world) if a.dump_outputs else None
 
     # ---- end-to-end through the C ABI with HOST buffers (pinned), copies inside the timed region ----
     def pinned(x, dtype=np.float64):
@@ -672,6 +706,11 @@ def run_ours(a):
             line["configs"] = secondary
             line["configs_clocks"] = clocks2
         print(json.dumps(line), flush=True)
+    if dumped is not None:
+        os.makedirs(a.dump_outputs, exist_ok=True)
+        suffix = f"_rank{rank}" if world > 1 else ""
+        for k, v in dumped.items():
+            np.save(os.path.join(a.dump_outputs, f"{k}{suffix}.npy"), v)
     bf.close()
     if dist is not None:
         dist.barrier()
@@ -689,7 +728,13 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-configs", action="store_true", help="skip the secondary workloads (BASELINE configs 3 / 4 / 5, calibration)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed pass as DIR/<name>.npy (float64; "
+                    "a seeded sample of the filters above 64 MiB in all); with N > 1 every rank writes <name>_rank<r>.npy")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if a.impl == "reference":
         return run_reference_arm(a)
     return run_ours(a)

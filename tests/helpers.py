@@ -9,6 +9,8 @@ floor of 1e-7 * sqrt(R_i R_j): when the prior is >> R the reference's own FP64
 arithmetic only determines those entries to ~1e-8 (it computes 1 - K with
 K = 1 - O(1e-12); see tests/test_conditioning.py).
 """
+import os
+
 import numpy as np
 
 from oracle.eskf_oracle import (
@@ -21,6 +23,20 @@ from oracle.eskf_oracle import (
     camera_gen_rotated,
     quat_normalise,
 )
+
+GOLDEN_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+LEGACY_COLS = [0, 1, 2, 3, 7, 8, 9, 10, 11, 12, 13]  # all but the velocity columns (an older velocity definition)
+
+
+def legacy_imu_ref(kp):
+    """The reference's legacy imu_ref_mandala0_mono_upd_Kp<kp>_Km1.000.txt [rows, 14], decoded bit-exactly from
+    tests/golden/imu_ref_legacy.npz (see make_golden.py); the velocity columns 4:7 are not stored and read as NaN."""
+    with np.load(os.path.join(GOLDEN_DIR, "imu_ref_legacy.npz")) as z:
+        n = np.cumsum(z[f"Kp{kp}"], axis=0)
+    out = np.full((len(n), 14), np.nan)
+    out[:, LEGACY_COLS] = n / 1e9
+    return out
+
 
 GROUPS = {"p": (0, 3), "v": (3, 6), "q": (6, 10), "dofs": (10, 16), "notch": (16, 19), "pc": (19, 22), "qc": (22, 26)}
 HSET = [18, 19, 20, 21, 22, 23, 15]

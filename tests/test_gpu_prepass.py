@@ -4,7 +4,7 @@ device-resident streams that never touched the host."""
 import numpy as np
 import pytest
 
-from tests.helpers import cov_err, mandala_scenario, model_kwargs, state_err
+from tests.helpers import cov_err, legacy_imu_ref, mandala_scenario, model_kwargs, state_err
 
 pytestmark = pytest.mark.gpu
 
@@ -106,7 +106,7 @@ def test_gpu_prepass_reproduces_the_legacy_imu_ref_files(golden, kp, ifv, nfr):
     tests/test_oracle_golden.py (their velocity columns come from an older velocity definition)."""
     _, dev = _both(golden, "traj_mandala0_mono", nfr, ifv, euler_mode="zyx_legacy")
     rows = dev.imu_ref_rows.cpu().numpy()[: dev.n_steps]
-    ref = golden[f"imu_ref_legacy_Kp{kp}"]
+    ref = legacy_imu_ref(kp)
     assert rows.shape == ref.shape
     assert np.all(dev.n_prop.cpu().numpy() == ifv)
     cols = [0, 1, 2, 3, 7, 8, 9, 10, 11, 12, 13]

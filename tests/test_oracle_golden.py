@@ -10,6 +10,7 @@ from oracle.eskf_oracle import (
     camera_from_arrays,
     run_reference_flow,
 )
+from tests.helpers import legacy_imu_ref
 
 # the golden files are written with 9 decimals (tools/files.py:68-82)
 ROUND_FLOOR = 5.0e-10 + 1e-15
@@ -82,7 +83,7 @@ def test_legacy_imu_ref_pins_interpolation_path(golden, kp, ifv, nfr):
     cam = camera_from_arrays(tr[:, 0], tr[:, 1:4], tr[:, 4:8], cfg)
     out = build_streams(cam, cfg, Probe(cfg.length, cfg.angle))
     rows, n_prop = out[-1], out[4]
-    ref = golden[f"imu_ref_legacy_Kp{kp}"]
+    ref = legacy_imu_ref(kp)
     assert rows.shape == ref.shape
     assert np.all(n_prop == ifv)
     cols = [0, 1, 2, 3, 7, 8, 9, 10, 11, 12, 13]

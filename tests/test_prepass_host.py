@@ -6,7 +6,7 @@ import numpy as np
 import pytest
 
 from oracle.eskf_oracle import OracleConfig
-from tests.helpers import Scenario
+from tests.helpers import Scenario, legacy_imu_ref
 
 ROUND_FLOOR = 5.0e-10  # the artefacts are printed with 9 decimals (files.py:68-82)
 
@@ -53,7 +53,7 @@ def test_product_prepass_reproduces_the_legacy_imu_ref_files(golden, kp, ifv, nf
 
     a = golden["traj_mandala0_mono"][:nfr]
     s = build_streams(Camera(a[:, 0], a[:, 1:4], a[:, 4:8], scale=10.0, euler_mode="zyx_legacy"), ifv, 50.0, np.deg2rad(30.0))
-    ref = golden[f"imu_ref_legacy_Kp{kp}"]
+    ref = legacy_imu_ref(kp)
     assert s.imu_ref_rows.shape == ref.shape and np.all(s.n_prop == ifv)
     cols = [0, 1, 2, 3, 7, 8, 9, 10, 11, 12, 13]  # (velocity columns: an older velocity definition, tests/test_oracle_golden.py)
     assert np.abs(s.imu_ref_rows[:, cols] - ref[:, cols]).max() <= ROUND_FLOOR
