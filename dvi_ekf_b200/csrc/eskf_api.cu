@@ -424,7 +424,7 @@ static int pick_fpc(const eskf_t* h, int64_t fpt, bool multi_traj) {
   for (int i = 0; i < ns; ++i) {  // descending
     const int c = shapes[i];
     if (!fits(c)) continue;
-    const int64_t ctas = (multi_traj && k3) ? ((h->N + fpt - 1) / fpt) * ((fpt + c - 1) / c) : (h->N + c - 1) / c;
+    const int64_t ctas = (multi_traj && k3) ? stacked_grid(h->N, fpt, c) : (h->N + c - 1) / c;
     const int64_t waves = (ctas + h->sm_count - 1) / h->sm_count;
     if (best == 0 || waves < best_waves) {
       best = c;
@@ -747,6 +747,8 @@ int eskf_run(eskf_t* h, const eskf_streams_t* sp, double* stats_out, double* sta
     } else {
       if ((rc = stage_reserve(h, 8, tb))) return rc;
       dtrace = (double*)h->stage[8];
+      // rows the kernels do not write (steps a trajectory does not execute) keep the caller's content, as in place
+      CK(cudaMemcpyAsync(dtrace, sp->trace_x, tb, cudaMemcpyHostToDevice, h->stream));
     }
   }
   double* dsum = nullptr;

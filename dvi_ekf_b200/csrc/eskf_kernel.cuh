@@ -69,7 +69,7 @@ struct KArgs {
   const double* imu_pf;   // [T][N][6]  noisy IMU samples per filter, or nullptr
   const double* meas_pf;  // [E][N][8]  noisy camera measurement (pos 3, quat 4, notch) per filter, or nullptr
   double* snap;           // [E][N][14] v(3) q(4) p_cam(3) q_cam(4) after every update, or nullptr
-  double* fx_dump;        // [N][FX3_SIZE] Jacobian record of the LAST IMU step of the launch (eskf_get_jacobians), or nullptr
+  double* fx_dump;        // [N][FX3_SIZE] Jacobian record of the filter's LAST executed IMU step of the launch (eskf_get_jacobians), or nullptr
 };
 
 // one FilterTraj row's worth of nominal state in the layout of x (include/eskf.h)

@@ -295,6 +295,15 @@ __device__ __forceinline__ int epoch_steps3(const KArgs& a, const Ctx3& c, int64
   return (int)(n < 0 ? 0 : (n > left ? left : n));
 }
 
+// the last IMU step the CTA's trajectory executes in this launch (-1: none), where export mode files the Jacobian record:
+// the epochs' steps as epoch_steps3 counts them, which may add up to less than n_steps (stacked trajectories share the
+// stream length, each has its own n_prop)
+__device__ __forceinline__ int64_t last_step3(const KArgs& a, const Ctx3& c) {
+  int64_t k = 0;
+  for (int64_t e = 0; e < a.E; ++e) k += epoch_steps3(a, c, e, k);
+  return k - 1;
+}
+
 // ---------------------------------------------------------------------------------------------
 // cooperative, coalesced tile store (all threads of the CTA)
 template <int F, int NTHR>
@@ -414,6 +423,7 @@ __device__ __forceinline__ void role3_imu(const KArgs& a, const Ctx3& c, int lan
   __syncthreads();  // prologue
   PT_DECL();
   JIT_DECL();
+  const int64_t k_jac = EX ? last_step3(a, c) : -1;  // (export mode: the step whose Jacobian record is filed)
   int64_t k = 0;
   for (int64_t e = 0; e < a.E; ++e) {
     const int n = epoch_steps3(a, c, e, k);
@@ -451,7 +461,7 @@ __device__ __forceinline__ void role3_imu(const KArgs& a, const Ctx3& c, int lan
 #pragma unroll
           for (int j = FX3_AB / 2; j < FX3_MAIN / 2; ++j) dst[j * F] = d2{fx[2 * j], fx[2 * j + 1]};
 #if ESKF_OPT_JACDUMP
-          if (EX && a.fx_dump && kk == a.T - 1) {  // Filter.Fx / Filter.Fi read-out: the record of the last step of the launch
+          if (EX && a.fx_dump && kk == k_jac) {  // Filter.Fx / Filter.Fi read-out: the record of the last step of the launch
             double* fd = a.fx_dump + (c.f0 + lane) * FX3_SIZE;
 #pragma unroll
             for (int j = FX3_AB; j < FX3_MAIN; ++j) fd[j] = fx[j];
@@ -602,6 +612,7 @@ __device__ __forceinline__ void role3_cam(const KArgs& a, const Ctx3& c, int lan
   PT_DECL();
   JIT_DECL();
   const bool h1s = h1_by_stager<EX>(a);  // rows 18:21 of Fx are the STAGER's work in this launch (see role3_stage)
+  const int64_t k_jac = EX ? last_step3(a, c) : -1;
   int64_t k = 0;
   for (int64_t e = 0; e < a.E; ++e) {
     const int n = epoch_steps3(a, c, e, k);
@@ -677,7 +688,7 @@ __device__ __forceinline__ void role3_cam(const KArgs& a, const Ctx3& c, int lan
 #pragma unroll
         for (int j = FX3_H1 / 2; j < FX3_AB / 2; ++j) dst[j * F] = d2{fx[2 * j], fx[2 * j + 1]};
 #if ESKF_OPT_JACDUMP
-        if (EX && a.fx_dump && kk == a.T - 1) {
+        if (EX && a.fx_dump && kk == k_jac) {
           double* fd = a.fx_dump + (c.f0 + lane) * FX3_SIZE;
 #pragma unroll
           for (int j = FX3_H1; j < FX3_AB; ++j) fd[j] = fx[j];
@@ -823,6 +834,7 @@ __device__ __forceinline__ void role3_jac(const KArgs& a, const Ctx3& c, int lan
   __syncthreads();  // prologue
   PT_DECL();
   JIT_DECL();
+  const int64_t k_jac = EX ? last_step3(a, c) : -1;
   int64_t k = 0;
   for (int64_t e = 0; e < a.E; ++e) {
     const int n = epoch_steps3(a, c, e, k);
@@ -908,7 +920,7 @@ __device__ __forceinline__ void role3_jac(const KArgs& a, const Ctx3& c, int lan
           for (int j = FX3_NPAIR_MAIN; j < FX3_NPAIR; ++j) dst[j * F] = d2{fx[2 * j], fx[2 * j + 1]};
         }
 #if ESKF_OPT_JACDUMP
-        if (EX && a.fx_dump && kk == a.T - 1) {  // (rows 18:24 of Fi are part of the read-out whether or not Q uses them)
+        if (EX && a.fx_dump && kk == k_jac) {  // (rows 18:24 of Fi are part of the read-out whether or not Q uses them)
           double* fd = a.fx_dump + (c.f0 + lane) * FX3_SIZE;
           if (!imu_q) {
             double Ro[9];
@@ -1660,14 +1672,10 @@ __global__ void __launch_bounds__(128 + 8 * F, 1) eskf_kernel3(const __grid_cons
   Ctx3 c;
   c.smem = smem;
   if constexpr (MT) {
-    // stacked trajectories: a CTA follows ONE trajectory's epoch structure, so every trajectory's filters_per_traj filters
-    // are cut into ceil(fpt / F) CTAs of their own (the last one ragged) -- fpt need not be a multiple of the CTA shape
-    const int64_t fpt = a.filters_per_traj, cpt = (fpt + F - 1) / F;
-    const int64_t tl = blockIdx.x / cpt, ch = blockIdx.x - tl * cpt;
-    c.f0 = tl * fpt + ch * F;
-    int64_t left = fpt - ch * F;
-    if (a.N - c.f0 < left) left = a.N - c.f0;
-    c.nf = (int)(left < F ? left : F);
+    // stacked trajectories: a CTA follows ONE trajectory's epoch structure (stacked_cta, eskf_math.cuh; the grid is
+    // stacked_grid) -- fpt need not be a multiple of the CTA shape
+    int64_t tl;
+    stacked_cta(blockIdx.x, a.N, a.filters_per_traj, F, c.f0, c.nf, tl);
   } else {
     c.f0 = (int64_t)blockIdx.x * F;
     c.nf = (int)((a.N - c.f0) < F ? (a.N - c.f0) : F);

@@ -40,10 +40,8 @@ cudaError_t launch_eskf_kernel3<ESKF_F>(const KArgs& a, cudaStream_t stream) {
                           : eskf_kernel3<F, ESKF_REG_S, ESKF_REG_C, 3>;
   cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return e;
-  // (stacked trajectories: ceil(fpt / F) CTAs per trajectory, see eskf_kernel3)
-  const int64_t cpt = (a.filters_per_traj + F - 1) / F;
-  const unsigned grid = a.n_traj > 1 ? (unsigned)(((a.N + a.filters_per_traj - 1) / a.filters_per_traj) * cpt)
-                                     : (unsigned)((a.N + F - 1) / F);
+  // (stacked trajectories: ceil(fpt / F) CTAs per trajectory, fewer for a partially covered last one: stacked_grid)
+  const unsigned grid = a.n_traj > 1 ? (unsigned)stacked_grid(a.N, a.filters_per_traj, F) : (unsigned)((a.N + F - 1) / F);
   kern<<<grid, 128 + 8 * F, smem, stream>>>(a);
   return cudaGetLastError();
 }

@@ -1205,4 +1205,24 @@ struct alignas(16) d2 {
   double x, y;
 };
 
+// ---- CTA mapping of stacked trajectories (eskf_kernel3, n_traj > 1) --------------------------------------------------
+// A CTA follows ONE trajectory's epoch structure, so every trajectory's fpt filters are cut into ceil(fpt / F) CTAs of
+// their own, the last one ragged.  A batch of N filters (a shard starts at a trajectory boundary) holds N / fpt whole
+// trajectories and, when N % fpt != 0, a partially covered last one: that one gets only the ceil((N % fpt) / F) CTAs that
+// hold filters, and they come last, so the decode below is the same for every block and no CTA is empty.
+ESKF_HD int64_t stacked_grid(int64_t N, int64_t fpt, int F) {
+  const int64_t cpt = (fpt + F - 1) / F;
+  return (N / fpt) * cpt + ((N % fpt) + F - 1) / F;
+}
+// block -> first filter f0, number of filters nf (1..F) and trajectory tl, counted from the batch's first trajectory
+ESKF_HD void stacked_cta(int64_t block, int64_t N, int64_t fpt, int F, int64_t& f0, int& nf, int64_t& tl) {
+  const int64_t cpt = (fpt + F - 1) / F;
+  tl = block / cpt;
+  const int64_t ch = block - tl * cpt;
+  f0 = tl * fpt + ch * F;
+  int64_t left = fpt - ch * F;
+  if (N - f0 < left) left = N - f0;
+  nf = (int)(left < F ? left : F);
+}
+
 }  // namespace eskf

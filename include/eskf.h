@@ -129,7 +129,8 @@ int eskf_run(eskf_t* h, const eskf_streams_t* streams, double* stats_out, double
 int eskf_get_state(eskf_t* h, double* x, double* P, double* u_old, double* R_old, int32_t* status, int mem);
 
 /* Filter.Fx / Filter.Fi (Filter.py:249-268; the reference sets both on every propagate): after eskf_keep_jacobians(h, 1)
- * the kernels file the Jacobian record of the LAST IMU step of every eskf_propagate / eskf_run launch (720 B per filter),
+ * the kernels file the Jacobian record of the LAST IMU step of every eskf_propagate / eskf_run launch (720 B per filter;
+ * with stacked trajectories, the last step of the filter's own trajectory: sum(n_prop) may be less than n_steps),
  * and eskf_get_jacobians expands it into the dense matrices the reference holds: Fx [N,24,24], Fi [N,24,13]; either
  * pointer may be NULL.  Default kernel only. */
 int eskf_keep_jacobians(eskf_t* h, int on);

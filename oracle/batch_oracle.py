@@ -195,6 +195,7 @@ class BatchOracle:
         Fi[:, 18:21, 3:6] = dt * Ro @ _skew(p_p)
         Fi[:, 21:24, 3:6] = -dt * np.swapaxes(R_p, 1, 2)
         self.P = Fx @ self.P @ np.swapaxes(Fx, 1, 2) + (Fi * self.Qd[:, None, :]) @ np.swapaxes(Fi, 1, 2)
+        self.Fx, self.Fi = Fx, Fi  # Filter.Fx / Filter.Fi of the last step
         self.om_old, self.acc_old = om.copy(), acc.copy()
         self.R_old = _q2R(self.x[:, 6:10])
 

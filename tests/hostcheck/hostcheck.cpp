@@ -178,4 +178,24 @@ int hc_update3(const double* model, double* x, double* P, const double* u, const
   return 1;
 }
 
+// CTA mapping of stacked trajectories (stacked_grid / stacked_cta, what eskf_launch3.cu and eskf_kernel3 run) for every
+// batch size N = 1 .. n_traj * fpt - filter_id0 of one geometry: one row {N, grid, block, f0, nf, traj, tl} per block, traj =
+// the trajectory the kernel derives from the CTA's first global filter id, tl = the decoded one counted from the batch's
+// first trajectory.  Returns the number of rows (-1: cap too small).
+int64_t hc_stacked_sweep(int F, int64_t fpt, int64_t n_traj, int64_t filter_id0, int64_t* rows, int64_t cap) {
+  int64_t r = 0;
+  for (int64_t N = 1; filter_id0 + N <= n_traj * fpt; ++N) {
+    const int64_t grid = stacked_grid(N, fpt, F);
+    for (int64_t b = 0; b < grid; ++b) {
+      if (r >= cap) return -1;
+      int64_t f0, tl;
+      int nf;
+      stacked_cta(b, N, fpt, F, f0, nf, tl);
+      int64_t* o = rows + 7 * r++;
+      o[0] = N, o[1] = grid, o[2] = b, o[3] = f0, o[4] = nf, o[5] = (filter_id0 + f0) / fpt, o[6] = tl;
+    }
+  }
+  return r;
+}
+
 }  // extern "C"

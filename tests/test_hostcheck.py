@@ -239,6 +239,47 @@ def test_lockstep_random_tunings(hc, golden, fn, ufn):
     assert wus < 1e-11 and wuP < 1e-11, (wus, wuP)
 
 
+def test_stacked_cta_mapping_covers_every_filter_once(hc):
+    """The CTA mapping of stacked trajectories (stacked_grid / stacked_cta, eskf_math.cuh), exhaustively: every CTA shape,
+    filters_per_traj 1..70, 1..4 trajectories, shards starting at trajectory 0, 1 or 2 and every batch size the streams
+    cover.  Every filter belongs to exactly one CTA, every CTA holds 1..F existing filters of ONE trajectory, the trajectory
+    the kernel derives from the CTA's first global id exists, and the grid launches no CTA without filters (when N is not a
+    multiple of filters_per_traj, ceil(N / fpt) * ceil(fpt / F) CTAs would read parameter rows past the batch)."""
+    fn = hc.hc_stacked_sweep
+    i64 = ctypes.c_int64
+    fn.argtypes = [ctypes.c_int, i64, i64, i64, ctypes.POINTER(i64), i64]
+    fn.restype = i64
+    geometries = 0
+    for F in (28, 16, 8, 4):
+        for fpt in range(1, 71):
+            cpt = -(-fpt // F)
+            for n_traj in range(1, 5):
+                for id0 in (0, fpt, 2 * fpt):
+                    if id0 >= n_traj * fpt:
+                        continue
+                    cap = (n_traj * fpt - id0) * (n_traj * cpt + 1)
+                    buf = np.empty((cap, 7), dtype=np.int64)
+                    r = fn(F, fpt, n_traj, id0, buf.ctypes.data_as(ctypes.POINTER(i64)), cap)
+                    assert r > 0
+                    N, grid, blk, f0, nf, traj, tl = buf[:r].T
+                    where = f"F={F} fpt={fpt} n_traj={n_traj} filter_id0={id0}"
+                    bad = (nf < 1) | (nf > F) | (f0 < 0) | (f0 + nf > N)
+                    assert not bad.any(), (where, "empty / oversized / out-of-range CTA", buf[:r][bad][:3])
+                    bad = ((id0 + f0) // fpt != (id0 + f0 + nf - 1) // fpt) | (traj >= n_traj) | (traj != id0 // fpt + tl)
+                    assert not bad.any(), (where, "CTA straddles trajectories / no such trajectory", buf[:r][bad][:3])
+                    # exactly-once coverage: per batch size, the CTAs sorted by first filter tile 0..N-1 without gap or overlap
+                    o = np.lexsort((f0, N))
+                    N, f0, nf, blk, grid = N[o], f0[o], nf[o], blk[o], grid[o]
+                    first = np.r_[True, N[1:] != N[:-1]]
+                    last = np.r_[N[1:] != N[:-1], True]
+                    assert (f0[first] == 0).all() and (f0[last] + nf[last] == N[last]).all(), where
+                    assert (f0[1:][~first[1:]] == (f0 + nf)[:-1][~first[1:]]).all(), where
+                    counts = np.diff(np.r_[np.flatnonzero(first), len(N)])
+                    assert (counts == grid[first]).all(), where  # the grid is the number of CTAs that hold filters
+                    geometries += 1
+    assert geometries == 4 * 70 * 9
+
+
 def test_streaming_pass2_is_bit_identical(hc, golden):
     """fx3_apply_stream (pass 2 fused with the transposed reload, eskf_cov3.cuh) performs the same operations in the same
     order per accumulator as the reload followed by fx3_apply_inplace: identical bits on random tiles and records."""
