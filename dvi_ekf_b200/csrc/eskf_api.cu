@@ -277,6 +277,84 @@ __global__ void stats_final_kernel(const double* __restrict__ partial, int64_t n
   out[threadIdx.x] = a;
 }
 
+// ---- filter consistency (eskf_keep_consistency): post-pass over the records the export instantiation filed ------------
+// cons_eval_kernel, one thread per (epoch, filter): NIS as filed, NEES of the estimated DOFs from the posterior DOFs and DOF
+// block (nees_dofs, eskf_math.cuh); NaN for an update that was not applied and for any non-finite value.  Writes the
+// filter-major outputs [N, E] and both values back into the record (CONS_NIS, CONS_NEES) for the epoch reduction.
+struct ConsArgs {
+  int64_t N, E;
+  double gt[6];
+  int frozen_mask;
+};
+__global__ void cons_eval_kernel(double* __restrict__ rec, double* __restrict__ nis, double* __restrict__ nees, const ConsArgs p) {
+  const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (idx >= p.E * p.N) return;
+  const int64_t e = idx / p.N, f = idx - e * p.N;
+  double* r = rec + e * CONS_SIZE * p.N + f;  // element j at r[j N]
+  const bool applied = r[CONS_NEES * p.N] != 0.0;
+  double eps[6], B[36];
+#pragma unroll
+  for (int i = 0; i < 6; ++i) eps[i] = r[(CONS_DOFS + i) * p.N] - p.gt[i];
+#pragma unroll
+  for (int i = 0; i < 36; ++i) B[i] = r[(CONS_B + i) * p.N];
+  double vn = r[CONS_NIS * p.N];
+  double ve = nees_dofs(B, eps, p.frozen_mask);
+  if (!applied || !isfinite(vn)) vn = NAN;
+  if (!applied || !isfinite(ve)) ve = NAN;
+  nis[f * p.E + e] = vn;
+  nees[f * p.E + e] = ve;
+  r[CONS_NIS * p.N] = vn;
+  r[CONS_NEES * p.N] = ve;
+}
+
+// epoch_sum [E][ESKF_NCONS], deterministically like stats_sum: block b of epoch e sums the finite values of filters
+// b RED_ROWS .. (b + 1) RED_ROWS - 1 through a fixed tree, cons_final_kernel adds the blocks of an epoch in order.
+// [0] finite NIS, [1] sum, [2] sum of squares, [3..5] the same for the NEES, [6] filters whose NIS or (d > 0) NEES is NaN.
+__global__ void cons_partial_kernel(const double* __restrict__ rec, int64_t N, int64_t nblk, int with_nees,
+                                    double* __restrict__ partial) {
+  __shared__ double sh[256][7];
+  const int64_t e = blockIdx.x / nblk, b = blockIdx.x - e * nblk;
+  const double* vn = rec + e * CONS_SIZE * N + CONS_NIS * N;
+  const double* ve = rec + e * CONS_SIZE * N + CONS_NEES * N;
+  double acc[7];
+#pragma unroll
+  for (int i = 0; i < 7; ++i) acc[i] = 0.0;
+  for (int64_t r = b * RED_ROWS + threadIdx.x; r < (b + 1) * RED_ROWS && r < N; r += 256) {
+    const double a = vn[r], c = ve[r];
+    const bool fa = isfinite(a), fc = isfinite(c);
+    if (fa) {
+      acc[0] += 1.0;
+      acc[1] += a;
+      acc[2] += a * a;
+    }
+    if (fc) {
+      acc[3] += 1.0;
+      acc[4] += c;
+      acc[5] += c * c;
+    }
+    if (!fa || (with_nees && !fc)) acc[6] += 1.0;
+  }
+#pragma unroll
+  for (int i = 0; i < 7; ++i) sh[threadIdx.x][i] = acc[i];
+  __syncthreads();
+  for (int o = 128; o > 0; o >>= 1) {
+    if ((int)threadIdx.x < o) {
+#pragma unroll
+      for (int i = 0; i < 7; ++i) sh[threadIdx.x][i] += sh[threadIdx.x + o][i];
+    }
+    __syncthreads();
+  }
+  if (threadIdx.x < ESKF_NCONS) partial[blockIdx.x * ESKF_NCONS + threadIdx.x] = threadIdx.x < 7 ? sh[0][threadIdx.x] : 0.0;
+}
+__global__ void cons_final_kernel(const double* __restrict__ partial, int64_t nblk, int64_t E, double* __restrict__ out) {
+  const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (idx >= E * ESKF_NCONS) return;
+  const int64_t e = idx / ESKF_NCONS, i = idx - e * ESKF_NCONS;
+  double a = 0.0;
+  for (int64_t b = 0; b < nblk; ++b) a += partial[(e * nblk + b) * ESKF_NCONS + i];
+  out[idx] = a;
+}
+
 // Filter.Fx (24 x 24) and Filter.Fi (24 x 13) as the reference assembles them (Filter.py:249-342), from the fx3 record the
 // producer roles filed for the last IMU step of a launch (KArgs::fx_dump): the dense matrices the register-tile algebra of
 // eskf_cov3.cuh applies implicitly.
@@ -354,6 +432,12 @@ struct eskf_handle {
   int sm_count = 148;
   double* fxrec = nullptr;  // [N][FX3_SIZE] Jacobian record of the last step (eskf_keep_jacobians), or nullptr
   size_t pp_budget = 0;  // bytes the pre- / post-pass buffers of one eskf_run may take (0: everything inside the kernel)
+  // filter consistency (eskf_keep_consistency): the records of one run [E][CONS_SIZE][N] and the results of the last run,
+  // one buffer: nis [N][E], nees [N][E], epoch_sum [E][ESKF_NCONS], the partial sums of the reduction
+  bool cons_on = false;
+  int64_t cons_E = -1;  // epochs of the last run that filed them (-1: none since eskf_keep_consistency)
+  double *cons_rec = nullptr, *cons_out = nullptr;
+  size_t cons_rec_sz = 0, cons_out_sz = 0;
 };
 
 #define CK(call)                                                  \
@@ -387,6 +471,38 @@ static int stage_in(eskf_t* h, int slot, const void* src, size_t bytes, int mem,
   if (rc) return rc;
   CK(cudaMemcpyAsync(h->stage[slot], src, bytes, cudaMemcpyHostToDevice, h->stream));
   *out = h->stage[slot];
+  return ESKF_OK;
+}
+
+// the buffers of the consistency records and results of a run over E epochs.  Both are allocated before an old one is
+// released, so that a run that does not fit (ESKF_ENOMEM) leaves the results of the last run readable.
+static int64_t cons_nblk(const eskf_t* h) { return (h->N + RED_ROWS - 1) / RED_ROWS; }
+static int cons_reserve(eskf_t* h, int64_t E) {
+  const size_t n = (size_t)h->N, e = (size_t)E;
+  const size_t rb = e * CONS_SIZE * n * sizeof(double);
+  const size_t ob = (2 * n * e + e * ESKF_NCONS + (size_t)cons_nblk(h) * e * ESKF_NCONS) * sizeof(double);
+  void *nr = nullptr, *no = nullptr;
+  cudaError_t err = cudaSuccess;
+  if (rb > h->cons_rec_sz) err = cudaMalloc(&nr, rb);
+  if (err == cudaSuccess && ob > h->cons_out_sz) err = cudaMalloc(&no, ob);
+  if (err != cudaSuccess) {
+    cudaGetLastError();  // (an allocation failure is not sticky: clear it for the launches of later calls)
+    cudaFree(nr);
+    g_err = "eskf_run: the consistency records of " + std::to_string((long long)h->N) + " filters x " +
+            std::to_string((long long)E) + " epochs (" + std::to_string((unsigned long long)(rb + ob)) +
+            " bytes) do not fit in device memory: " + cudaGetErrorString(err);
+    return err == cudaErrorMemoryAllocation ? ESKF_ENOMEM : ESKF_ECUDA;
+  }
+  if (nr) {
+    CK(cudaFree(h->cons_rec));
+    h->cons_rec = (double*)nr;
+    h->cons_rec_sz = rb;
+  }
+  if (no) {
+    CK(cudaFree(h->cons_out));
+    h->cons_out = (double*)no;
+    h->cons_out_sz = ob;
+  }
   return ESKF_OK;
 }
 
@@ -545,6 +661,8 @@ int eskf_destroy(eskf_t* h) {
   cudaFree(h->status);
   cudaFree(h->stats_sum_dev);
   cudaFree(h->fxrec);
+  cudaFree(h->cons_rec);
+  cudaFree(h->cons_out);
   for (int i = 0; i < N_STAGE; ++i)
     if (h->stage[i]) cudaFree(h->stage[i]);
   delete h;
@@ -720,8 +838,16 @@ int eskf_run(eskf_t* h, const eskf_streams_t* sp, double* stats_out, double* sta
       }
     }
   }
-  const void *ddt, *doa, *dnp, *dcam, *dno, *dcr, *dir;
   int rc;
+  if (h->cons_on) {
+    if (kernel_of(h) != 3) {
+      g_err = "eskf_run: filter consistency needs the default kernel (eskf_set_variant(h, 1) selects the first one)";
+      return ESKF_EINVAL;
+    }
+    if ((rc = cons_reserve(h, E))) return rc;
+    h->cons_E = -1;  // (valid again once this run has filed its records)
+  }
+  const void *ddt, *doa, *dnp, *dcam, *dno, *dcr, *dir;
   if ((rc = stage_in(h, 0, sp->dt, (size_t)nt * T * sizeof(double), smem_kind, &ddt))) return rc;
   if ((rc = stage_in(h, 1, sp->om_acc, (size_t)nt * T * 6 * sizeof(double), smem_kind, &doa))) return rc;
   if ((rc = stage_in(h, 2, sp->n_prop, (size_t)nt * E * sizeof(int32_t), smem_kind, &dnp))) return rc;
@@ -772,6 +898,7 @@ int eskf_run(eskf_t* h, const eskf_streams_t* sp, double* stats_out, double* sta
   a.stats_out = dstats;
   a.stats_sum = nullptr;  // (the kernels' own atomic sums are not used any more: see stats_partial_kernel)
   a.trace = dtrace;
+  a.cons = (h->cons_on && E > 0) ? h->cons_rec : nullptr;
   a.seed = sp->seed;
   a.noise_free0 = sp->noise_free_filter0;
   a.noise_mod = sp->noise_id_modulus;
@@ -847,6 +974,27 @@ int eskf_run(eskf_t* h, const eskf_streams_t* sp, double* stats_out, double* sta
     stats_final_kernel<<<1, 32, 0, h->stream>>>((const double*)h->stage[12], nblk, dsum);
     CK(cudaGetLastError());
     h->launches += 2;
+  }
+  if (h->cons_on) {
+    if (E > 0) {
+      NvtxRange nvtx_c("eskf_run: consistency post-pass");
+      double* nis = h->cons_out;
+      double* nees = nis + h->N * E;
+      double* esum = nees + h->N * E;
+      double* part = esum + E * ESKF_NCONS;
+      ConsArgs ca;
+      ca.N = h->N;
+      ca.E = E;
+      for (int i = 0; i < 6; ++i) ca.gt[i] = sp->gt_dofs[i];
+      ca.frozen_mask = h->model.frozen_mask & 63;
+      const int64_t n2 = h->N * E, nblk = cons_nblk(h);
+      cons_eval_kernel<<<(unsigned)((n2 + 127) / 128), 128, 0, h->stream>>>(h->cons_rec, nis, nees, ca);
+      cons_partial_kernel<<<(unsigned)(nblk * E), 256, 0, h->stream>>>(h->cons_rec, h->N, nblk, ca.frozen_mask != 63, part);
+      cons_final_kernel<<<(unsigned)((E * ESKF_NCONS + 127) / 128), 128, 0, h->stream>>>(part, nblk, E, esum);
+      CK(cudaGetLastError());
+      h->launches += 3;
+    }
+    h->cons_E = E;
   }
   if (dtrace && smem_kind == ESKF_MEM_HOST) {
     CK(cudaMemcpyAsync(sp->trace_x, dtrace, tb, cudaMemcpyDeviceToHost, h->stream));
@@ -950,6 +1098,10 @@ int64_t eskf_launch_count(const eskf_t* h) { return h ? h->launches : 0; }
 
 int eskf_set_variant(eskf_t* h, int variant) {
   if (!h || (variant != 0 && variant != 1 && variant != 3)) return ESKF_EINVAL;
+  if (variant == 1 && h->cons_on) {
+    g_err = "eskf_set_variant: filter consistency is on (default kernel only)";
+    return ESKF_EINVAL;
+  }
   h->variant = variant;
   return ESKF_OK;
 }
@@ -996,6 +1148,45 @@ int eskf_get_jacobians(eskf_t* h, double* Fx, double* Fi, int mem) {
     if (Fi) CK(cudaMemcpyAsync(Fi, dFi, bi, cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
   }
+  return ESKF_OK;
+}
+
+int eskf_keep_consistency(eskf_t* h, int on) {
+  if (!h) return ESKF_EINVAL;
+  if (on && kernel_of(h) != 3) {
+    g_err = "eskf_keep_consistency: default kernel only (eskf_set_variant(h, 1) selects the first one)";
+    return ESKF_EINVAL;
+  }
+  CK(cudaSetDevice(h->device));
+  h->cons_on = on != 0;
+  h->cons_E = -1;
+  if (!on && (h->cons_rec || h->cons_out)) {
+    CK(cudaStreamSynchronize(h->stream));
+    CK(cudaFree(h->cons_rec));
+    CK(cudaFree(h->cons_out));
+    h->cons_rec = h->cons_out = nullptr;
+    h->cons_rec_sz = h->cons_out_sz = 0;
+  }
+  return ESKF_OK;
+}
+
+int eskf_get_consistency(eskf_t* h, double* nis, double* nees, double* epoch_sum, int64_t* n_epochs, int mem) {
+  if (!h) return ESKF_EINVAL;
+  if (h->cons_E < 0) {
+    g_err = "eskf_get_consistency: no eskf_run since eskf_keep_consistency(h, 1)";
+    return ESKF_EINVAL;
+  }
+  const int64_t E = h->cons_E;
+  if (n_epochs) *n_epochs = E;
+  if (E == 0) return ESKF_OK;
+  CK(cudaSetDevice(h->device));
+  const cudaMemcpyKind kd = (mem == ESKF_MEM_HOST) ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice;
+  const size_t nb = (size_t)h->N * E * sizeof(double);
+  const double* src = h->cons_out;
+  if (nis) CK(cudaMemcpyAsync(nis, src, nb, kd, h->stream));
+  if (nees) CK(cudaMemcpyAsync(nees, src + h->N * E, nb, kd, h->stream));
+  if (epoch_sum) CK(cudaMemcpyAsync(epoch_sum, src + 2 * h->N * E, (size_t)E * ESKF_NCONS * sizeof(double), kd, h->stream));
+  if (mem == ESKF_MEM_HOST) CK(cudaStreamSynchronize(h->stream));
   return ESKF_OK;
 }
 

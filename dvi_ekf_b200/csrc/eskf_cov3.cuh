@@ -685,6 +685,20 @@ ESKF_HD void upd3_gain(int g, double* rec, const double* res, double (&K)[3][7],
   }
 }
 
+// NIS r^T inv(S) r of the update (eskf_keep_consistency): the residual and the inverse upd3_gain used, from the record
+template <int QS>
+ESKF_HD double upd3_nis(const double* rec, const double* res) {
+  double nis = 0.0;
+#pragma unroll
+  for (int j = 0; j < 7; ++j) {
+    double t = 0.0;
+#pragma unroll
+    for (int m = 0; m < 7; ++m) t += u3_get<QS>(rec, U3_SINV + 7 * j + m) * res[m];
+    nis += res[j] * t;
+  }
+  return nis;
+}
+
 // U2a: X <- (I - K H) X  (Joseph factor, Filter.py:384), then lanes 5..7 publish the columns h_m of W.
 // The diagonal entries of I - K H are formed first, 1 - K[h_a][a], exactly as the reference's I - K @ H does:
 // with a prior >> R they are O(1e-12) and everything they multiply is cancellation dominated, so the order

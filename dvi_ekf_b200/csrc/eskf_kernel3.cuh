@@ -970,6 +970,10 @@ __device__ __forceinline__ void role3_jac(const KArgs& a, const Ctx3& c, int lan
         put_notch((int)(k & 1), notch, dofs);
         if (EX && a.trace && k > 0) trace_dofs(a.trace + ((c.f0 + lane) * a.T + k - 1) * NX, dofs, notch);
       }
+      if (EX && a.cons) {  // consistency record: the DOFs after the update (before it, if it was not applied)
+#pragma unroll
+        for (int i = 0; i < 6; ++i) a.cons[(e * CONS_SIZE + CONS_DOFS + i) * a.N + c.f0 + lane] = dofs[i];
+      }
     }
     PT_MARK(6);
     JIT();
@@ -1389,7 +1393,7 @@ __device__ __forceinline__ bool inv7_group3(double* rec, int g, const double* rd
 #define COV3_SYNCWARP() __syncwarp(gmask)
 #endif
 
-template <int F, int NTHR>
+template <int F, int NTHR, bool EX>
 __device__ __forceinline__ void role3_cov(const KArgs& a, const Ctx3& c, int ct) {
   using L = Lay3<F>;
   const int cf = ct >> 3;  // filter of this lane (padded filters run on an identity tile, never stored)
@@ -1616,11 +1620,15 @@ __device__ __forceinline__ void role3_cov(const KArgs& a, const Ctx3& c, int ct)
     JIT();
     PT_MARK(6);
     const bool upd_c = inv_ok && (sxc[SX3_OK * F] != 0.0);
+    double nis = NAN;  // (export mode: consistency record)
     if (upd_c) {
       double K[3][7], res[7], dl[3];
 #pragma unroll
       for (int m = 0; m < 7; ++m) res[m] = sxc[(SX3_RES + m) * F];
       upd3_gain<4>(cg, rec, res, K, dl);
+      if constexpr (EX) {
+        if (a.cons && cg == 0) nis = upd3_nis<4>(rec, res);
+      }
 #pragma unroll
       for (int v = 0; v < 3; ++v) sxw[(SX3_DELTA + 3 * cg + v) * F] = dl[v];
       if (a.K_out && cf < c.nf) {
@@ -1631,6 +1639,13 @@ __device__ __forceinline__ void role3_cov(const KArgs& a, const Ctx3& c, int ct)
       }
     }
     if (cg == 0) sxw[SX3_OK2 * F] = upd_c ? 1.0 : 0.0;
+    if constexpr (EX) {
+      if (a.cons && cg == 0 && cf < c.nf) {
+        double* r = a.cons + e * CONS_SIZE * a.N + c.f0 + cf;
+        r[CONS_NIS * a.N] = nis;
+        r[CONS_NEES * a.N] = upd_c ? 1.0 : 0.0;
+      }
+    }
     PT_MARK(7);
     JIT();
     __syncthreads();  // U1 | U2  (also orders the K / K R records of the eight lanes)
@@ -1648,6 +1663,15 @@ __device__ __forceinline__ void role3_cov(const KArgs& a, const Ctx3& c, int ct)
       upd3_finish<4, F, 1>(X, cg, rec, sxc + SX3_RD * F, dth, dthc);
 #endif
     }
+    if constexpr (EX) {  // the DOF block of the posterior covariance: rows 9..14 of the tiles of lanes 3 and 4 (columns 9..14)
+      if (a.cons && (cg == 3 || cg == 4) && cf < c.nf) {
+        double* r = a.cons + (e * CONS_SIZE + CONS_B + 3 * (cg - 3)) * a.N + c.f0 + cf;
+#pragma unroll
+        for (int i = 0; i < 6; ++i)
+#pragma unroll
+          for (int v = 0; v < 3; ++v) r[(6 * i + v) * a.N] = X[9 + i][v];
+      }
+    }
     PT_MARK(10);
     // no CTA barrier here: the scalar roles go on to the first steps of the next epoch while the covariance warps
     // finish the Joseph form (what they exchange next is ordered by the record pipeline and by the next U0 | U1)
@@ -1659,9 +1683,9 @@ __device__ __forceinline__ void role3_cov(const KArgs& a, const Ctx3& c, int ct)
 }
 
 // ---------------------------------------------------------------------------------------------
-// MODE: bit 0 = export mode (FilterTraj rows, Jacobian record of the last step), bit 1 = stacked trajectories.  Separate
-// instantiations, so that the production kernel of a single-trajectory batch carries neither (a few integer instructions
-// in the prologue are enough to change the register allocation of the whole kernel).
+// MODE: bit 0 = export mode (FilterTraj rows, Jacobian record of the last step, consistency records), bit 1 = stacked
+// trajectories.  Separate instantiations, so that the production kernel of a single-trajectory batch carries neither (a few
+// integer instructions in the prologue are enough to change the register allocation of the whole kernel).
 template <int F, int REG_S, int REG_C, int MODE>
 __global__ void __launch_bounds__(128 + 8 * F, 1) eskf_kernel3(const __grid_constant__ KArgs a) {
   constexpr bool EX = (MODE & 1) != 0, MT = (MODE & 2) != 0;
@@ -1715,7 +1739,7 @@ __global__ void __launch_bounds__(128 + 8 * F, 1) eskf_kernel3(const __grid_cons
   // sub-partition -- a remapping that put two scalar roles on the sub-partition with the single covariance warp hung)
   if (warp >= 4) {
     reg_inc3<REG_C>();
-    role3_cov<F, NTHR>(a, c, tid - 128);
+    role3_cov<F, NTHR, EX>(a, c, tid - 128);
   } else {
     // (ptxas 12.9 crashes on kernels with more than one setmaxnreg.dec value, so all four scalar roles
     // share REG_S although the Jacobian warp's sub-partition would have room for more)

@@ -30,10 +30,10 @@ cudaError_t launch_eskf_kernel3<ESKF_F>(const KArgs& a, cudaStream_t stream) {
   static_assert(ESKF_REG_S == 0 || ESKF_REG_S + 2 * ESKF_REG_C <= 504, "register split exceeds a sub-partition");
   constexpr size_t smem = (size_t)Lay3<F>::TOTAL * sizeof(double);
   static_assert(smem <= 232448, "shared memory per CTA");
-  // export mode (FilterTraj rows, eskf_streams_t.trace_x; Jacobian record of the last step, eskf_keep_jacobians) and the
-  // CTA mapping of stacked trajectories are separate instantiations: the production kernel of a single-trajectory batch
-  // carries none of their code (the dump alone cost 10 % through register allocation)
-  const int mode = ((a.trace || a.fx_dump) ? 1 : 0) | (a.n_traj > 1 ? 2 : 0);
+  // export mode (FilterTraj rows, eskf_streams_t.trace_x; Jacobian record of the last step, eskf_keep_jacobians; consistency
+  // records, eskf_keep_consistency) and the CTA mapping of stacked trajectories are separate instantiations: the production
+  // kernel of a single-trajectory batch carries none of their code (the dump alone cost 10 % through register allocation)
+  const int mode = ((a.trace || a.fx_dump || a.cons) ? 1 : 0) | (a.n_traj > 1 ? 2 : 0);
   auto kern = mode == 0   ? eskf_kernel3<F, ESKF_REG_S, ESKF_REG_C, 0>
               : mode == 1 ? eskf_kernel3<F, ESKF_REG_S, ESKF_REG_C, 1>
               : mode == 2 ? eskf_kernel3<F, ESKF_REG_S, ESKF_REG_C, 2>

@@ -1225,4 +1225,61 @@ ESKF_HD void stacked_cta(int64_t block, int64_t N, int64_t fpt, int F, int64_t& 
   nf = (int)(left < F ? left : F);
 }
 
+// ---- filter consistency of eskf_run (eskf_keep_consistency) ------------------------------------------------------------
+// Record of one (epoch e, filter f), element-major so that the filters of a warp store and the post-pass reads coalesced:
+// element j at cons[(e * CONS_SIZE + j) * N + f].  The export instantiation of eskf_kernel3 files it, cons_eval_kernel
+// (eskf_api.cu) turns it into the NIS / NEES outputs.
+constexpr int CONS_NIS = 0;    // r^T inv(S) r of the update, NaN if it was not applied (covariance lane 0)
+constexpr int CONS_DOFS = 1;   // 6: dofs after the update (JACOB role)
+constexpr int CONS_NEES = 7;   // kernel: 1 if the update was applied, else 0; cons_eval_kernel overwrites it with the NEES
+constexpr int CONS_B = 8;      // 36: covariance block of error-state rows / columns 9..14 after the update, as the tile holds
+                               // it (the transpose of the reference's, which a quadratic form does not see; lanes 3 and 4)
+constexpr int CONS_SIZE = 44;  // doubles
+
+// NEES of the estimated DOFs: eps^T inv(B_m) eps, B_m the rows and columns of the 6x6 block B (row-major) whose bit of
+// frozen_mask is clear.  LU with partial pivoting on the whole (unsymmetrised) sub-block, as np.linalg.solve (LAPACK gesv)
+// does.  NaN when every DOF is frozen or a pivot is zero or not finite.
+ESKF_HD double nees_dofs(const double* B, const double* eps, int frozen_mask) {
+  const double nan = NAN;
+  int idx[6], d = 0;
+  for (int i = 0; i < 6; ++i)
+    if (!((frozen_mask >> i) & 1)) idx[d++] = i;
+  if (d == 0) return nan;
+  double A[6][6], b[6], x[6];
+  for (int i = 0; i < d; ++i) {
+    b[i] = eps[idx[i]];
+    for (int j = 0; j < d; ++j) A[i][j] = B[6 * idx[i] + idx[j]];
+  }
+  for (int k = 0; k < d; ++k) {
+    int p = k;
+    for (int i = k + 1; i < d; ++i)
+      if (fabs(A[i][k]) > fabs(A[p][k])) p = i;
+    const double piv = A[p][k];
+    if (!(fabs(piv) > 0.0) || piv * 0.0 != 0.0) return nan;  // zero, NaN or infinite pivot
+    if (p != k) {
+      for (int j = 0; j < d; ++j) {
+        const double t = A[k][j];
+        A[k][j] = A[p][j];
+        A[p][j] = t;
+      }
+      const double t = b[k];
+      b[k] = b[p];
+      b[p] = t;
+    }
+    for (int i = k + 1; i < d; ++i) {
+      const double l = A[i][k] / piv;
+      for (int j = k + 1; j < d; ++j) A[i][j] -= l * A[k][j];
+      b[i] -= l * b[k];
+    }
+  }
+  for (int i = d - 1; i >= 0; --i) {
+    double s = b[i];
+    for (int j = i + 1; j < d; ++j) s -= A[i][j] * x[j];
+    x[i] = s / A[i][i];
+  }
+  double q = 0.0;
+  for (int i = 0; i < d; ++i) q += eps[idx[i]] * x[i];
+  return q;
+}
+
 }  // namespace eskf

@@ -16,7 +16,7 @@ from typing import Optional, Sequence
 import numpy as np
 
 from . import _lib
-from ._lib import MEM_DEVICE, MEM_HOST, NSTAT, EskfModel, EskfStreams, check
+from ._lib import MEM_DEVICE, MEM_HOST, NCONS, NSTAT, EskfModel, EskfStreams, check
 
 
 def _is_torch(a) -> bool:
@@ -291,6 +291,33 @@ class BatchFilter:
         check(self._lib.eskf_get_jacobians(self._h, Fx.ctypes.data_as(C.c_void_p), Fi.ctypes.data_as(C.c_void_p), MEM_HOST),
               "eskf_get_jacobians")
         return Fx, Fi
+
+    def keep_consistency(self, on: bool = True):
+        """Every later ``run`` files the NIS of each filter's updates and the NEES of its estimated DOFs after them
+        (eskf_keep_consistency, include/eskf.h); read them with ``get_consistency``.  Runs the export instantiation of the
+        persistent kernel and needs N * E * 368 bytes of device memory; default kernel only."""
+        check(self._lib.eskf_keep_consistency(self._h, 1 if on else 0), "eskf_keep_consistency")
+
+    def get_consistency(self, device: bool = False):
+        """(nis [N,E], nees [N,E], epoch_sum [E,8]) of the last ``run`` since ``keep_consistency()``: NaN where the update was
+        not applied or the value is not finite; epoch_sum holds per epoch the count, sum and sum of squares of the finite NIS
+        ([0:3]) and NEES ([3:6]) and the number of filters with a NaN ([6]).  numpy arrays, or CUDA tensors with ``device``."""
+        E = C.c_int64()
+        check(self._lib.eskf_get_consistency(self._h, None, None, None, C.byref(E), MEM_HOST), "eskf_get_consistency")
+        E = int(E.value)
+        if device:
+            import torch
+
+            dev = torch.device("cuda", self.device)
+            out = [torch.empty(shape, dtype=torch.float64, device=dev) for shape in ((self.n, E), (self.n, E), (E, NCONS))]
+            ptrs, mem = [C.c_void_p(t.data_ptr()) for t in out], MEM_DEVICE
+        else:
+            out = [np.empty(shape) for shape in ((self.n, E), (self.n, E), (E, NCONS))]
+            ptrs, mem = [a.ctypes.data_as(C.c_void_p) for a in out], MEM_HOST
+        check(self._lib.eskf_get_consistency(self._h, *ptrs, None, mem), "eskf_get_consistency")
+        if device:
+            self.sync()  # (the copies ran on the handle's stream)
+        return tuple(out)
 
     def set_prepass_budget(self, n_bytes: int):
         """Memory ``run`` may use to keep the Monte-Carlo generator and the update-MSE statistics out of the persistent kernel

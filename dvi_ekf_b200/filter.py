@@ -16,6 +16,7 @@ import numpy as np
 from . import rotations as rot
 from .camera import Camera, Streams, build_streams, load_notch, load_trajectory
 from .config import Config
+from .consistency import NIS_DIM, candidate_objective, summarise_consistency
 from .engine import BatchFilter
 from .probe import GT_IMU_DOFS
 
@@ -325,6 +326,7 @@ class Simulator:
         self.mse_avg: Optional[float] = None
         self._kf_best = None
         self.stats = None
+        self.consistency = None  # summary of the last run(consistency=True)
 
     @property
     def config(self):
@@ -375,12 +377,19 @@ class Simulator:
         variables of the reference (random-walk std of the 6 DOFs and of the notch acceleration, measurement std of the
         camera position, orientation and notch) -- unlike the reference's setter (Simulator.py:76-86, which keeps only
         ``val[7:8]`` and never refreshes the variances) all 14 take effect.  Every candidate runs ``runs_per_candidate``
-        Monte-Carlo filters (run 0 of each candidate is noise free); returns the mean DOF MSE (``metric="dof"``,
-        Filter.calculate_dof_metric) or the mean update MSE (``"update"``) per candidate, [M]."""
+        Monte-Carlo filters (run 0 of each candidate is noise free); returns per candidate, [M], the mean DOF MSE
+        (``metric="dof"``, Filter.calculate_dof_metric), the mean update MSE (``"update"``) or the filter's inconsistency
+        ``|ln(ANIS / 7)|`` (``"nis"``) / ``|ln(ANEES / d)|`` (``"nees"``, d estimated DOFs), the averages taken over every finite
+        value of the candidate's runs and epochs (``consistency.candidate_objective``; +inf without one)."""
         X = np.atleast_2d(np.asarray(X, dtype=float))
         if X.shape[1] != 14:
             raise ValueError("candidates must have 14 columns: rw_std (7), meas_std (7)")
+        if metric not in ("dof", "update", "nis", "nees"):
+            raise ValueError(f"unknown metric {metric!r}: dof, update, nis or nees")
         cfg, s, b = self.config, self.streams, self.config.batch
+        dim_dofs = 6 - sum(1 for f in cfg.frozen_dofs if f)
+        if metric == "nees" and dim_dofs == 0:
+            raise ValueError("metric 'nees' needs at least one estimated DOF (frozen_dofs freezes all six)")
         m, r = len(X), int(runs_per_candidate or self.num_kf_runs)
         n = m * r
         Qd = np.zeros((n, 13))
@@ -398,11 +407,16 @@ class Simulator:
                          zero_frozen_dofs=not self.legacy_golden, device=self.device) as bf:
             bf.set_noise(Qd, Rd, self.kf.stdev_nom[None].copy())
             bf.set_state(x0, self._cov0[None], s.u0[None], None)
+            if metric in ("nis", "nees"):
+                bf.keep_consistency()
             # noise keyed by the run id INSIDE the candidate (noise_id_modulus = r): every candidate sees the same
             # r noise realisations, so candidates differ only by their parameters
             st, _ = bf.run(s.dt, s.om_acc, s.n_prop, s.cam, s.notch, cam_ref=s.cam_ref, imu_ref=s.imu_ref,
                            gt_dofs=cfg.gt_imu_dofs, seed=b.seed, imu_noise_std=imu_std, cam_noise_std=cam_std,
                            noise_free_filter0=True, noise_id_modulus=r)
+            if metric in ("nis", "nees"):
+                nis, nees, _ = bf.get_consistency()
+                return candidate_objective(nis if metric == "nis" else nees, m, NIS_DIM if metric == "nis" else dim_dofs)
         col = 6 if metric == "dof" else 8
         vals = st[:, col].reshape(m, r)
         if metric != "dof":
@@ -413,7 +427,9 @@ class Simulator:
                  metric: str = "dof"):
         """``Simulator.optimise`` (Simulator.py:163-245): differential evolution over the 14 noise parameters, with the
         objective of a whole generation evaluated by ONE batched launch (scipy ``vectorized=True``,
-        ``updating="deferred"``).  Returns the scipy result; the best parameters become ``optim_std``."""
+        ``updating="deferred"``).  ``metric`` is that of ``evaluate_candidates``: "dof" or "update" minimise an error,
+        "nis" / "nees" the distance of ANIS / ANEES from 7 / d (the usual objective for tuning Q and R: a filter whose
+        covariance matches its errors).  Returns the scipy result; the best parameters become ``optim_std``."""
         from scipy.optimize import differential_evolution
 
         def fun(x):  # x: (14, S) for a population of S members
@@ -433,10 +449,12 @@ class Simulator:
     def reset_kf(self) -> None:
         self.kf = Filter(self)
 
-    def run(self, disp_config=False, save_best=False, verbose=True, n_filters: Optional[int] = None):
+    def run(self, disp_config=False, save_best=False, verbose=True, n_filters: Optional[int] = None, consistency: bool = False):
         """Simulator.run (Simulator.py:121-158) as ONE batched launch: ``num_kf_runs`` (or ``n_filters``)
         independent filters, run 0 noise free (the reference's deterministic run), the others with
-        Monte-Carlo IMU / camera noise and DOF initial-condition perturbations (``batch:`` section)."""
+        Monte-Carlo IMU / camera noise and DOF initial-condition perturbations (``batch:`` section).
+        ``consistency``: ``self.consistency`` becomes ``consistency.summarise_consistency`` of the run (ANIS / ANEES per
+        epoch and their chi-square intervals)."""
         cfg, s = self.config, self.streams
         n = int(n_filters or self.num_kf_runs)
         b = cfg.batch
@@ -449,11 +467,15 @@ class Simulator:
                          zero_frozen_dofs=not self.legacy_golden, device=self.device) as bf:
             bf.set_noise(np.diag(self.kf.Q)[None].copy(), np.diag(self.kf.R)[None].copy(), self.kf.stdev_nom[None].copy())
             bf.set_state(x0, self._cov0[None], s.u0[None], None)
+            if consistency:
+                bf.keep_consistency()
             imu_std = np.hstack((cfg.imu.stdev_omega, cfg.imu.stdev_accel)) if b.imu_noise else None
             cam_std = np.array(cfg.meas_noise_std) if b.cam_noise else None
             st, sm = bf.run(s.dt, s.om_acc, s.n_prop, s.cam, s.notch, cam_ref=s.cam_ref, imu_ref=s.imu_ref,
                             gt_dofs=cfg.gt_imu_dofs, seed=b.seed, imu_noise_std=imu_std, cam_noise_std=cam_std)
             self.final_states = bf.get_state()[0]
+            if consistency:
+                self.consistency = summarise_consistency(bf.get_consistency()[2], 6 - sum(1 for f in cfg.frozen_dofs if f))
         self.stats = st
         # Simulator.py:138-158 appends ``kf.mse`` of every run -- which is 0 at the reference's HEAD, because the call that
         # would set it is commented out (Filter.py:92,167-168).  ``mses`` / ``mse_best`` / ``mse_avg`` keep exactly that

@@ -136,6 +136,29 @@ int eskf_get_state(eskf_t* h, double* x, double* P, double* u_old, double* R_old
 int eskf_keep_jacobians(eskf_t* h, int on);
 int eskf_get_jacobians(eskf_t* h, double* Fx, double* Fi, int mem);
 
+#define ESKF_NCONS 8
+/* Filter consistency of eskf_run (no reference counterpart): after eskf_keep_consistency(h, 1) every eskf_run files, per
+ * filter i and epoch e (every epoch has one update, n_prop[e] = 0 included):
+ *   nis[i,e]  = r^T inv(S) r, r the 7-dim residual of the update (Filter.py:363-375), S = H P- H^T + R the innovation
+ *               covariance it inverts; 7 in expectation for a consistent filter;
+ *   nees[i,e] = eps^T inv(B) eps over the ESTIMATED DOFs (bit k of frozen_mask clear, d = 6 - popcount(frozen_mask & 63)
+ *               of them): eps = dofs+ - gt_dofs after the update (rad / cm, the units of x[10:16]), B the block of error-state
+ *               rows / columns 9..14 of the covariance after the update (Joseph form and reset), solved by LU with partial
+ *               pivoting; d in expectation; NaN when d = 0.
+ * Both are NaN where the update was not applied (ESKF_STATUS_* cases) and where the value is not finite.
+ * epoch_sum[e, 0:8] sums over the handle's filters, FINITE values only (a diverged filter is counted, never propagates):
+ *   [0] number of finite NIS, [1] sum of NIS, [2] sum of NIS^2, [3] number of finite NEES, [4] sum, [5] sum of squares,
+ *   [6] filters whose NIS, or NEES when d > 0, is NaN at e, [7] reserved (0).
+ * Fixed reduction tree, no atomics: the same inputs give the same bits; plain sums, so shards combine by all-reduce.
+ * eskf_get_consistency returns those of the LAST such run: nis, nees [N,E]; epoch_sum [E,ESKF_NCONS]; *n_epochs = E.
+ * Any pointer may be NULL (query E first).  The run files the records through the export instantiation of the persistent
+ * kernel and needs N * E * 352 bytes of device memory for them (plus N * E * 16 for the results): eskf_run returns
+ * ESKF_ENOMEM, before anything is launched and with the handle unchanged, when they do not fit.  eskf_propagate /
+ * eskf_update neither file nor clear them; eskf_get_consistency before any such run is ESKF_EINVAL.  Default kernel only
+ * (variant 1: ESKF_EINVAL). */
+int eskf_keep_consistency(eskf_t* h, int on);
+int eskf_get_consistency(eskf_t* h, double* nis, double* nees, double* epoch_sum, int64_t* n_epochs, int mem);
+
 /* blocks until everything queued on the handle's stream has finished */
 int eskf_sync(eskf_t* h);
 
