@@ -16,12 +16,14 @@ FLAG_ZERO_FROZEN = 1
 STATUS_UPDATE_SKIPPED, STATUS_ASIN_DOMAIN = 1, 2
 NSTAT = 16
 NCONS = 8
+NDOFSUM = 80
 
 EXPORTS = (
     "eskf_create", "eskf_destroy", "eskf_set_state", "eskf_set_noise", "eskf_propagate", "eskf_update",
     "eskf_run", "eskf_get_state", "eskf_sync", "eskf_launch_count", "eskf_set_tuning", "eskf_last_error",
     "eskf_version", "eskf_fp64_peak", "eskf_set_variant", "eskf_noise_dump", "eskf_prepass", "eskf_prepass_last_error",
     "eskf_set_prepass_budget", "eskf_keep_jacobians", "eskf_get_jacobians", "eskf_keep_consistency", "eskf_get_consistency",
+    "eskf_get_dof_history", "eskf_get_dof_envelope",
 )
 
 
@@ -116,6 +118,8 @@ def load():
     lib.eskf_get_jacobians.argtypes = [vp, vp, vp, i32]
     lib.eskf_keep_consistency.argtypes = [vp, i32]
     lib.eskf_get_consistency.argtypes = [vp, vp, vp, vp, C.POINTER(i64), i32]
+    lib.eskf_get_dof_history.argtypes = [vp, vp, vp, C.POINTER(i64), i32]
+    lib.eskf_get_dof_envelope.argtypes = [vp, vp, C.POINTER(i64), i32]
     lib.eskf_fp64_peak.argtypes = [i32, vp, i32, C.POINTER(C.c_double), C.POINTER(C.c_double)]
     lib.eskf_noise_dump.argtypes = [i32, vp, C.c_uint64, i64, i64, i64, i64, i32, vp, i32]
     lib.eskf_prepass.argtypes = [i32, vp, C.POINTER(EskfModel), C.POINTER(EskfPrepassIn), C.POINTER(EskfPrepassOut),

@@ -9,6 +9,8 @@ from __future__ import annotations
 
 import numpy as np
 
+from ._lib import NDOFSUM
+
 NIS_DIM = 7  # measurement dimension (camera position, orientation, notch)
 
 
@@ -66,4 +68,71 @@ def candidate_objective(values, n_candidates: int, dim: int):
     ok = cnt > 0
     with np.errstate(divide="ignore"):
         out[ok] = np.abs(np.log(tot[ok] / cnt[ok] / dim))
+    return out
+
+
+_PAIRS = [(i, j) for i in range(6) for j in range(i + 1, 6)]  # the pair order of the dof_sum row, (0,1), (0,2), ..., (4,5)
+
+
+def summarise_dofs(dof_sum, frozen_dofs, alpha: float = 0.05) -> dict:
+    """Per-DOF Monte-Carlo envelope from ``dof_sum`` [E, 80] (``BatchFilter.get_dof_envelope`` of one handle, or the
+    all-reduced sum of several shards'; layout in include/eskf.h, eskf_get_dof_envelope); ``frozen_dofs`` six flags (the
+    config's ``frozen_dofs``).  With M the contributing filters of an epoch, eps = dofs - gt_dofs and B_ii the filter's
+    variance of DOF i, returns a dict of numpy arrays (NaN for frozen DOFs and for epochs with M = 0):
+
+    - ``bias`` [E,6] = mean eps; ``rmse`` [E,6] = sqrt(mean eps^2); ``std`` [E,6], the sample std of eps (NaN when M < 2);
+    - ``sigma_filter`` [E,6] = sqrt(mean B_ii), the filter's claimed sigma; ``inflation`` [E,6] = rmse / sigma_filter, the
+      factor by which that sigma is too small (1 for a consistent filter);
+    - ``anees_dof`` [E,6] = mean eps^2 / B_ii, 1 in expectation, and ``anees_interval`` [E,2], its (1 - alpha) chi-square
+      acceptance interval ``[chi2.ppf(alpha/2, M), chi2.ppf(1 - alpha/2, M)] / M``;
+    - ``coverage`` [E,6,3]: fraction of the filters with |eps| <= k sigma, k = 1, 2, 3; ``coverage_expected`` [3] =
+      erf(k / sqrt 2); ``coverage_interval`` [E,3,2], the binomial acceptance interval
+      ``[binom.ppf(alpha/2, M, p_k), binom.ppf(1 - alpha/2, M, p_k)] / M``;
+    - ``err_second_moment`` [E,6,6] = sum eps eps^T / M (the ensemble's error correlation, bias included) and
+      ``filter_cov`` [E,6,6] = sum B / M (the filter's claimed one, symmetrised);
+    - ``count`` [E] = M and ``excluded`` [E], the filters left out at the epoch.
+    """
+    from scipy.special import erf
+    from scipy.stats import binom, chi2
+
+    s = np.asarray(dof_sum, dtype=float).reshape(-1, NDOFSUM)
+    fr = np.asarray(frozen_dofs, dtype=bool).reshape(6)
+    E = len(s)
+    m = s[:, 0].copy()
+    has = m > 0
+    mm = np.where(has, m, 1.0)[:, None]  # (a divisor that is only used where M > 0)
+    dof = s[:, 2:44].reshape(E, 6, 7)
+    est = np.where(has[:, None] & ~fr[None, :], 1.0, np.nan)  # 1 for an estimated DOF of an epoch with M > 0, else NaN
+    s1, s2, sb, sr = dof[:, :, 0], dof[:, :, 1], dof[:, :, 2], dof[:, :, 3]
+    bias = s1 / mm * est
+    msq = s2 / mm * est
+    with np.errstate(invalid="ignore", divide="ignore"):
+        var = np.where(m[:, None] >= 2, np.maximum(s2 - s1 * s1 / mm, 0.0) / np.maximum(mm - 1, 1.0), np.nan) * est
+    sig = np.sqrt(sb / mm) * est
+    out = {"count": m, "excluded": s[:, 1].copy(), "bias": bias, "rmse": np.sqrt(msq), "std": np.sqrt(var), "sigma_filter": sig}
+    with np.errstate(invalid="ignore", divide="ignore"):
+        out["inflation"] = out["rmse"] / sig
+    out["anees_dof"] = sr / mm * est
+    iv = np.full((E, 2), np.nan)
+    if has.any():
+        iv[has, 0] = chi2.ppf(alpha / 2, m[has]) / m[has]
+        iv[has, 1] = chi2.ppf(1 - alpha / 2, m[has]) / m[has]
+    out["anees_interval"] = iv
+    k = np.arange(1, 4)
+    p = erf(k / np.sqrt(2.0))
+    out["coverage"] = dof[:, :, 4:7] / mm[:, :, None] * est[:, :, None]
+    out["coverage_expected"] = p
+    civ = np.full((E, 3, 2), np.nan)
+    if has.any():
+        mh = m[has][:, None]
+        civ[has, :, 0] = binom.ppf(alpha / 2, mh, p[None]) / mh
+        civ[has, :, 1] = binom.ppf(1 - alpha / 2, mh, p[None]) / mh
+    out["coverage_interval"] = civ
+    mask2 = est[:, :, None] * est[:, None, :]
+    for key, diag, off in (("err_second_moment", s2, s[:, 44:59]), ("filter_cov", sb, s[:, 59:74])):
+        a = np.zeros((E, 6, 6))
+        a[:, np.arange(6), np.arange(6)] = diag
+        for c, (i, j) in enumerate(_PAIRS):
+            a[:, i, j] = a[:, j, i] = off[:, c]
+        out[key] = a / mm[:, :, None] * mask2
     return out

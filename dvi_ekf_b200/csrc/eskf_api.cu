@@ -346,14 +346,116 @@ __global__ void cons_partial_kernel(const double* __restrict__ rec, int64_t N, i
   }
   if (threadIdx.x < ESKF_NCONS) partial[blockIdx.x * ESKF_NCONS + threadIdx.x] = threadIdx.x < 7 ? sh[0][threadIdx.x] : 0.0;
 }
-__global__ void cons_final_kernel(const double* __restrict__ partial, int64_t nblk, int64_t E, double* __restrict__ out) {
+// out [E][width] from the partial rows [E][nblk][width] of cons_partial_kernel (width ESKF_NCONS) or dof_partial_kernel
+// (ESKF_NDOFSUM): the blocks of an epoch added in order
+__global__ void cons_final_kernel(const double* __restrict__ partial, int64_t nblk, int64_t E, int width, double* __restrict__ out) {
   const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (idx >= E * ESKF_NCONS) return;
-  const int64_t e = idx / ESKF_NCONS, i = idx - e * ESKF_NCONS;
+  if (idx >= E * width) return;
+  const int64_t e = idx / width, i = idx - e * width;
   double a = 0.0;
-  for (int64_t b = 0; b < nblk; ++b) a += partial[(e * nblk + b) * ESKF_NCONS + i];
+  for (int64_t b = 0; b < nblk; ++b) a += partial[(e * nblk + b) * width + i];
   out[idx] = a;
 }
+
+// ---- per-DOF history and Monte-Carlo envelope: a second post-pass over the consistency records, run by the getters --------
+// (eskf_get_dof_history / eskf_get_dof_envelope) on the records of the last run, never by eskf_run itself.
+// dof_history_kernel: filter rows f0 .. f0 + nf - 1 of dofs / var [N][E][6] (either may be nullptr; row f0 at index 0).  A
+// block transposes a tile of 32 filters x 8 epochs through shared memory: every warp reads 32 consecutive filters of one
+// record element (256 B), and writes runs of 48 consecutive doubles (8 epochs of one filter).
+constexpr int HT_F = 32, HT_E = 8;
+__global__ void __launch_bounds__(256) dof_history_kernel(const double* __restrict__ rec, int64_t N, int64_t E, int64_t f0,
+                                                          int64_t nf, double* __restrict__ dofs, double* __restrict__ var) {
+  __shared__ double sd[HT_F][HT_E * 6 + 1], sv[HT_F][HT_E * 6 + 1];
+  const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
+  const int64_t fb = (int64_t)blockIdx.x * HT_F;
+  for (int64_t e0 = (int64_t)blockIdx.y * HT_E; e0 < E; e0 += (int64_t)gridDim.y * HT_E) {
+    const int64_t f = fb + tx, e = e0 + ty;
+    if (f < nf && e < E) {
+      const double* r = rec + e * CONS_SIZE * N + f0 + f;
+#pragma unroll
+      for (int i = 0; i < 6; ++i) {
+        if (dofs) sd[tx][6 * ty + i] = r[(CONS_DOFS + i) * N];
+        if (var) sv[tx][6 * ty + i] = r[(CONS_B + 7 * i) * N];
+      }
+    }
+    __syncthreads();
+    const int nc = 6 * (int)(E - e0 < HT_E ? E - e0 : HT_E);
+    for (int k = threadIdx.x; k < HT_F * HT_E * 6; k += 256) {
+      const int lf = k / (HT_E * 6), c = k - lf * (HT_E * 6);
+      if (fb + lf < nf && c < nc) {
+        const int64_t o = ((fb + lf) * E + e0) * 6 + c;
+        if (dofs) dofs[o] = sd[lf][c];
+        if (var) var[o] = sv[lf][c];
+      }
+    }
+    __syncthreads();
+  }
+}
+
+// dof_partial_kernel: the envelope rows [E][ESKF_NDOFSUM] deterministically, as cons_partial_kernel does the epoch sums:
+// block b of epoch e takes filters b RED_ROWS .. (b + 1) RED_ROWS - 1.  Each filter's DSUM_USED terms (dof_terms) do not fit
+// a per-thread accumulator, so every warp reduces the terms of its 32 filters at once, over fixed trees: recursive halving
+// over the lanes for each full group of 32 columns (after five exchange steps lane l holds the warp's sum of column
+// 32 g + l), an xor butterfly for each of the remaining columns (lane c - 64 keeps column c).  Every lane accumulates its
+// columns over the warp's rows in order, and the eight warps are added in order at the end.  cons_final_kernel adds the
+// blocks.
+__global__ void __launch_bounds__(256) dof_partial_kernel(const double* __restrict__ rec, const ConsArgs p, int64_t nblk,
+                                                          double* __restrict__ partial) {
+  constexpr int NG = DSUM_USED / 32;  // full column groups; the tail DSUM_USED - 32 NG < 32 columns
+  static_assert(DSUM_USED - 32 * NG < 32, "tail");
+  __shared__ double sh[8][32 * (NG + 1)];
+  const int64_t e = blockIdx.x / nblk, b = blockIdx.x - e * nblk;
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  const int64_t r1 = (b + 1) * RED_ROWS < p.N ? (b + 1) * RED_ROWS : p.N;
+  const double* re = rec + e * CONS_SIZE * p.N;
+  double acc[NG + 1];
+#pragma unroll
+  for (int g = 0; g <= NG; ++g) acc[g] = 0.0;
+  for (int64_t r0 = b * RED_ROWS + 32 * w; r0 < r1; r0 += 256) {  // (warp-uniform)
+    const int64_t r = r0 + lane;
+    double t[DSUM_USED];
+#pragma unroll
+    for (int c = 0; c < DSUM_USED; ++c) t[c] = 0.0;
+    if (r < r1) {
+      double eps[6];
+#pragma unroll
+      for (int i = 0; i < 6; ++i) eps[i] = re[(CONS_DOFS + i) * p.N + r] - p.gt[i];
+      dof_terms(re[CONS_NIS * p.N + r], eps, re + CONS_B * p.N + r, p.N, p.frozen_mask, t);
+    }
+    // (the tail first, then the groups from the last: fewer terms live at once)
+#pragma unroll
+    for (int c = 32 * NG; c < DSUM_USED; ++c) {
+      double v = t[c];
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+      if (lane == c - 32 * NG) acc[NG] += v;
+    }
+#pragma unroll
+    for (int g = NG - 1; g >= 0; --g) {
+      double* v = t + 32 * g;
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) {
+        const bool up = (lane & o) != 0;  // keeps the upper half of the columns, sends the lower one
+#pragma unroll
+        for (int j = 0; j < o; ++j) {
+          const double keep = up ? v[j + o] : v[j], send = up ? v[j] : v[j + o];
+          v[j] = keep + __shfl_xor_sync(0xffffffffu, send, o);
+        }
+      }
+      acc[g] += v[0];
+    }
+  }
+#pragma unroll
+  for (int g = 0; g <= NG; ++g) sh[w][32 * g + lane] = acc[g];
+  __syncthreads();
+  if (threadIdx.x < ESKF_NDOFSUM) {
+    double a = 0.0;
+    if (threadIdx.x < DSUM_USED)
+      for (int k = 0; k < 8; ++k) a += sh[k][threadIdx.x];
+    partial[blockIdx.x * ESKF_NDOFSUM + threadIdx.x] = a;
+  }
+}
+static_assert(DSUM_USED <= ESKF_NDOFSUM && ESKF_NDOFSUM <= 256, "envelope row");
 
 // Filter.Fx (24 x 24) and Filter.Fi (24 x 13) as the reference assembles them (Filter.py:249-342), from the fx3 record the
 // producer roles filed for the last IMU step of a launch (KArgs::fx_dump): the dense matrices the register-tile algebra of
@@ -433,11 +535,13 @@ struct eskf_handle {
   double* fxrec = nullptr;  // [N][FX3_SIZE] Jacobian record of the last step (eskf_keep_jacobians), or nullptr
   size_t pp_budget = 0;  // bytes the pre- / post-pass buffers of one eskf_run may take (0: everything inside the kernel)
   // filter consistency (eskf_keep_consistency): the records of one run [E][CONS_SIZE][N] and the results of the last run,
-  // one buffer: nis [N][E], nees [N][E], epoch_sum [E][ESKF_NCONS], the partial sums of the reduction
+  // one buffer: nis [N][E], nees [N][E], epoch_sum [E][ESKF_NCONS], the partial sums of the reduction, then the envelope row
+  // [E][ESKF_NDOFSUM] and its partial sums (eskf_get_dof_envelope)
   bool cons_on = false;
   int64_t cons_E = -1;  // epochs of the last run that filed them (-1: none since eskf_keep_consistency)
   double *cons_rec = nullptr, *cons_out = nullptr;
   size_t cons_rec_sz = 0, cons_out_sz = 0;
+  ConsArgs cons_args{};  // gt_dofs and frozen mask of the last run that filed them
 };
 
 #define CK(call)                                                  \
@@ -480,7 +584,8 @@ static int64_t cons_nblk(const eskf_t* h) { return (h->N + RED_ROWS - 1) / RED_R
 static int cons_reserve(eskf_t* h, int64_t E) {
   const size_t n = (size_t)h->N, e = (size_t)E;
   const size_t rb = e * CONS_SIZE * n * sizeof(double);
-  const size_t ob = (2 * n * e + e * ESKF_NCONS + (size_t)cons_nblk(h) * e * ESKF_NCONS) * sizeof(double);
+  const size_t nb = (size_t)cons_nblk(h);
+  const size_t ob = (2 * n * e + (e + nb * e) * (ESKF_NCONS + ESKF_NDOFSUM)) * sizeof(double);
   void *nr = nullptr, *no = nullptr;
   cudaError_t err = cudaSuccess;
   if (rb > h->cons_rec_sz) err = cudaMalloc(&nr, rb);
@@ -990,9 +1095,10 @@ int eskf_run(eskf_t* h, const eskf_streams_t* sp, double* stats_out, double* sta
       const int64_t n2 = h->N * E, nblk = cons_nblk(h);
       cons_eval_kernel<<<(unsigned)((n2 + 127) / 128), 128, 0, h->stream>>>(h->cons_rec, nis, nees, ca);
       cons_partial_kernel<<<(unsigned)(nblk * E), 256, 0, h->stream>>>(h->cons_rec, h->N, nblk, ca.frozen_mask != 63, part);
-      cons_final_kernel<<<(unsigned)((E * ESKF_NCONS + 127) / 128), 128, 0, h->stream>>>(part, nblk, E, esum);
+      cons_final_kernel<<<(unsigned)((E * ESKF_NCONS + 127) / 128), 128, 0, h->stream>>>(part, nblk, E, ESKF_NCONS, esum);
       CK(cudaGetLastError());
       h->launches += 3;
+      h->cons_args = ca;  // (for the envelope of eskf_get_dof_envelope)
     }
     h->cons_E = E;
   }
@@ -1186,6 +1292,74 @@ int eskf_get_consistency(eskf_t* h, double* nis, double* nees, double* epoch_sum
   if (nis) CK(cudaMemcpyAsync(nis, src, nb, kd, h->stream));
   if (nees) CK(cudaMemcpyAsync(nees, src + h->N * E, nb, kd, h->stream));
   if (epoch_sum) CK(cudaMemcpyAsync(epoch_sum, src + 2 * h->N * E, (size_t)E * ESKF_NCONS * sizeof(double), kd, h->stream));
+  if (mem == ESKF_MEM_HOST) CK(cudaStreamSynchronize(h->stream));
+  return ESKF_OK;
+}
+
+// the epochs of the last run that filed consistency records, or ESKF_EINVAL (shared by the getters of its records)
+static int cons_epochs(eskf_t* h, const char* what, int mem, int64_t* n_epochs, int64_t* E) {
+  if (!h || (mem != ESKF_MEM_HOST && mem != ESKF_MEM_DEVICE)) return ESKF_EINVAL;
+  if (h->cons_E < 0) {
+    g_err = std::string(what) + ": no eskf_run since eskf_keep_consistency(h, 1)";
+    return ESKF_EINVAL;
+  }
+  *E = h->cons_E;
+  if (n_epochs) *n_epochs = *E;
+  return ESKF_OK;
+}
+
+constexpr size_t DOF_STAGE_BYTES = (size_t)64 << 20;  // staging of eskf_get_dof_history into host memory
+
+int eskf_get_dof_history(eskf_t* h, double* dofs, double* var, int64_t* n_epochs, int mem) {
+  int64_t E;
+  int rc = cons_epochs(h, "eskf_get_dof_history", mem, n_epochs, &E);
+  if (rc || E == 0 || (!dofs && !var)) return rc;
+  CK(cudaSetDevice(h->device));
+  const int64_t row = 6 * E;  // doubles per filter and array
+  const unsigned gy = (unsigned)((E + HT_E - 1) / HT_E < 65535 ? (E + HT_E - 1) / HT_E : 65535);
+  auto launch = [&](int64_t f0, int64_t nf, double* d, double* v) {
+    dof_history_kernel<<<dim3((unsigned)((nf + HT_F - 1) / HT_F), gy), 256, 0, h->stream>>>(h->cons_rec, h->N, E, f0, nf, d, v);
+    h->launches += 1;
+  };
+  if (mem == ESKF_MEM_DEVICE) {
+    launch(0, h->N, dofs, var);
+    CK(cudaGetLastError());
+    return ESKF_OK;
+  }
+  // host destination: filter rows a chunk at a time through a staging buffer of at most DOF_STAGE_BYTES (the whole history
+  // of a large batch, N * E * 96 bytes, need not fit in device memory); one row per chunk at least
+  const int64_t arrays = (dofs ? 1 : 0) + (var ? 1 : 0);
+  int64_t chunk = (int64_t)(DOF_STAGE_BYTES / ((size_t)arrays * row * sizeof(double)));
+  chunk = chunk < 1 ? 1 : (chunk > h->N ? h->N : chunk);
+  if ((rc = stage_reserve(h, 2, (size_t)(arrays * chunk * row) * sizeof(double)))) return rc;
+  double* sd = dofs ? (double*)h->stage[2] : nullptr;
+  double* sv = var ? (double*)h->stage[2] + (dofs ? chunk * row : 0) : nullptr;
+  for (int64_t f0 = 0; f0 < h->N; f0 += chunk) {
+    const int64_t nf = h->N - f0 < chunk ? h->N - f0 : chunk;
+    const size_t nb = (size_t)(nf * row) * sizeof(double);
+    launch(f0, nf, sd, sv);
+    CK(cudaGetLastError());
+    if (dofs) CK(cudaMemcpyAsync(dofs + f0 * row, sd, nb, cudaMemcpyDeviceToHost, h->stream));
+    if (var) CK(cudaMemcpyAsync(var + f0 * row, sv, nb, cudaMemcpyDeviceToHost, h->stream));
+  }
+  CK(cudaStreamSynchronize(h->stream));
+  return ESKF_OK;
+}
+
+int eskf_get_dof_envelope(eskf_t* h, double* dof_sum, int64_t* n_epochs, int mem) {
+  int64_t E;
+  int rc = cons_epochs(h, "eskf_get_dof_envelope", mem, n_epochs, &E);
+  if (rc || E == 0 || !dof_sum) return rc;
+  CK(cudaSetDevice(h->device));
+  const int64_t nblk = cons_nblk(h);
+  double* row = h->cons_out + 2 * h->N * E + (E + nblk * E) * ESKF_NCONS;  // (the layout of cons_reserve)
+  double* part = row + E * ESKF_NDOFSUM;
+  dof_partial_kernel<<<(unsigned)(nblk * E), 256, 0, h->stream>>>(h->cons_rec, h->cons_args, nblk, part);
+  cons_final_kernel<<<(unsigned)((E * ESKF_NDOFSUM + 127) / 128), 128, 0, h->stream>>>(part, nblk, E, ESKF_NDOFSUM, row);
+  CK(cudaGetLastError());
+  h->launches += 2;
+  const cudaMemcpyKind kd = (mem == ESKF_MEM_HOST) ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice;
+  CK(cudaMemcpyAsync(dof_sum, row, (size_t)E * ESKF_NDOFSUM * sizeof(double), kd, h->stream));
   if (mem == ESKF_MEM_HOST) CK(cudaStreamSynchronize(h->stream));
   return ESKF_OK;
 }

@@ -1282,4 +1282,55 @@ ESKF_HD double nees_dofs(const double* B, const double* eps, int frozen_mask) {
   return q;
 }
 
+// Per-DOF Monte-Carlo envelope (eskf_get_dof_envelope): the row of one epoch, DSUM_USED of its ESKF_NDOFSUM doubles.
+constexpr int DSUM_M = 0;      // contributing filters
+constexpr int DSUM_EXCL = 1;   // excluded filters
+constexpr int DSUM_DOF = 2;    // 7 per DOF i at DSUM_DOF + 7 i: eps, eps^2, B_ii, eps^2 / B_ii, eps^2 <= k^2 B_ii (k = 1, 2, 3)
+constexpr int DSUM_EE = 44;    // 15: eps_i eps_j, pairs i < j row-major (0,1), (0,2), ..., (4,5)
+constexpr int DSUM_BB = 59;    // 15: (B_ij + B_ji) / 2, the same pairs
+constexpr int DSUM_USED = 74;  // the rest of the row is reserved (0)
+
+// The terms of one record for that row, t[0 .. DSUM_USED - 1]: nis as cons_eval_kernel left it, eps = dofs - gt_dofs,
+// B the 6x6 DOF block (row-major, element (i, j) at B[(6 i + j) ld]: ld = N reads it in place from a record).  The filter
+// contributes (t[DSUM_M] = 1) when the NIS is finite and, for every estimated DOF i (bit i of frozen_mask clear), eps_i and
+// B_ii are finite and B_ii > 0 and, for every pair of estimated DOFs, B_ij and B_ji are finite; otherwise t[DSUM_EXCL] = 1
+// and every other term is 0.  Terms of frozen DOFs, and of pairs that involve one, are 0.  The coverage counts compare eps^2
+// with k^2 B_ii as written (no square root), so a boundary case is inside.
+ESKF_HD bool dof_fin(double v) { return v * 0.0 == 0.0; }  // false for NaN and +-inf
+ESKF_HD bool dof_terms(double nis, const double* eps, const double* B, int64_t ld, int frozen_mask, double* t) {
+  bool ok = dof_fin(nis);
+#pragma unroll
+  for (int i = 0; i < 6; ++i) {
+    if ((frozen_mask >> i) & 1) continue;
+    const double bii = B[7 * i * ld];
+    ok = ok && dof_fin(eps[i]) && dof_fin(bii) && bii > 0.0;
+#pragma unroll
+    for (int j = i + 1; j < 6; ++j)
+      if (!((frozen_mask >> j) & 1)) ok = ok && dof_fin(B[(6 * i + j) * ld]) && dof_fin(B[(6 * j + i) * ld]);
+  }
+  t[DSUM_M] = ok ? 1.0 : 0.0;
+  t[DSUM_EXCL] = ok ? 0.0 : 1.0;
+  int p = 0;
+#pragma unroll
+  for (int i = 0; i < 6; ++i) {
+    const bool use = ok && !((frozen_mask >> i) & 1);
+    const double e = use ? eps[i] : 0.0, b = use ? B[7 * i * ld] : 1.0, e2 = e * e;
+    double* ti = t + DSUM_DOF + 7 * i;
+    ti[0] = e;
+    ti[1] = e2;
+    ti[2] = use ? b : 0.0;
+    ti[3] = use ? e2 / b : 0.0;
+    ti[4] = (use && e2 <= b) ? 1.0 : 0.0;
+    ti[5] = (use && e2 <= 4.0 * b) ? 1.0 : 0.0;
+    ti[6] = (use && e2 <= 9.0 * b) ? 1.0 : 0.0;
+#pragma unroll
+    for (int j = i + 1; j < 6; ++j, ++p) {
+      const bool uj = use && !((frozen_mask >> j) & 1);
+      t[DSUM_EE + p] = uj ? eps[i] * eps[j] : 0.0;
+      t[DSUM_BB + p] = uj ? 0.5 * (B[(6 * i + j) * ld] + B[(6 * j + i) * ld]) : 0.0;
+    }
+  }
+  return ok;
+}
+
 }  // namespace eskf

@@ -16,7 +16,7 @@ from typing import Optional, Sequence
 import numpy as np
 
 from . import _lib
-from ._lib import MEM_DEVICE, MEM_HOST, NCONS, NSTAT, EskfModel, EskfStreams, check
+from ._lib import MEM_DEVICE, MEM_HOST, NCONS, NDOFSUM, NSTAT, EskfModel, EskfStreams, check
 
 
 def _is_torch(a) -> bool:
@@ -318,6 +318,41 @@ class BatchFilter:
         if device:
             self.sync()  # (the copies ran on the handle's stream)
         return tuple(out)
+
+    def _cons_outputs(self, fn, name, shapes, device):
+        """arrays of ``shapes(E)`` filled by the consistency getter ``fn(h, *ptrs, n_epochs, mem)`` (E queried first)"""
+        E = C.c_int64()
+        check(fn(self._h, *([None] * len(shapes(0))), C.byref(E), MEM_HOST), name)
+        E = int(E.value)
+        if device:
+            import torch
+
+            dev = torch.device("cuda", self.device)
+            out = [torch.empty(shape, dtype=torch.float64, device=dev) for shape in shapes(E)]
+            ptrs, mem = [C.c_void_p(t.data_ptr()) for t in out], MEM_DEVICE
+        else:
+            out = [np.empty(shape) for shape in shapes(E)]
+            ptrs, mem = [a.ctypes.data_as(C.c_void_p) for a in out], MEM_HOST
+        check(fn(self._h, *ptrs, None, mem), name)
+        if device:
+            self.sync()  # (the kernels and copies ran on the handle's stream)
+        return out
+
+    def get_dof_history(self, device: bool = False):
+        """(dofs [N,E,6], var [N,E,6]) of the last ``run`` since ``keep_consistency()`` (eskf_get_dof_history,
+        include/eskf.h): every filter's calibration DOFs x[10:16] after each epoch's update, as the consistency records hold
+        them (before it where the update was not applied: nis NaN), and the diagonal of the DOF covariance block at the same
+        instant.  numpy arrays, or CUDA tensors with ``device``."""
+        return tuple(self._cons_outputs(self._lib.eskf_get_dof_history, "eskf_get_dof_history",
+                                        lambda E: ((self.n, E, 6), (self.n, E, 6)), device))
+
+    def get_dof_envelope(self, device: bool = False):
+        """dof_sum [E, 80] of the last ``run`` since ``keep_consistency()`` (eskf_get_dof_envelope, include/eskf.h): per
+        epoch, sums over this handle's contributing filters of the DOF errors, their squares, the filter variances, the
+        normalised squared errors, the 1 / 2 / 3 sigma coverage counts and the pair products, for
+        ``consistency.summarise_dofs``.  Computed from the records on every call; shards add their sums.  numpy array, or
+        CUDA tensor with ``device``."""
+        return self._cons_outputs(self._lib.eskf_get_dof_envelope, "eskf_get_dof_envelope", lambda E: ((E, NDOFSUM),), device)[0]
 
     def set_prepass_budget(self, n_bytes: int):
         """Memory ``run`` may use to keep the Monte-Carlo generator and the update-MSE statistics out of the persistent kernel

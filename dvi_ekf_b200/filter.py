@@ -16,7 +16,7 @@ import numpy as np
 from . import rotations as rot
 from .camera import Camera, Streams, build_streams, load_notch, load_trajectory
 from .config import Config
-from .consistency import NIS_DIM, candidate_objective, summarise_consistency
+from .consistency import NIS_DIM, candidate_objective, summarise_consistency, summarise_dofs
 from .engine import BatchFilter
 from .probe import GT_IMU_DOFS
 
@@ -327,6 +327,7 @@ class Simulator:
         self._kf_best = None
         self.stats = None
         self.consistency = None  # summary of the last run(consistency=True)
+        self.dof_envelope = None  # per-DOF envelope of the last run(consistency=True)
 
     @property
     def config(self):
@@ -454,7 +455,8 @@ class Simulator:
         independent filters, run 0 noise free (the reference's deterministic run), the others with
         Monte-Carlo IMU / camera noise and DOF initial-condition perturbations (``batch:`` section).
         ``consistency``: ``self.consistency`` becomes ``consistency.summarise_consistency`` of the run (ANIS / ANEES per
-        epoch and their chi-square intervals)."""
+        epoch and their chi-square intervals), ``self.dof_envelope`` ``consistency.summarise_dofs`` of it (bias, RMSE,
+        claimed sigma, inflation, per-DOF ANEES and coverage per DOF and epoch)."""
         cfg, s = self.config, self.streams
         n = int(n_filters or self.num_kf_runs)
         b = cfg.batch
@@ -476,6 +478,7 @@ class Simulator:
             self.final_states = bf.get_state()[0]
             if consistency:
                 self.consistency = summarise_consistency(bf.get_consistency()[2], 6 - sum(1 for f in cfg.frozen_dofs if f))
+                self.dof_envelope = summarise_dofs(bf.get_dof_envelope(), cfg.frozen_dofs)
         self.stats = st
         # Simulator.py:138-158 appends ``kf.mse`` of every run -- which is 0 at the reference's HEAD, because the call that
         # would set it is commented out (Filter.py:92,167-168).  ``mses`` / ``mse_best`` / ``mse_avg`` keep exactly that

@@ -36,7 +36,9 @@ def mc_initial_states(x0_row, n: int, first_id: int, seed: int):
 
 def allreduce_stats(stats_sum, group=None):
     """Sum of the per-rank statistics vectors (eskf_run's stats_sum), in place; a torch tensor on the device the
-    process group works on (NCCL: the GPU; gloo: the CPU).  No-op without an initialised process group."""
+    process group works on (NCCL: the GPU; gloo: the CPU).  No-op without an initialised process group.  It serves any
+    per-rank sum the same way: the consistency epoch sums (``get_consistency``) and the per-DOF envelope ``dof_sum``
+    (``get_dof_envelope``, for ``consistency.summarise_dofs``) as well."""
     import torch.distributed as dist
 
     if dist.is_available() and dist.is_initialized():

@@ -159,6 +159,34 @@ int eskf_get_jacobians(eskf_t* h, double* Fx, double* Fi, int mem);
 int eskf_keep_consistency(eskf_t* h, int on);
 int eskf_get_consistency(eskf_t* h, double* nis, double* nees, double* epoch_sum, int64_t* n_epochs, int mem);
 
+#define ESKF_NDOFSUM 80
+/* Per-DOF view of the same records (no reference counterpart), for the calibration DOFs x[10:16] (three rotations in rad,
+ * three translations in cm).  Both calls read the records of the LAST eskf_run since eskf_keep_consistency(h, 1), as
+ * eskf_get_consistency does, with its rules: ESKF_EINVAL before any such run, after eskf_keep_consistency(h, 0) and with
+ * variant 1; any pointer may be NULL; *n_epochs = E (E = 0 gives empty outputs); mem is ESKF_MEM_HOST (the call
+ * synchronises) or ESKF_MEM_DEVICE (asynchronous on the handle's stream).  Neither changes anything eskf_run returned, and
+ * eskf_run does no work for them.
+ *
+ * eskf_get_dof_history: dofs [N,E,6], the DOFs as the record holds them (after the update; before it where it was not
+ * applied, which a NaN nis marks), and var [N,E,6], the diagonal of the DOF covariance block at the same instant.  A host
+ * destination is filled through a device staging buffer of at most 64 MiB, filter rows at a time: the two arrays take
+ * N * E * 96 bytes and need not fit in device memory.
+ *
+ * eskf_get_dof_envelope: dof_sum [E,ESKF_NDOFSUM], per epoch sums over the handle's filters, computed by the call from the
+ * records.  With eps_i = dofs_i - gt_dofs[i] (the gt_dofs of that run) and B the 6x6 DOF block of the record, filter f
+ * CONTRIBUTES at epoch e when its nis is finite and, for every estimated DOF i (bit i of frozen_mask clear), eps_i and B_ii
+ * are finite and B_ii > 0 and, for every pair of estimated DOFs, B_ij and B_ji are finite.  Row e:
+ *   [0]  M, the contributing filters;  [1]  N - M, the excluded ones;
+ *   [2 + 7 i .. 2 + 7 i + 6] for DOF i = 0..5: sum eps_i, sum eps_i^2, sum B_ii, sum eps_i^2 / B_ii, and the number of
+ *        filters with eps_i^2 <= B_ii, eps_i^2 <= 4 B_ii, eps_i^2 <= 9 B_ii (compared as written: no square root);
+ *   [44 .. 58] sum eps_i eps_j over the 15 pairs i < j, row-major (0,1), (0,2), ..., (4,5);
+ *   [59 .. 73] sum (B_ij + B_ji) / 2 over the same pairs;   [74 .. 79] reserved (0).
+ * Sums over contributing filters only; entries of frozen DOFs, and of pairs that involve one, are 0.  Fixed reduction tree,
+ * no atomics: the same records give the same bits.  Plain sums: shards combine them by all-reduce.  The run reserves the
+ * row and its partial sums with the records (ESKF_ENOMEM before launch covers them). */
+int eskf_get_dof_history(eskf_t* h, double* dofs, double* var, int64_t* n_epochs, int mem);
+int eskf_get_dof_envelope(eskf_t* h, double* dof_sum, int64_t* n_epochs, int mem);
+
 /* blocks until everything queued on the handle's stream has finished */
 int eskf_sync(eskf_t* h);
 
