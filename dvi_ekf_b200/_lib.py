@@ -17,13 +17,14 @@ STATUS_UPDATE_SKIPPED, STATUS_ASIN_DOMAIN = 1, 2
 NSTAT = 16
 NCONS = 8
 NDOFSUM = 80
+NCARRY = 4
 
 EXPORTS = (
     "eskf_create", "eskf_destroy", "eskf_set_state", "eskf_set_noise", "eskf_propagate", "eskf_update",
     "eskf_run", "eskf_get_state", "eskf_sync", "eskf_launch_count", "eskf_set_tuning", "eskf_last_error",
     "eskf_version", "eskf_fp64_peak", "eskf_set_variant", "eskf_noise_dump", "eskf_prepass", "eskf_prepass_last_error",
     "eskf_set_prepass_budget", "eskf_keep_jacobians", "eskf_get_jacobians", "eskf_keep_consistency", "eskf_get_consistency",
-    "eskf_get_dof_history", "eskf_get_dof_envelope",
+    "eskf_get_dof_history", "eskf_get_dof_envelope", "eskf_run_epochs",
 )
 
 
@@ -107,6 +108,7 @@ def load():
     lib.eskf_propagate.argtypes = [vp, vp, vp, i64, i32, i32]
     lib.eskf_update.argtypes = [vp, vp, vp, i32, vp, i32]
     lib.eskf_run.argtypes = [vp, C.POINTER(EskfStreams), vp, vp, i32]
+    lib.eskf_run_epochs.argtypes = [vp, C.POINTER(EskfStreams), i64, i64, vp, vp, vp, vp, i32]
     lib.eskf_get_state.argtypes = [vp, vp, vp, vp, vp, vp, i32]
     lib.eskf_sync.argtypes = [vp]
     lib.eskf_launch_count.argtypes = [vp]

@@ -9,6 +9,7 @@
 #include <string.h>
 
 #include <string>
+#include <vector>
 
 #include "eskf_kernel3.cuh"
 
@@ -86,6 +87,9 @@ __global__ void noise_dump_kernel(double* out, uint64_t seed, int64_t filter_id0
 // that warp's sub-partition (12 % of the launch at 4096 filters, profiles/r02_*); as separate, fully parallel kernels they
 // cost a few per cent of that.  Same generator, same operations in the same order: the results are bit-identical
 // (tests/test_gpu_noise.py compares both paths).
+// A segment of the trajectory (eskf_run_epochs) indexes the buffers by the segment's steps and epochs (T, E) and the streams
+// and the noise counter by global step and epoch: trajectory t's step j is global step k0[t] + j (k0 = nullptr: 0) of the
+// T_all-long stream, epoch e is global epoch e0 + e of the E_all-long ones.
 struct PPArgs {
   int64_t N, T, E;
   int n_traj;
@@ -93,6 +97,8 @@ struct PPArgs {
   uint64_t seed;
   double imu_noise[6], cam_noise[7];
   int noise_on, noise_free0, noise_mod, per_filter;
+  const int64_t* k0;
+  int64_t T_all, E_all, e0;
 };
 
 __device__ __forceinline__ void pp_ids(const PPArgs& p, int64_t f, int64_t& traj, int64_t& gid, bool& noisy) {
@@ -110,13 +116,15 @@ __global__ void pp_imu_kernel(double* __restrict__ out, const double* __restrict
   int64_t traj, gid;
   bool noisy;
   pp_ids(p, f, traj, gid, noisy);
-  const double* src = p.per_filter ? om_acc + (f * p.T + j) * 6 : om_acc + (traj * p.T + j) * 6;
+  const int64_t g = (p.k0 ? p.k0[traj] : 0) + j;  // global step
+  if (g >= p.T_all) return;  // (past the end of this trajectory's stream: never read)
+  const double* src = p.per_filter ? om_acc + (f * p.T_all + g) * 6 : om_acc + (traj * p.T_all + g) * 6;
   double u[6];
 #pragma unroll
   for (int i = 0; i < 6; ++i) u[i] = src[i];
   if (noisy) {
     double z[8];
-    normal8(p.seed, (uint64_t)gid, (uint64_t)j, RNG_KIND_IMU, z);
+    normal8(p.seed, (uint64_t)gid, (uint64_t)g, RNG_KIND_IMU, z);
 #pragma unroll
     for (int i = 0; i < 6; ++i) u[i] += p.imu_noise[i] * z[i];
   }
@@ -135,14 +143,15 @@ __global__ void pp_meas_kernel(double* __restrict__ out, const double* __restric
   int64_t traj, gid;
   bool noisy;
   pp_ids(p, f, traj, gid, noisy);
-  const int64_t mrow = traj * p.E + e;
+  const int64_t eg = p.e0 + e;  // global epoch
+  const int64_t mrow = traj * p.E_all + eg;
   double cam[7];
 #pragma unroll
   for (int i = 0; i < 7; ++i) cam[i] = camm[mrow * 7 + i];
   double notch = notchm[mrow];
   if (noisy) {
     double z[8];
-    normal8(p.seed, (uint64_t)gid, (uint64_t)e, RNG_KIND_CAM, z);
+    normal8(p.seed, (uint64_t)gid, (uint64_t)eg, RNG_KIND_CAM, z);
     double dth[3];
 #pragma unroll
     for (int i = 0; i < 3; ++i) {
@@ -167,7 +176,8 @@ __global__ void pp_meas_kernel(double* __restrict__ out, const double* __restric
 // every update.  Stage 1, one thread per (epoch, filter): the two squared-error sums of the epoch (the same operations as
 // role3_stage's flush_stats), written over the first two entries of the snapshot.  Stage 2, one thread per filter: the
 // running sums over the epochs IN ORDER (the same additions as in the kernel), rows [7] (last epoch) and [8] (sum over
-// the epochs) of the statistics, and their contribution to stats_sum.
+// the epochs) of the statistics, and their contribution to stats_sum.  A segment of the trajectory continues the sums of
+// carry_in and leaves them in carry_out ([N][ESKF_NCARRY], entries 0 and 1; either may be nullptr).
 __global__ void pp_stats1_kernel(double* __restrict__ snap, const double* __restrict__ cam_ref,
                                  const double* __restrict__ imu_ref, const PPArgs p) {
   const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -177,8 +187,8 @@ __global__ void pp_stats1_kernel(double* __restrict__ snap, const double* __rest
   bool noisy;
   pp_ids(p, f, traj, gid, noisy);
   double* xs = snap + idx * 14;
-  const double* ir = imu_ref + (traj * p.E + e) * 6;
-  const double* cr = cam_ref + (traj * p.E + e) * 6;
+  const double* ir = imu_ref + (traj * p.E_all + p.e0 + e) * 6;
+  const double* cr = cam_ref + (traj * p.E_all + p.e0 + e) * 6;
   double xr[14];
 #pragma unroll
   for (int i = 0; i < 14; ++i) xr[i] = xs[i];
@@ -196,11 +206,16 @@ __global__ void pp_stats1_kernel(double* __restrict__ snap, const double* __rest
   xs[1] = accB;
 }
 
-__global__ void pp_stats2_kernel(const double* __restrict__ snap, double* stats_out, double* stats_sum, const PPArgs p) {
+__global__ void pp_stats2_kernel(const double* __restrict__ snap, double* stats_out, double* stats_sum, const PPArgs p,
+                                 const double* carry_in, double* carry_out) {
   const int64_t f = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   double r7 = 0.0, r8 = 0.0;
   if (f < p.N) {
     double mseA_last = 0.0, mseA_sum = 0.0, mseB_last = 0.0, mseB_sum = 0.0;
+    if (carry_in) {
+      mseA_sum = carry_in[f * ESKF_NCARRY + 0];
+      mseB_sum = carry_in[f * ESKF_NCARRY + 1];
+    }
     for (int64_t e = 0; e < p.E; ++e) {
       const double* xs = snap + (e * p.N + f) * 14;
       mseA_last = xs[0];
@@ -210,6 +225,10 @@ __global__ void pp_stats2_kernel(const double* __restrict__ snap, double* stats_
     }
     r7 = (mseA_last + mseB_last) / 12.0;
     r8 = (mseA_sum + mseB_sum) / 12.0;
+    if (carry_out) {
+      carry_out[f * ESKF_NCARRY + 0] = mseA_sum;
+      carry_out[f * ESKF_NCARRY + 1] = mseB_sum;
+    }
     if (stats_out) {
       stats_out[f * ESKF_NSTAT + 7] = r7;
       stats_out[f * ESKF_NSTAT + 8] = r8;
@@ -225,6 +244,38 @@ __global__ void pp_stats2_kernel(const double* __restrict__ snap, double* stats_
       atomicAdd(stats_sum + 7, r7);
       atomicAdd(stats_sum + 8, r8);
     }
+  }
+}
+
+// ---- segments of the trajectory (eskf_run_epochs) --------------------------------------------------------------------
+// kb[t] and kb[n_traj + t]: the global steps at which trajectory t's epochs e0 and e1 start, k(e) = sum over e' < e of
+// n_prop[t, e'] clamped as epoch_steps3 clamps every epoch (a negative entry counts 0 steps, none goes past T).  Clamping
+// each term to what is left makes the running sum saturate at T, so k(e) = min(T, sum of max(n_prop, 0)): an exact integer
+// reduction.  The one definition of a segment's first step, for the persistent kernel (KArgs::k_base) and the pre-pass.
+__global__ void __launch_bounds__(256) seg_base_kernel(const int32_t* __restrict__ n_prop, int64_t E, int64_t T, int64_t e0,
+                                                       int64_t e1, int n_traj, int64_t* __restrict__ kb) {
+  __shared__ long long sh[2][256];
+  const int t = blockIdx.x;
+  const int32_t* np_ = n_prop + (int64_t)t * E;
+  long long s0 = 0, s1 = 0;
+  for (int64_t e = threadIdx.x; e < e1; e += 256) {
+    const long long n = np_[e] > 0 ? np_[e] : 0;
+    if (e < e0) s0 += n;
+    s1 += n;
+  }
+  sh[0][threadIdx.x] = s0;
+  sh[1][threadIdx.x] = s1;
+  __syncthreads();
+  for (int o = 128; o > 0; o >>= 1) {
+    if ((int)threadIdx.x < o) {
+      sh[0][threadIdx.x] += sh[0][threadIdx.x + o];
+      sh[1][threadIdx.x] += sh[1][threadIdx.x + o];
+    }
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) {
+    kb[t] = sh[0][0] < T ? sh[0][0] : T;
+    kb[n_traj + t] = sh[1][0] < T ? sh[1][0] : T;
   }
 }
 
@@ -516,7 +567,9 @@ struct NvtxRange {
 }  // namespace
 
 // ---------------------------------------------------------------------------------------------
-constexpr int N_STAGE = 13;  // 0..8: arguments / results of the calls; 9..11: pre- / post-pass buffers of eskf_run; 12: partial sums
+// 0..8: arguments / results of the calls; 9..11: pre- / post-pass buffers of eskf_run; 12: partial sums; 13: first steps of a
+// segment (seg_base_kernel); 14, 15: host carry of eskf_run_epochs
+constexpr int N_STAGE = 16;
 struct eskf_handle {
   int device = 0;
   cudaStream_t stream = nullptr;
@@ -900,10 +953,16 @@ int eskf_update(eskf_t* h, const double* cam, const double* notch, int per_filte
   return ESKF_OK;
 }
 
-int eskf_run(eskf_t* h, const eskf_streams_t* sp, double* stats_out, double* stats_sum, int mem) {
-  NvtxRange nvtx_("eskf_run");
+// eskf_run and eskf_run_epochs: epochs [e0, e1) of the trajectory in `sp`.  `whole` (eskf_run) makes the launch eskf_run has
+// always made.  A segment -- a range other than [0, E), or a carry -- runs the instantiation with MODE bit 2: every CTA rebases
+// onto its trajectory's first step (k_base, seg_base_kernel) and the range's first epoch, the pre- and post-pass buffers and the
+// consistency records are sized by the segment, and the accumulators come from / go to the carry.
+static int run_epochs(eskf_t* h, const eskf_streams_t* sp, int64_t e0, int64_t e1, const double* carry_in, double* carry_out,
+                      double* stats_out, double* stats_sum, int mem, bool whole) {
+  const std::string fn = whole ? "eskf_run" : "eskf_run_epochs";
+  NvtxRange nvtx_(fn.c_str());
   if (!h || !sp || !sp->dt || !sp->om_acc || !sp->n_prop || !sp->cam || !sp->notch || sp->n_traj < 1) {
-    g_err = "eskf_run: bad argument";
+    g_err = fn + ": bad argument";
     return ESKF_EINVAL;
   }
   CK(cudaSetDevice(h->device));
@@ -911,17 +970,17 @@ int eskf_run(eskf_t* h, const eskf_streams_t* sp, double* stats_out, double* sta
   const int64_t T = sp->n_steps, E = sp->n_epochs, nt = sp->n_traj;
   const int64_t fpt = nt > 1 ? sp->filters_per_traj : h->N;
   if (T < 0 || E < 0 || sp->filter_id0 < 0) {
-    g_err = "eskf_run: n_steps, n_epochs and filter_id0 must not be negative";
+    g_err = fn + ": n_steps, n_epochs and filter_id0 must not be negative";
     return ESKF_EINVAL;
   }
   if (nt > 1) {
     // the kernels pick the trajectory of a filter from its GLOBAL id: (filter_id0 + f) / filters_per_traj
     if (fpt <= 0 || (sp->filter_id0 % fpt) != 0) {
-      g_err = "eskf_run: filter_id0 must be a multiple of filters_per_traj (a shard starts at a trajectory boundary)";
+      g_err = fn + ": filter_id0 must be a multiple of filters_per_traj (a shard starts at a trajectory boundary)";
       return ESKF_EINVAL;
     }
     if (sp->filter_id0 + h->N > nt * fpt) {
-      g_err = "eskf_run: filter_id0 + n_filters exceeds n_traj * filters_per_traj (the streams of " +
+      g_err = fn + ": filter_id0 + n_filters exceeds n_traj * filters_per_traj (the streams of " +
               std::to_string((long long)nt) + " trajectories do not cover these filters)";
       return ESKF_EINVAL;
     }
@@ -932,24 +991,52 @@ int eskf_run(eskf_t* h, const eskf_streams_t* sp, double* stats_out, double* sta
       for (int64_t e = 0; e < E; ++e) {
         const int32_t np_ = sp->n_prop[tr * E + e];
         if (np_ < 0) {
-          g_err = "eskf_run: negative n_prop entry";
+          g_err = fn + ": negative n_prop entry";
           return ESKF_EINVAL;
         }
         tot += np_;
       }
       if (tot > T) {
-        g_err = "eskf_run: sum(n_prop) = " + std::to_string((long long)tot) + " exceeds n_steps = " + std::to_string((long long)T);
+        g_err = fn + ": sum(n_prop) = " + std::to_string((long long)tot) + " exceeds n_steps = " + std::to_string((long long)T);
         return ESKF_EINVAL;
       }
     }
   }
+  if (!whole) {
+    if (e0 < 0 || e0 > e1 || e1 > E) {
+      g_err = fn + ": epoch range [" + std::to_string((long long)e0) + ", " + std::to_string((long long)e1) +
+              ") is not within [0, n_epochs = " + std::to_string((long long)E) + "]";
+      return ESKF_EINVAL;
+    }
+    if (kernel_of(h) != 3) {
+      g_err = fn + ": segments need the default kernel (eskf_set_variant(h, 1) selects the first one)";
+      return ESKF_EINVAL;
+    }
+  }
+  const size_t cb = (size_t)h->N * ESKF_NCARRY * sizeof(double);
+  if (!whole && e0 == e1) {  // an empty range launches nothing: the carry passes through, the statistics are not written
+    if (carry_out && carry_out != carry_in) {
+      if (mem == ESKF_MEM_DEVICE) {
+        if (carry_in) CK(cudaMemcpyAsync(carry_out, carry_in, cb, cudaMemcpyDeviceToDevice, h->stream));
+        else CK(cudaMemsetAsync(carry_out, 0, cb, h->stream));
+      } else if (carry_in) {
+        memcpy(carry_out, carry_in, cb);
+      } else {
+        memset(carry_out, 0, cb);
+      }
+    }
+    if (h->cons_on) h->cons_E = 0;
+    return ESKF_OK;
+  }
+  const int64_t Es = e1 - e0;  // epochs of this launch
+  const bool seg = !whole && (e0 > 0 || e1 < E || carry_in || carry_out);
   int rc;
   if (h->cons_on) {
     if (kernel_of(h) != 3) {
-      g_err = "eskf_run: filter consistency needs the default kernel (eskf_set_variant(h, 1) selects the first one)";
+      g_err = fn + ": filter consistency needs the default kernel (eskf_set_variant(h, 1) selects the first one)";
       return ESKF_EINVAL;
     }
-    if ((rc = cons_reserve(h, E))) return rc;
+    if ((rc = cons_reserve(h, Es))) return rc;
     h->cons_E = -1;  // (valid again once this run has filed its records)
   }
   const void *ddt, *doa, *dnp, *dcam, *dno, *dcr, *dir;
@@ -984,10 +1071,36 @@ int eskf_run(eskf_t* h, const eskf_streams_t* sp, double* stats_out, double* sta
   }
   double* dsum = nullptr;
   if (stats_sum) dsum = (mem == ESKF_MEM_DEVICE) ? stats_sum : h->stats_sum_dev;
+  const void* dcin = nullptr;
+  double* dcout = nullptr;
+  int64_t* kb = nullptr;  // [2][n_traj]: first step of every trajectory's epoch e0, then of its epoch e1
+  if (seg) {
+    if ((rc = stage_in(h, 14, carry_in, cb, mem, &dcin))) return rc;
+    if (carry_out) {
+      if (mem == ESKF_MEM_DEVICE) {
+        dcout = carry_out;
+      } else {
+        if ((rc = stage_reserve(h, 15, cb))) return rc;
+        dcout = (double*)h->stage[15];
+      }
+    }
+    if ((rc = stage_reserve(h, 13, (size_t)2 * nt * sizeof(int64_t)))) return rc;
+    kb = (int64_t*)h->stage[13];
+    seg_base_kernel<<<(unsigned)nt, 256, 0, h->stream>>>((const int32_t*)dnp, E, T, e0, e1, (int)nt, kb);
+    CK(cudaGetLastError());
+    h->launches += 1;
+  }
   KArgs a;
   base_args(h, a);
   a.T = T;
-  a.E = E;
+  a.E = whole ? E : Es;
+  if (seg) {
+    a.k_base = kb;
+    a.e_base = e0;
+    a.E_all = E;
+    a.carry_in = (const double*)dcin;
+    a.carry_out = dcout;
+  }
   a.n_traj = (int)nt;
   a.filters_per_traj = fpt;
   a.filter_id0 = sp->filter_id0;
@@ -1020,10 +1133,32 @@ int eskf_run(eskf_t* h, const eskf_streams_t* sp, double* stats_out, double* sta
   PPArgs pp;
   memset(&pp, 0, sizeof(pp));
 #if ESKF_OPT_PP
-  if (kernel_of(h) == 3 && h->pp_budget > 0 && T > 0 && E > 0) {
+  if (kernel_of(h) == 3 && h->pp_budget > 0 && T > 0 && a.E > 0) {
+    // a segment's sample buffer holds the most steps any trajectory takes in it, plus the sample the STAGER stages ahead
+    int64_t Ts = T;
+    if (seg && a.noise_on) {
+      int64_t most = 0;
+      if (smem_kind == ESKF_MEM_HOST) {  // (validated above: no negative entry, no sum past n_steps)
+        for (int64_t tr = 0; tr < nt; ++tr) {
+          int64_t n = 0;
+          for (int64_t e = e0; e < e1; ++e) n += sp->n_prop[tr * E + e];
+          most = n > most ? n : most;
+        }
+      } else {  // device-resident n_prop: read the segment's first steps back (the call synchronises here)
+        std::vector<int64_t> hk((size_t)(2 * nt));
+        CK(cudaMemcpyAsync(hk.data(), kb, hk.size() * sizeof(int64_t), cudaMemcpyDeviceToHost, h->stream));
+        CK(cudaStreamSynchronize(h->stream));
+        for (int64_t tr = 0; tr < nt; ++tr) most = hk[nt + tr] - hk[tr] > most ? hk[nt + tr] - hk[tr] : most;
+      }
+      Ts = most + 1;
+    }
     pp.N = h->N;
-    pp.T = T;
-    pp.E = E;
+    pp.T = Ts;
+    pp.E = a.E;
+    pp.k0 = kb;
+    pp.T_all = T;
+    pp.E_all = E;
+    pp.e0 = seg ? e0 : 0;
     pp.n_traj = (int)nt;
     pp.fpt = fpt;
     pp.filter_id0 = sp->filter_id0;
@@ -1035,14 +1170,14 @@ int eskf_run(eskf_t* h, const eskf_streams_t* sp, double* stats_out, double* sta
     pp.noise_mod = a.noise_mod;
     pp.per_filter = 0;
     const bool want_stats = dcr && dir && dstats;
-    const size_t b_imu = a.noise_on ? (size_t)h->N * T * 6 * sizeof(double) : 0;
-    const size_t b_meas = a.noise_on ? (size_t)h->N * E * 8 * sizeof(double) : 0;
-    const size_t b_snap = want_stats ? (size_t)h->N * E * 14 * sizeof(double) : 0;
+    const size_t b_imu = a.noise_on ? (size_t)h->N * Ts * 6 * sizeof(double) : 0;
+    const size_t b_meas = a.noise_on ? (size_t)h->N * a.E * 8 * sizeof(double) : 0;
+    const size_t b_snap = want_stats ? (size_t)h->N * a.E * 14 * sizeof(double) : 0;
     if (b_imu + b_meas + b_snap <= h->pp_budget) {
       if (a.noise_on) {
         if ((rc = stage_reserve(h, 9, b_imu))) return rc;
         if ((rc = stage_reserve(h, 10, b_meas))) return rc;
-        const int64_t n1 = h->N * T, n2 = h->N * E;
+        const int64_t n1 = h->N * Ts, n2 = h->N * a.E;
         NvtxRange nvtx_pp("eskf_run: Monte-Carlo pre-pass");
         pp_imu_kernel<<<(unsigned)((n1 + 255) / 256), 256, 0, h->stream>>>((double*)h->stage[9], a.om_acc, pp);
         pp_meas_kernel<<<(unsigned)((n2 + 255) / 256), 256, 0, h->stream>>>((double*)h->stage[10], a.cam, a.notch, pp);
@@ -1065,9 +1200,9 @@ int eskf_run(eskf_t* h, const eskf_streams_t* sp, double* stats_out, double* sta
   }
   if (pp_stats) {
     NvtxRange nvtx_ps("eskf_run: statistics post-pass");
-    const int64_t n2 = h->N * E;
+    const int64_t n2 = h->N * a.E;
     pp_stats1_kernel<<<(unsigned)((n2 + 127) / 128), 128, 0, h->stream>>>(a.snap, a.cam_ref, a.imu_ref, pp);
-    pp_stats2_kernel<<<(unsigned)((h->N + 63) / 64), 64, 0, h->stream>>>(a.snap, dstats, nullptr, pp);
+    pp_stats2_kernel<<<(unsigned)((h->N + 63) / 64), 64, 0, h->stream>>>(a.snap, dstats, nullptr, pp, a.carry_in, a.carry_out);
     CK(cudaGetLastError());
     h->launches += 2;
   }
@@ -1081,6 +1216,7 @@ int eskf_run(eskf_t* h, const eskf_streams_t* sp, double* stats_out, double* sta
     h->launches += 2;
   }
   if (h->cons_on) {
+    const int64_t E = a.E;  // (a segment's records: its epochs only)
     if (E > 0) {
       NvtxRange nvtx_c("eskf_run: consistency post-pass");
       double* nis = h->cons_out;
@@ -1106,13 +1242,24 @@ int eskf_run(eskf_t* h, const eskf_streams_t* sp, double* stats_out, double* sta
     CK(cudaMemcpyAsync(sp->trace_x, dtrace, tb, cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
   }
-  if (mem == ESKF_MEM_HOST && (stats_out || stats_sum)) {
+  if (mem == ESKF_MEM_HOST && (stats_out || stats_sum || dcout)) {
     if (stats_out) CK(cudaMemcpyAsync(stats_out, dstats, sb, cudaMemcpyDeviceToHost, h->stream));
     if (stats_sum) CK(cudaMemcpyAsync(stats_sum, dsum, ESKF_NSTAT * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+    if (dcout) CK(cudaMemcpyAsync(carry_out, dcout, cb, cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
   }
   return ESKF_OK;
 }
+
+int eskf_run(eskf_t* h, const eskf_streams_t* sp, double* stats_out, double* stats_sum, int mem) {
+  return run_epochs(h, sp, 0, sp ? sp->n_epochs : 0, nullptr, nullptr, stats_out, stats_sum, mem, true);
+}
+
+int eskf_run_epochs(eskf_t* h, const eskf_streams_t* sp, int64_t epoch_begin, int64_t epoch_end, const double* carry_in,
+                    double* carry_out, double* stats_out, double* stats_sum, int mem) {
+  return run_epochs(h, sp, epoch_begin, epoch_end, carry_in, carry_out, stats_out, stats_sum, mem, false);
+}
+
 
 int eskf_get_state(eskf_t* h, double* x, double* P, double* u_old, double* R_old, int32_t* status, int mem) {
   if (!h) return ESKF_EINVAL;

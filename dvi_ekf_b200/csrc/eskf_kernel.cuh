@@ -72,6 +72,13 @@ struct KArgs {
   double* fx_dump;        // [N][FX3_SIZE] Jacobian record of the filter's LAST executed IMU step of the launch (eskf_get_jacobians), or nullptr
   // (members added below this line keep the parameter offsets of the ones above: the production instantiation does not move)
   double* cons;           // [E][CONS_SIZE][N] consistency record of every update (eskf_keep_consistency, eskf_math.cuh), or nullptr
+  // a segment of the trajectory (eskf_run_epochs; eskf_kernel3, MODE bit 2 only): epochs [e_base, e_base + E) of streams whose
+  // per-epoch rows are E_all long, trajectory t starting at step k_base[t]; the per-filter accumulators the statistics row
+  // cannot hold come from carry_in and go to carry_out ([N][ESKF_NCARRY], either may be nullptr)
+  const int64_t* k_base;
+  int64_t e_base, E_all;
+  const double* carry_in;
+  double* carry_out;
 };
 
 // one FilterTraj row's worth of nominal state in the layout of x (include/eskf.h)

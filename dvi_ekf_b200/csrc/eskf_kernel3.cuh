@@ -271,8 +271,6 @@ __device__ __forceinline__ void scalar_barrier() { asm volatile("bar.sync 1, 128
 __device__ __forceinline__ void pk_ready_arrive() { asm volatile("bar.arrive 2, 64;" ::: "memory"); }
 __device__ __forceinline__ void pk_ready_wait() { asm volatile("bar.sync 2, 64;" ::: "memory"); }
 
-struct Ctx3;
-__device__ __forceinline__ int epoch_steps3(const KArgs& a, const Ctx3& c, int64_t e, int64_t k);
 
 struct Ctx3 {
   double* smem;
@@ -280,17 +278,39 @@ struct Ctx3 {
   int nf;          // filters of this CTA that exist
   int64_t gid0;    // global id of the CTA's first filter
   int64_t traj;
-  const int32_t* n_prop;
-  const double* dtp;
+  const int32_t* n_prop;  // the CTA's trajectory, from the launch's first epoch
+  const double* dtp;      // the same, from the launch's first step
   uint64_t* mbar;  // full[2], empty[2]
+  int64_t k0;      // a segment of the trajectory (MODE bit 2): global step of the launch's step 0 (read through k0_of)
 };
 
-// IMU steps of epoch e, k steps into the stream: n_prop[e] clamped to what is left of the stream, so that inconsistent
+// The rebasing of a segment (MODE bit 2, eskf_run_epochs) as the roles see it.  In the other instantiations every term is
+// a constant or the very expression they had before, so that their code does not change: a value kept in a register for the
+// whole launch instead of a parameter read at its use is enough to change the register allocation of the kernel.
+template <bool SG>
+__device__ __forceinline__ int64_t k0_of(const Ctx3& c) {  // global step of the launch's step 0
+  return SG ? c.k0 : 0;
+}
+template <bool SG>
+__device__ __forceinline__ int64_t erow3(const KArgs& a, const Ctx3& c, int64_t e) {  // row of launch epoch e in [n_traj, E]
+  return SG ? c.traj * a.E_all + a.e_base + e : c.traj * a.E + e;
+}
+template <bool SG>
+__device__ __forceinline__ const double* carry_in3(const KArgs& a) {
+  return SG ? a.carry_in : nullptr;
+}
+template <bool SG>
+__device__ __forceinline__ double* carry_out3(const KArgs& a) {
+  return SG ? a.carry_out : nullptr;
+}
+
+// IMU steps of epoch e, k steps into the launch: n_prop[e] clamped to what is left of the stream, so that inconsistent
 // DEVICE-resident streams (sum(n_prop) > n_steps; host streams are validated by eskf_run) can never index past the sample
 // stream, the ring or the trace rows
+template <bool SG>
 __device__ __forceinline__ int epoch_steps3(const KArgs& a, const Ctx3& c, int64_t e, int64_t k) {
   if (!c.n_prop) return (int)a.T;
-  const int64_t left = a.T - k;
+  const int64_t left = a.T - k0_of<SG>(c) - k;
   const int64_t n = c.n_prop[e];
   return (int)(n < 0 ? 0 : (n > left ? left : n));
 }
@@ -298,9 +318,10 @@ __device__ __forceinline__ int epoch_steps3(const KArgs& a, const Ctx3& c, int64
 // the last IMU step the CTA's trajectory executes in this launch (-1: none), where export mode files the Jacobian record:
 // the epochs' steps as epoch_steps3 counts them, which may add up to less than n_steps (stacked trajectories share the
 // stream length, each has its own n_prop)
+template <bool SG>
 __device__ __forceinline__ int64_t last_step3(const KArgs& a, const Ctx3& c) {
   int64_t k = 0;
-  for (int64_t e = 0; e < a.E; ++e) k += epoch_steps3(a, c, e, k);
+  for (int64_t e = 0; e < a.E; ++e) k += epoch_steps3<SG>(a, c, e, k);
   return k - 1;
 }
 
@@ -394,7 +415,7 @@ __device__ __forceinline__ bool h1_by_stager(const KArgs& a) {
 
 // ---------------------------------------------------------------------------------------------
 // role 0: IMU nominal state
-template <int F, int NTHR, bool EX>
+template <int F, int NTHR, bool EX, bool SG>
 __device__ __forceinline__ void role3_imu(const KArgs& a, const Ctx3& c, int lane) {
   using L = Lay3<F>;
   const bool act = lane < c.nf;
@@ -423,10 +444,10 @@ __device__ __forceinline__ void role3_imu(const KArgs& a, const Ctx3& c, int lan
   __syncthreads();  // prologue
   PT_DECL();
   JIT_DECL();
-  const int64_t k_jac = EX ? last_step3(a, c) : -1;  // (export mode: the step whose Jacobian record is filed)
+  const int64_t k_jac = EX ? last_step3<SG>(a, c) : -1;  // (export mode: the step whose Jacobian record is filed)
   int64_t k = 0;
   for (int64_t e = 0; e < a.E; ++e) {
-    const int n = epoch_steps3(a, c, e, k);
+    const int n = epoch_steps3<SG>(a, c, e, k);
     for (int it = 0; it < n; ++it) {
       const int64_t kk = k + it;
 #if !ESKF_OPT_LATEACQ
@@ -470,7 +491,7 @@ __device__ __forceinline__ void role3_imu(const KArgs& a, const Ctx3& c, int lan
         }
 #endif
         imu_nominal_step(p, v, q, Rwb, dt, om_old, acc_old, om, acc, Rold);
-        if (EX && a.trace) trace_pvq(a.trace + ((c.f0 + lane) * a.T + kk) * NX, p, v, q);
+        if (EX && a.trace) trace_pvq(a.trace + ((c.f0 + lane) * a.T + k0_of<SG>(c) + kk) * NX, p, v, q);
         const int s = (int)((kk + 1) & 1);
 #pragma unroll
         for (int i = 0; i < 9; ++i) {
@@ -532,7 +553,7 @@ __device__ __forceinline__ void role3_imu(const KArgs& a, const Ctx3& c, int lan
 #pragma unroll
         for (int i = 0; i < 4; ++i) q[i] = qn[i];
         quat_to_rot(q, Rwb);  // R_WB of the next step; R_WB_old keeps the pre-update value (quirk Q8)
-        if (EX && a.trace && k > 0) trace_pvq(a.trace + ((c.f0 + lane) * a.T + k - 1) * NX, p, v, q);  // FilterTraj.append_updated_states
+        if (EX && a.trace && k0_of<SG>(c) + k > 0) trace_pvq(a.trace + ((c.f0 + lane) * a.T + k0_of<SG>(c) + k - 1) * NX, p, v, q);  // FilterTraj.append_updated_states
         const int s = (int)(k & 1);
 #pragma unroll
         for (int i = 0; i < 9; ++i) sx[(SX3_RW + 9 * s + i) * F] = Rwb[i];
@@ -587,7 +608,7 @@ __device__ __forceinline__ void role3_imu(const KArgs& a, const Ctx3& c, int lan
 
 // ---------------------------------------------------------------------------------------------
 // role 1: camera nominal state + measurement residual
-template <int F, int NTHR, bool EX>
+template <int F, int NTHR, bool EX, bool SG>
 __device__ __forceinline__ void role3_cam(const KArgs& a, const Ctx3& c, int lane) {
   using L = Lay3<F>;
   const bool act = lane < c.nf;
@@ -607,15 +628,19 @@ __device__ __forceinline__ void role3_cam(const KArgs& a, const Ctx3& c, int lan
 #pragma unroll
     for (int i = 0; i < 4; ++i) qc[i] = xg[22 + i];
     st = a.status[c.f0 + lane];
+    if (carry_in3<SG>(a)) {  // a continued trajectory: updates applied so far, and the status word of the checkpoint
+      n_upd = carry_in3<SG>(a)[(c.f0 + lane) * ESKF_NCARRY + 2];
+      st = (int32_t)carry_in3<SG>(a)[(c.f0 + lane) * ESKF_NCARRY + 3];
+    }
   }
   __syncthreads();  // prologue
   PT_DECL();
   JIT_DECL();
   const bool h1s = h1_by_stager<EX>(a);  // rows 18:21 of Fx are the STAGER's work in this launch (see role3_stage)
-  const int64_t k_jac = EX ? last_step3(a, c) : -1;
+  const int64_t k_jac = EX ? last_step3<SG>(a, c) : -1;
   int64_t k = 0;
   for (int64_t e = 0; e < a.E; ++e) {
-    const int n = epoch_steps3(a, c, e, k);
+    const int n = epoch_steps3<SG>(a, c, e, k);
     for (int it = 0; it < n; ++it) {
       const int64_t kk = k + it;
 #if !ESKF_OPT_LATEACQ
@@ -646,7 +671,7 @@ __device__ __forceinline__ void role3_cam(const KArgs& a, const Ctx3& c, int lan
         const double dt = un[6 * F];
         const double notch_d = sx[(SX3_PK + PK3 * s + 16) * F];
         cam_nominal_step(pc, qc, vpre, Rwb, dt, om_old, om, pkp, pkR, pkz, notch_d);
-        if (EX && a.trace) trace_cam(a.trace + ((c.f0 + lane) * a.T + kk) * NX, pc, qc);
+        if (EX && a.trace) trace_cam(a.trace + ((c.f0 + lane) * a.T + k0_of<SG>(c) + kk) * NX, pc, qc);
       }
       PT_MARK(1);
       JIT();
@@ -754,7 +779,7 @@ __device__ __forceinline__ void role3_cam(const KArgs& a, const Ctx3& c, int lan
 #pragma unroll
         for (int i = 0; i < 4; ++i) qc[i] = qn[i];
         n_upd += 1.0;
-        if (EX && a.trace && k > 0) trace_cam(a.trace + ((c.f0 + lane) * a.T + k - 1) * NX, pc, qc);
+        if (EX && a.trace && k0_of<SG>(c) + k > 0) trace_cam(a.trace + ((c.f0 + lane) * a.T + k0_of<SG>(c) + k - 1) * NX, pc, qc);
       } else {
         st |= ESKF_STATUS_UPDATE_SKIPPED;
       }
@@ -790,6 +815,10 @@ __device__ __forceinline__ void role3_cam(const KArgs& a, const Ctx3& c, int lan
     a.status[c.f0 + lane] = st;
     sx[(SX3_ST + 4) * F] = n_upd;
     sx[(SX3_ST + 5) * F] = (double)st;
+    if (carry_out3<SG>(a)) {
+      carry_out3<SG>(a)[(c.f0 + lane) * ESKF_NCARRY + 2] = n_upd;
+      carry_out3<SG>(a)[(c.f0 + lane) * ESKF_NCARRY + 3] = (double)st;
+    }
   }
   __syncthreads();
   store_tiles3<F, NTHR>(a, c, threadIdx.x);
@@ -799,7 +828,7 @@ __device__ __forceinline__ void role3_cam(const KArgs& a, const Ctx3& c, int lan
 // role 2: dofs / notch, probe kinematics, Jacobian blocks (rows 21:24 and the noise rows; rows 3:9 come from the IMU
 // role, rows 18:21 from the CAMERA role).
 // The probe kinematics and their trigonometry cache live in shared memory (PK slots, TR), not in registers.
-template <int F, int NTHR, bool EX>
+template <int F, int NTHR, bool EX, bool SG>
 __device__ __forceinline__ void role3_jac(const KArgs& a, const Ctx3& c, int lane) {
   using L = Lay3<F>;
   const bool act = lane < c.nf;
@@ -834,10 +863,10 @@ __device__ __forceinline__ void role3_jac(const KArgs& a, const Ctx3& c, int lan
   __syncthreads();  // prologue
   PT_DECL();
   JIT_DECL();
-  const int64_t k_jac = EX ? last_step3(a, c) : -1;
+  const int64_t k_jac = EX ? last_step3<SG>(a, c) : -1;
   int64_t k = 0;
   for (int64_t e = 0; e < a.E; ++e) {
-    const int n = epoch_steps3(a, c, e, k);
+    const int n = epoch_steps3<SG>(a, c, e, k);
     for (int it = 0; it < n; ++it) {
       const int64_t kk = k + it;
 #if !ESKF_OPT_LATEACQ
@@ -860,7 +889,7 @@ __device__ __forceinline__ void role3_jac(const KArgs& a, const Ctx3& c, int lan
           for (int i = 0; i < PK_SIZE; ++i) pk.b[i * F] = po.b[i * F];
         }
         put_notch(sn, notch, dofs);
-        if (EX && a.trace) trace_dofs(a.trace + ((c.f0 + lane) * a.T + kk) * NX, dofs, notch);
+        if (EX && a.trace) trace_dofs(a.trace + ((c.f0 + lane) * a.T + k0_of<SG>(c) + kk) * NX, dofs, notch);
       }
       JIT();
       pk_ready_arrive();  // the CAMERA warp takes rows 18:21 from here
@@ -968,7 +997,7 @@ __device__ __forceinline__ void role3_jac(const KArgs& a, const Ctx3& c, int lan
         for (int i = 0; i < 3; ++i) notch[i] += sx[(SX3_DELTA + 15 + i) * F];
         probe_update_v(a.model, dofs, notch, pkv((int)(k & 1)), trv);
         put_notch((int)(k & 1), notch, dofs);
-        if (EX && a.trace && k > 0) trace_dofs(a.trace + ((c.f0 + lane) * a.T + k - 1) * NX, dofs, notch);
+        if (EX && a.trace && k0_of<SG>(c) + k > 0) trace_dofs(a.trace + ((c.f0 + lane) * a.T + k0_of<SG>(c) + k - 1) * NX, dofs, notch);
       }
       if (EX && a.cons) {  // consistency record: the DOFs after the update (before it, if it was not applied)
 #pragma unroll
@@ -999,7 +1028,7 @@ __device__ __forceinline__ void role3_jac(const KArgs& a, const Ctx3& c, int lan
 
 // ---------------------------------------------------------------------------------------------
 // role 3: sample-stream stager + Monte-Carlo noise
-template <int F, int NTHR, bool EX>
+template <int F, int NTHR, bool EX, bool SG>
 __device__ __forceinline__ void role3_stage(const KArgs& a, const Ctx3& c, int lane) {
   using L = Lay3<F>;
   const bool act = lane < c.nf;
@@ -1038,13 +1067,13 @@ __device__ __forceinline__ void role3_stage(const KArgs& a, const Ctx3& c, int l
   // pre-pass mode: the (noisy) samples of every filter were prepared by eskf_pp_streams_kernel -- same generator, same sums
   const bool noisy = a.noise_on && !(a.noise_free0 && gid == 0) && !a.imu_pf;
   const double* oap = a.imu_pf ? a.imu_pf + (c.f0 + lane) * 6
-                      : a.om_acc ? (a.stream_per_filter ? a.om_acc + (c.f0 + lane) * a.T * 6 : a.om_acc + c.traj * a.T * 6)
+                      : a.om_acc ? (a.stream_per_filter ? a.om_acc + (c.f0 + lane) * a.T * 6 : (SG ? a.om_acc + (c.traj * a.T + c.k0) * 6 : a.om_acc + c.traj * a.T * 6))
                                  : nullptr;
   const int64_t oas = a.imu_pf ? a.N * 6 : 6;  // doubles between consecutive samples of this lane's stream
 #else
   const bool noisy = a.noise_on && !(a.noise_free0 && gid == 0);
   const double* oap =
-      a.om_acc ? (a.stream_per_filter ? a.om_acc + (c.f0 + lane) * a.T * 6 : a.om_acc + c.traj * a.T * 6) : nullptr;
+      a.om_acc ? (a.stream_per_filter ? a.om_acc + (c.f0 + lane) * a.T * 6 : (SG ? a.om_acc + (c.traj * a.T + c.k0) * 6 : a.om_acc + c.traj * a.T * 6)) : nullptr;
   const int64_t oas = 6;
 #endif
 #if ESKF_OPT_TMA
@@ -1056,11 +1085,11 @@ __device__ __forceinline__ void role3_stage(const KArgs& a, const Ctx3& c, int l
   // A buffer is re-filled only after every lane of this warp has passed the scalar barrier that follows its last read.
   uint64_t* chbar = reinterpret_cast<uint64_t*>(c.smem + L::CHBAR);
   double* chunk = c.smem + L::CHUNK;
-  const double* oa0 = a.om_acc ? a.om_acc + c.traj * a.T * 6 : nullptr;
+  const double* oa0 = a.om_acc ? a.om_acc + (c.traj * a.T + k0_of<SG>(c)) * 6 : nullptr;
   const bool tma_pf = a.imu_pf != nullptr && c.nf > 0;
   const bool tma = !tma_pf && oa0 && c.dtp && !a.stream_per_filter && ((reinterpret_cast<uintptr_t>(oa0) & 15) == 0) &&
                    ((reinterpret_cast<uintptr_t>(c.dtp) & 15) == 0);
-  const int64_t n_chunks = tma ? a.T / CH3_STEPS : 0;
+  const int64_t n_chunks = tma ? (a.T - k0_of<SG>(c)) / CH3_STEPS : 0;
   auto issue_chunk = [&](int64_t ch) {
     if (lane == 0 && ch < n_chunks) {
       asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
@@ -1071,7 +1100,7 @@ __device__ __forceinline__ void role3_stage(const KArgs& a, const Ctx3& c, int l
     }
   };
   auto issue_step = [&](int64_t j) {
-    if (lane == 0 && tma_pf && j < a.T) {
+    if (lane == 0 && tma_pf && j < a.T - k0_of<SG>(c)) {
       asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
       const uint32_t bytes = (uint32_t)c.nf * 48u;
       mbar_expect_tx(chbar + (j & 1), bytes);
@@ -1114,7 +1143,7 @@ __device__ __forceinline__ void role3_stage(const KArgs& a, const Ctx3& c, int l
 #endif
     if (noisy) {
       double z[8];
-      normal8(a.seed, (uint64_t)gid, (uint64_t)j, RNG_KIND_IMU, z);
+      normal8(a.seed, (uint64_t)gid, (uint64_t)(k0_of<SG>(c) + j), RNG_KIND_IMU, z);
 #pragma unroll
       for (int i = 0; i < 6; ++i) u[i] += a.imu_noise[i] * z[i];
     }
@@ -1135,14 +1164,14 @@ __device__ __forceinline__ void role3_stage(const KArgs& a, const Ctx3& c, int l
       return;
     }
 #endif
-    const int64_t mrow = a.meas_per_filter ? (c.f0 + lane) : (c.traj * a.E + e);
+    const int64_t mrow = a.meas_per_filter ? (c.f0 + lane) : erow3<SG>(a, c, e);
     double cam[7];
 #pragma unroll
     for (int i = 0; i < 7; ++i) cam[i] = a.cam[mrow * 7 + i];
     double notch = a.notch[mrow];
     if (noisy) {
       double z[8];
-      normal8(a.seed, (uint64_t)gid, (uint64_t)e, RNG_KIND_CAM, z);
+      normal8(a.seed, (uint64_t)gid, (uint64_t)((SG ? a.e_base : 0) + e), RNG_KIND_CAM, z);
       double dth[3];
 #pragma unroll
       for (int i = 0; i < 3; ++i) {
@@ -1176,8 +1205,8 @@ __device__ __forceinline__ void role3_stage(const KArgs& a, const Ctx3& c, int l
     if (!pend) return;
     pend = false;
     const double* xs = a.x + (c.f0 + lane) * NX;
-    const double* ir = a.imu_ref + (c.traj * a.E + se) * 6;
-    const double* cr = a.cam_ref + (c.traj * a.E + se) * 6;
+    const double* ir = a.imu_ref + erow3<SG>(a, c, se) * 6;
+    const double* cr = a.cam_ref + erow3<SG>(a, c, se) * 6;
     double xr[26];
 #pragma unroll
     for (int i = 3; i < 10; ++i) xr[i] = __ldcg(xs + i);
@@ -1198,6 +1227,10 @@ __device__ __forceinline__ void role3_stage(const KArgs& a, const Ctx3& c, int l
     mseB_last = accB;
     mseB_sum += accB;
   };
+  if (act && carry_in3<SG>(a)) {  // a continued trajectory: the running sums so far (kept apart: row [8] adds them only at the end)
+    mseA_sum = carry_in3<SG>(a)[(c.f0 + lane) * ESKF_NCARRY + 0];
+    mseB_sum = carry_in3<SG>(a)[(c.f0 + lane) * ESKF_NCARRY + 1];
+  }
   if (act) {
     const double* ug = a.u + (c.f0 + lane) * 6;
 #pragma unroll
@@ -1208,13 +1241,13 @@ __device__ __forceinline__ void role3_stage(const KArgs& a, const Ctx3& c, int l
   issue_chunk(0);
   issue_step(0);
 #endif
-  if (act && a.T > 0 && oap) stage_sample(0);
+  if (act && a.T - k0_of<SG>(c) > 0 && oap) stage_sample(0);
   __syncthreads();  // prologue
   PT_DECL();
   JIT_DECL();
   int64_t k = 0;
   for (int64_t e = 0; e < a.E; ++e) {
-    const int n = epoch_steps3(a, c, e, k);
+    const int n = epoch_steps3<SG>(a, c, e, k);
     if (act && a.do_update) stage_meas(e);
     const int fl = n < STATS_IT3 ? n : STATS_IT3;
     for (int it = 0;; ++it) {
@@ -1222,7 +1255,7 @@ __device__ __forceinline__ void role3_stage(const KArgs& a, const Ctx3& c, int l
       if (it == fl && act) flush_stats(e - 1);
 #endif
       if (it >= n) break;
-      if (act && k + it + 1 < a.T && ESKF3_SCALAR_ON(it)) stage_sample(k + it + 1);
+      if (act && k + it + 1 < a.T - k0_of<SG>(c) && ESKF3_SCALAR_ON(it)) stage_sample(k + it + 1);
       if (h1s) {
         JIT();
         fx_slot_acquire(c.mbar, k + it);  // the covariance warps are done with the record of step kk - 2
@@ -1274,6 +1307,10 @@ __device__ __forceinline__ void role3_stage(const KArgs& a, const Ctx3& c, int l
     sx[(SX3_ST + 1) * F] = mseA_sum;
     sx[(SX3_ST + 2) * F] = mseB_last;
     sx[(SX3_ST + 3) * F] = mseB_sum;
+    if (carry_out3<SG>(a)) {  // (with the post-pass statistics, pp_stats2_kernel overwrites both after the launch)
+      carry_out3<SG>(a)[(c.f0 + lane) * ESKF_NCARRY + 0] = mseA_sum;
+      carry_out3<SG>(a)[(c.f0 + lane) * ESKF_NCARRY + 1] = mseB_sum;
+    }
   }
   __syncthreads();
   store_tiles3<F, NTHR>(a, c, threadIdx.x);
@@ -1393,7 +1430,7 @@ __device__ __forceinline__ bool inv7_group3(double* rec, int g, const double* rd
 #define COV3_SYNCWARP() __syncwarp(gmask)
 #endif
 
-template <int F, int NTHR, bool EX>
+template <int F, int NTHR, bool EX, bool SG>
 __device__ __forceinline__ void role3_cov(const KArgs& a, const Ctx3& c, int ct) {
   using L = Lay3<F>;
   const int cf = ct >> 3;  // filter of this lane (padded filters run on an identity tile, never stored)
@@ -1461,7 +1498,7 @@ __device__ __forceinline__ void role3_cov(const KArgs& a, const Ctx3& c, int ct)
 
   int64_t k = 0;
   for (int64_t e = 0; e < a.E; ++e) {
-    const int n = epoch_steps3(a, c, e, k);
+    const int n = epoch_steps3<SG>(a, c, e, k);
     PT_MARK(15);
     JIT();
     if (n > 0) fx_slot_wait(c.mbar, k);  // the Jacobian record of the first step of the epoch is complete
@@ -1684,11 +1721,12 @@ __device__ __forceinline__ void role3_cov(const KArgs& a, const Ctx3& c, int ct)
 
 // ---------------------------------------------------------------------------------------------
 // MODE: bit 0 = export mode (FilterTraj rows, Jacobian record of the last step, consistency records), bit 1 = stacked
-// trajectories.  Separate instantiations, so that the production kernel of a single-trajectory batch carries neither (a few
-// integer instructions in the prologue are enough to change the register allocation of the whole kernel).
+// trajectories, bit 2 = a segment of the trajectory (eskf_run_epochs: KArgs::k_base, e_base, E_all, carry_in / carry_out).
+// Separate instantiations, so that the production kernel of a single-trajectory batch carries none of them (a few integer
+// instructions in the prologue are enough to change the register allocation of the whole kernel).
 template <int F, int REG_S, int REG_C, int MODE>
 __global__ void __launch_bounds__(128 + 8 * F, 1) eskf_kernel3(const __grid_constant__ KArgs a) {
-  constexpr bool EX = (MODE & 1) != 0, MT = (MODE & 2) != 0;
+  constexpr bool EX = (MODE & 1) != 0, MT = (MODE & 2) != 0, SG = (MODE & 4) != 0;
   extern __shared__ __align__(16) double smem[];
   using L = Lay3<F>;
   constexpr int NTHR = 128 + 8 * F;
@@ -1706,8 +1744,15 @@ __global__ void __launch_bounds__(128 + 8 * F, 1) eskf_kernel3(const __grid_cons
   }
   c.gid0 = a.filter_id0 + c.f0;
   c.traj = (a.n_traj > 1) ? (c.gid0 / a.filters_per_traj) : 0;
-  c.n_prop = a.n_prop ? a.n_prop + c.traj * a.E : nullptr;
-  c.dtp = a.dt ? a.dt + c.traj * a.T : nullptr;
+  if constexpr (SG) {  // a segment: each CTA rebases onto its trajectory's first step and the segment's first epoch
+    c.k0 = a.k_base[c.traj];
+    c.n_prop = a.n_prop ? a.n_prop + c.traj * a.E_all + a.e_base : nullptr;
+    c.dtp = a.dt ? a.dt + c.traj * a.T + c.k0 : nullptr;
+  } else {
+    c.k0 = 0;
+    c.n_prop = a.n_prop ? a.n_prop + c.traj * a.E : nullptr;
+    c.dtp = a.dt ? a.dt + c.traj * a.T : nullptr;
+  }
   c.mbar = reinterpret_cast<uint64_t*>(smem + L::MBAR);
   if (tid == 0) {
     mbar_init(c.mbar + 0, 3);      // full[s]:  the IMU, the CAMERA and the JACOB warp (rows 3:9, 18:21, 21:24)
@@ -1739,19 +1784,19 @@ __global__ void __launch_bounds__(128 + 8 * F, 1) eskf_kernel3(const __grid_cons
   // sub-partition -- a remapping that put two scalar roles on the sub-partition with the single covariance warp hung)
   if (warp >= 4) {
     reg_inc3<REG_C>();
-    role3_cov<F, NTHR, EX>(a, c, tid - 128);
+    role3_cov<F, NTHR, EX, SG>(a, c, tid - 128);
   } else {
     // (ptxas 12.9 crashes on kernels with more than one setmaxnreg.dec value, so all four scalar roles
     // share REG_S although the Jacobian warp's sub-partition would have room for more)
     reg_dec3<REG_S>();
     if (warp == 0)
-      role3_imu<F, NTHR, EX>(a, c, lane);
+      role3_imu<F, NTHR, EX, SG>(a, c, lane);
     else if (warp == 1)
-      role3_cam<F, NTHR, EX>(a, c, lane);
+      role3_cam<F, NTHR, EX, SG>(a, c, lane);
     else if (warp == 2)
-      role3_stage<F, NTHR, EX>(a, c, lane);
+      role3_stage<F, NTHR, EX, SG>(a, c, lane);
     else
-      role3_jac<F, NTHR, EX>(a, c, lane);
+      role3_jac<F, NTHR, EX, SG>(a, c, lane);
   }
 }
 

@@ -32,12 +32,17 @@ cudaError_t launch_eskf_kernel3<ESKF_F>(const KArgs& a, cudaStream_t stream) {
   static_assert(smem <= 232448, "shared memory per CTA");
   // export mode (FilterTraj rows, eskf_streams_t.trace_x; Jacobian record of the last step, eskf_keep_jacobians; consistency
   // records, eskf_keep_consistency) and the CTA mapping of stacked trajectories are separate instantiations: the production
-  // kernel of a single-trajectory batch carries none of their code (the dump alone cost 10 % through register allocation)
-  const int mode = ((a.trace || a.fx_dump || a.cons) ? 1 : 0) | (a.n_traj > 1 ? 2 : 0);
+  // kernel of a single-trajectory batch carries none of their code (the dump alone cost 10 % through register allocation).
+  // A segment of the trajectory (eskf_run_epochs) is a third bit: eskf_run keeps the kernels it had.
+  const int mode = ((a.trace || a.fx_dump || a.cons) ? 1 : 0) | (a.n_traj > 1 ? 2 : 0) | (a.k_base ? 4 : 0);
   auto kern = mode == 0   ? eskf_kernel3<F, ESKF_REG_S, ESKF_REG_C, 0>
               : mode == 1 ? eskf_kernel3<F, ESKF_REG_S, ESKF_REG_C, 1>
               : mode == 2 ? eskf_kernel3<F, ESKF_REG_S, ESKF_REG_C, 2>
-                          : eskf_kernel3<F, ESKF_REG_S, ESKF_REG_C, 3>;
+              : mode == 3 ? eskf_kernel3<F, ESKF_REG_S, ESKF_REG_C, 3>
+              : mode == 4 ? eskf_kernel3<F, ESKF_REG_S, ESKF_REG_C, 4>
+              : mode == 5 ? eskf_kernel3<F, ESKF_REG_S, ESKF_REG_C, 5>
+              : mode == 6 ? eskf_kernel3<F, ESKF_REG_S, ESKF_REG_C, 6>
+                          : eskf_kernel3<F, ESKF_REG_S, ESKF_REG_C, 7>;
   cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return e;
   // (stacked trajectories: ceil(fpt / F) CTAs per trajectory, fewer for a partially covered last one: stacked_grid)

@@ -16,7 +16,7 @@ from typing import Optional, Sequence
 import numpy as np
 
 from . import _lib
-from ._lib import MEM_DEVICE, MEM_HOST, NCONS, NDOFSUM, NSTAT, EskfModel, EskfStreams, check
+from ._lib import MEM_DEVICE, MEM_HOST, NCARRY, NCONS, NDOFSUM, NSTAT, EskfModel, EskfStreams, check
 
 
 def _is_torch(a) -> bool:
@@ -66,12 +66,17 @@ def _common_mem(args: Sequence[_Arg]) -> int:
 
 
 def check_run_geometry(n_filters: int, n_traj: int, filters_per_traj: int, filter_id0: int, n_steps: int, n_epochs: int,
-                       n_prop=None) -> None:
-    """The argument checks of ``eskf_run`` (csrc/eskf_api.cu), mirrored on the host so that a bad shard plan fails with a
-    clear ``ValueError`` before anything is launched: the kernels pick a filter's trajectory from its GLOBAL id,
-    ``(filter_id0 + f) // filters_per_traj``, and the sample stream by the running sum of ``n_prop``."""
+                       n_prop=None, epochs=None) -> None:
+    """The argument checks of ``eskf_run`` / ``eskf_run_epochs`` (csrc/eskf_api.cu), mirrored on the host so that a bad shard
+    plan or epoch range fails with a clear ``ValueError`` before anything is launched: the kernels pick a filter's trajectory
+    from its GLOBAL id, ``(filter_id0 + f) // filters_per_traj``, and the sample stream by the running sum of ``n_prop``;
+    ``epochs = (e0, e1)`` must satisfy 0 <= e0 <= e1 <= n_epochs."""
     if n_filters <= 0 or n_traj < 1 or n_steps < 0 or n_epochs < 0:
         raise ValueError("n_filters, n_traj must be positive and n_steps, n_epochs non-negative")
+    if epochs is not None:
+        e0, e1 = (int(v) for v in epochs)
+        if not 0 <= e0 <= e1 <= n_epochs:
+            raise ValueError(f"epoch range [{e0}, {e1}) is not within [0, n_epochs = {n_epochs}]")
     if filter_id0 < 0:
         raise ValueError("filter_id0 must be non-negative")
     if n_traj > 1:
@@ -89,6 +94,17 @@ def check_run_geometry(n_filters: int, n_traj: int, filters_per_traj: int, filte
         tot = npr.sum(axis=1)
         if (tot > n_steps).any():
             raise ValueError(f"sum(n_prop) = {int(tot.max())} exceeds n_steps = {n_steps}")
+
+
+def segment_steps(n_prop, n_steps: int, e0: int, e1: int):
+    """(k0, k1), each [n_traj]: the global steps at which every trajectory's epochs e0 and e1 start, as the kernels count
+    them -- the running sum of n_prop with every epoch clamped to what is left of the n_steps-long stream (a negative entry
+    counts 0).  A segment ``run(..., epochs=(e0, e1))`` executes steps [k0[t], k1[t]) of trajectory t and writes those
+    trace rows.  ``n_prop`` is [E] or [n_traj, E]."""
+    npr = np.atleast_2d(np.asarray(n_prop, dtype=np.int64))
+    c = np.minimum(np.cumsum(np.maximum(npr, 0), axis=1), n_steps)  # the clamped running sum saturates at n_steps
+    c = np.hstack((np.zeros((len(npr), 1), dtype=np.int64), c))
+    return c[:, e0].copy(), c[:, e1].copy()
 
 
 class BatchFilter:
@@ -110,6 +126,7 @@ class BatchFilter:
         h = C.c_void_p()
         check(self._lib.eskf_create(C.byref(m), self.n, self.device, C.c_void_p(stream), C.byref(h)), "eskf_create")
         self._h = h
+        self.last_carry = None  # carry returned by the last run(..., epochs=...)
         if variant is None:
             variant = int(os.environ.get("ESKF_B200_VARIANT", "0"))
         if variant:
@@ -214,13 +231,19 @@ class BatchFilter:
     def run(self, dt, om_acc, n_prop, cam, notch, cam_ref=None, imu_ref=None, gt_dofs=(0, 0, 0, 0, 0, 20.0),
             n_traj: int = 1, filters_per_traj: Optional[int] = None, seed: int = 0, filter_id0: int = 0,
             imu_noise_std=None, cam_noise_std=None, noise_free_filter0: bool = True, want_stats: bool = True,
-            stats_on_device: bool = False, trace=None, noise_id_modulus: int = 0):
+            stats_on_device: bool = False, trace=None, noise_id_modulus: int = 0, epochs=None, carry=None):
         """``Filter.run`` (Filter.py:144-185) for every filter, in one persistent kernel.
         Returns (stats [N,16], stats_sum [16]) (see include/eskf.h) or None.
         ``trace``: optional [N,T,26] float64 array (numpy for host streams, CUDA tensor for device streams) that
         receives the nominal state after every IMU step, updated state at the update instants (FilterTraj rows).
         ``noise_id_modulus`` r > 0: the noise of global filter g is that of id g % r (common random numbers for
-        groups of r filters that differ only by their parameters)."""
+        groups of r filters that differ only by their parameters).
+        ``epochs = (e0, e1)``: only epochs [e0, e1) of the trajectory passed (the whole one, not a slice), continuing from the
+        current state (eskf_run_epochs, include/eskf.h); returns (stats, stats_sum, carry), stats over epochs [0, e1), None
+        without ``want_stats`` and for an empty range (which runs nothing).  ``carry`` [N,4] (the running update-MSE sums, applied updates and status word) comes
+        from the previous segment's return value, None to start fresh; it and the returned one live where the statistics
+        do (numpy, or CUDA tensors with ``stats_on_device``), and the returned one is also kept as ``last_carry``.  Segments
+        run back to back give bit for bit what one run gives; a checkpoint is ``get_state()``, the carry and e1."""
         adt = _Arg(dt, None, name="dt")
         anp = _Arg(n_prop, None, dtype=np.int32, name="n_prop")
         T = adt.rows // n_traj
@@ -231,7 +254,7 @@ class BatchFilter:
             raise ValueError("stream shapes do not match (n_traj, T, E)")
         mem = _common_mem([adt, anp, aoa, acm, ano, acr, air])
         check_run_geometry(self.n, n_traj, int(filters_per_traj if filters_per_traj else self.n), int(filter_id0), T, E,
-                           n_prop if isinstance(n_prop, np.ndarray) else None)
+                           n_prop if isinstance(n_prop, np.ndarray) else None, epochs)
         s = EskfStreams()
         s.n_steps, s.n_epochs, s.n_traj, s.mem = T, E, n_traj, mem
         s.filters_per_traj = int(filters_per_traj if filters_per_traj else self.n)
@@ -252,6 +275,8 @@ class BatchFilter:
             if atr.mem != mem:
                 raise ValueError("trace must live where the streams live (host numpy / CUDA tensor)")
             s.trace_x = atr.ptr
+        if epochs is not None:
+            return self._run_epochs(s, int(epochs[0]), int(epochs[1]), carry, want_stats, stats_on_device)
         if not want_stats:
             check(self._lib.eskf_run(self._h, C.byref(s), None, None, MEM_HOST), "eskf_run")
             return None
@@ -269,6 +294,43 @@ class BatchFilter:
         check(self._lib.eskf_run(self._h, C.byref(s), st.ctypes.data_as(C.c_void_p), sm.ctypes.data_as(C.c_void_p), MEM_HOST),
               "eskf_run")
         return st, sm
+
+    def _run_epochs(self, s, e0: int, e1: int, carry, want_stats: bool, on_device: bool):
+        """eskf_run_epochs with the streams ``s``: (stats, stats_sum, carry) in host or device memory"""
+        if on_device:
+            import torch
+
+            dev = torch.device("cuda", self.device)
+            new = lambda shape: torch.empty(shape, dtype=torch.float64, device=dev)
+            ptr = lambda a: C.c_void_p(a.data_ptr())
+            mem = MEM_DEVICE
+            if carry is not None:
+                carry = torch.as_tensor(carry, dtype=torch.float64, device=dev).contiguous()
+        else:
+            new, ptr, mem = np.empty, (lambda a: a.ctypes.data_as(C.c_void_p)), MEM_HOST
+            if carry is not None:
+                carry = np.ascontiguousarray(carry.cpu().numpy() if _is_torch(carry) else carry, dtype=np.float64)
+        if carry is not None and tuple(carry.shape) != (self.n, NCARRY):
+            raise ValueError(f"carry must have shape {(self.n, NCARRY)}")
+        st, sm = (new((self.n, NSTAT)), new((NSTAT,))) if want_stats and e1 > e0 else (None, None)  # (empty: not written)
+        out = new((self.n, NCARRY))
+        arg = lambda a: None if a is None else ptr(a)
+        check(self._lib.eskf_run_epochs(self._h, C.byref(s), e0, e1, arg(carry), ptr(out), arg(st), arg(sm), mem), "eskf_run_epochs")
+        self.last_carry = out
+        return st, sm, out
+
+    def run_segments(self, dt, om_acc, n_prop, cam, notch, boundaries, carry=None, **kw):
+        """Generator: the trajectory in segments [boundaries[i], boundaries[i + 1]) (``run`` with ``epochs``), yielding
+        (e0, e1, stats, stats_sum) after each one, the carry threaded from one to the next (``last_carry`` holds the latest:
+        with ``get_state()`` and e1 it is the checkpoint to continue from).  The caller may inspect the state, checkpoint or
+        stop between segments; a generator that is not resumed runs nothing more, so the handle keeps the state of the last
+        finished segment.  ``kw`` are the keyword arguments of ``run``."""
+        b = [int(v) for v in boundaries]
+        if len(b) < 2 or any(x > y for x, y in zip(b, b[1:])):
+            raise ValueError("boundaries must be at least two non-decreasing epoch indices")
+        for e0, e1 in zip(b, b[1:]):
+            st, sm, carry = self.run(dt, om_acc, n_prop, cam, notch, epochs=(e0, e1), carry=carry, **kw)
+            yield e0, e1, st, sm
 
     def sync(self):
         check(self._lib.eskf_sync(self._h), "eskf_sync")

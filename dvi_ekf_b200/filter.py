@@ -450,13 +450,16 @@ class Simulator:
     def reset_kf(self) -> None:
         self.kf = Filter(self)
 
-    def run(self, disp_config=False, save_best=False, verbose=True, n_filters: Optional[int] = None, consistency: bool = False):
+    def run(self, disp_config=False, save_best=False, verbose=True, n_filters: Optional[int] = None, consistency: bool = False,
+            segment_epochs: Optional[int] = None):
         """Simulator.run (Simulator.py:121-158) as ONE batched launch: ``num_kf_runs`` (or ``n_filters``)
         independent filters, run 0 noise free (the reference's deterministic run), the others with
         Monte-Carlo IMU / camera noise and DOF initial-condition perturbations (``batch:`` section).
         ``consistency``: ``self.consistency`` becomes ``consistency.summarise_consistency`` of the run (ANIS / ANEES per
         epoch and their chi-square intervals), ``self.dof_envelope`` ``consistency.summarise_dofs`` of it (bias, RMSE,
-        claimed sigma, inflation, per-DOF ANEES and coverage per DOF and epoch)."""
+        claimed sigma, inflation, per-DOF ANEES and coverage per DOF and epoch).
+        ``segment_epochs`` k: the same run in launches of k epochs (``BatchFilter.run_segments``), with the same results; the
+        consistency records then take the memory of k epochs, not of the whole run, and their per-epoch rows are joined."""
         cfg, s = self.config, self.streams
         n = int(n_filters or self.num_kf_runs)
         b = cfg.batch
@@ -473,12 +476,28 @@ class Simulator:
                 bf.keep_consistency()
             imu_std = np.hstack((cfg.imu.stdev_omega, cfg.imu.stdev_accel)) if b.imu_noise else None
             cam_std = np.array(cfg.meas_noise_std) if b.cam_noise else None
-            st, sm = bf.run(s.dt, s.om_acc, s.n_prop, s.cam, s.notch, cam_ref=s.cam_ref, imu_ref=s.imu_ref,
-                            gt_dofs=cfg.gt_imu_dofs, seed=b.seed, imu_noise_std=imu_std, cam_noise_std=cam_std)
+            kw = dict(cam_ref=s.cam_ref, imu_ref=s.imu_ref, gt_dofs=cfg.gt_imu_dofs, seed=b.seed, imu_noise_std=imu_std,
+                      cam_noise_std=cam_std)
+            E = len(s.n_prop)
+            if segment_epochs and E:
+                k = int(segment_epochs)
+                if k <= 0:
+                    raise ValueError("segment_epochs must be positive")
+                esum, env = [], []
+                for _, _, st, sm in bf.run_segments(s.dt, s.om_acc, s.n_prop, s.cam, s.notch, [*range(0, E, k), E], **kw):
+                    if consistency:  # per-epoch rows: joining the segments' rows is exact
+                        esum.append(bf.get_consistency()[2])
+                        env.append(bf.get_dof_envelope())
+                if consistency:
+                    esum, env = np.concatenate(esum), np.concatenate(env)
+            else:
+                st, sm = bf.run(s.dt, s.om_acc, s.n_prop, s.cam, s.notch, **kw)
+                if consistency:
+                    esum, env = bf.get_consistency()[2], bf.get_dof_envelope()
             self.final_states = bf.get_state()[0]
             if consistency:
-                self.consistency = summarise_consistency(bf.get_consistency()[2], 6 - sum(1 for f in cfg.frozen_dofs if f))
-                self.dof_envelope = summarise_dofs(bf.get_dof_envelope(), cfg.frozen_dofs)
+                self.consistency = summarise_consistency(esum, 6 - sum(1 for f in cfg.frozen_dofs if f))
+                self.dof_envelope = summarise_dofs(env, cfg.frozen_dofs)
         self.stats = st
         # Simulator.py:138-158 appends ``kf.mse`` of every run -- which is 0 at the reference's HEAD, because the call that
         # would set it is commented out (Filter.py:92,167-168).  ``mses`` / ``mse_best`` / ``mse_avg`` keep exactly that

@@ -125,6 +125,38 @@ int eskf_update(eskf_t* h, const double* cam, const double* notch, int per_filte
  * handle's filters, the vector a multi-GPU launcher all-reduces). */
 int eskf_run(eskf_t* h, const eskf_streams_t* streams, double* stats_out, double* stats_sum, int mem);
 
+#define ESKF_NCARRY 4
+/* Epochs [epoch_begin, epoch_end) of the trajectory in `streams` (no reference counterpart), continuing from the handle's state:
+ * a run in segments, with control between them, bit-identical to one eskf_run.  `streams` is the WHOLE trajectory eskf_run
+ * takes, not a slice: trajectory t starts at step k0[t] = sum over e < epoch_begin of n_prop[t, e] (clamped to n_steps as the
+ * kernels clamp every epoch), the Monte-Carlo noise is drawn by global step and epoch, and the references, the trace rows and
+ * the per-epoch streams are read at their global rows.
+ *   carry_in / carry_out: NULL or [N,ESKF_NCARRY] in `mem` space (they may be the same array), the per-filter accumulators the
+ *     statistics row cannot hold without loss: [0] and [1] the two running squared-error sums of Filter.calculate_update_mse
+ *     (row [8] is (sum0 + sum1) / 12), [2] the applied updates, [3] the status word.  carry_in = NULL continues with zero
+ *     sums from the handle's status word, as eskf_run does; otherwise the sums start from it and the status word is set from
+ *     [3], so that its sticky bits survive eskf_set_state on a new handle.  The checkpoint of a run is eskf_get_state +
+ *     carry_out + epoch_end: enough to continue in another process, on another handle or on another GPU.
+ *   stats_out / stats_sum: as for eskf_run, accumulated over epochs [0, epoch_end); row [7] is the update MSE of epoch
+ *     epoch_end - 1.  After the last segment every column is bit-identical to the one-launch run.
+ *   trace_x: the rows of the segment's steps are written at their global step rows of [N,T,26] (and, where the segment
+ *     begins with epochs of 0 steps, the row before them, which their updates overwrite as in one launch); the other rows
+ *     keep the caller's content.  A host trace is staged whole (N * T * 208 bytes of device memory), as for eskf_run.
+ *   Jacobian record (eskf_keep_jacobians): the last step the segment executes.
+ *   Consistency (eskf_keep_consistency) and the per-DOF getters cover the segment: *n_epochs = epoch_end - epoch_begin, row k
+ *     is global epoch epoch_begin + k, bit-identical to that row of the whole run; the records and the ESKF_ENOMEM check are
+ *     sized by the segment (N * (epoch_end - epoch_begin) * 352 bytes).
+ *   Pre-pass budget (eskf_set_prepass_budget): sized by the segment's steps and epochs, so a segment can take the pre-pass
+ *     path where the whole run would not.  With device-resident streams the segment's step counts are read back to size it
+ *     (a small copy that makes the call synchronous); only when noise is on and a pre-pass is possible.
+ * Rules: 0 <= epoch_begin <= epoch_end <= n_epochs, otherwise ESKF_EINVAL; variant 1 (eskf_kernel): ESKF_EINVAL.  An empty
+ * range (epoch_begin == epoch_end) launches nothing and changes nothing on the handle except that the consistency getters
+ * then report zero epochs (with eskf_keep_consistency on); it copies carry_in to carry_out (zeros without carry_in) and does
+ * NOT write stats_out / stats_sum.  A refused call leaves the handle unchanged.  eskf_run(h, s, ...) with n_epochs > 0 is
+ * eskf_run_epochs(h, s, 0, n_epochs, NULL, NULL, ...). */
+int eskf_run_epochs(eskf_t* h, const eskf_streams_t* streams, int64_t epoch_begin, int64_t epoch_end, const double* carry_in,
+                    double* carry_out, double* stats_out, double* stats_sum, int mem);
+
 /* Filter._states / _P / buffers read-back.  Any pointer may be NULL. */
 int eskf_get_state(eskf_t* h, double* x, double* P, double* u_old, double* R_old, int32_t* status, int mem);
 
