@@ -284,15 +284,31 @@ __global__ void __launch_bounds__(256) seg_base_kernel(const int32_t* __restrict
 // whatever the CTA scheduling) and MASKED: a filter that diverged (non-finite row) or whose status word is set would
 // otherwise turn the reduced vector of a million healthy filters into NaN.  [0:10] sums over the healthy filters,
 // [10] filters with a non-zero status, [11] healthy filters (the divisor of every mean), [12] non-finite filters.
+// Every reduction of the rows or of the consistency records takes its blocks from a GroupMap (eskf_set_groups): with one
+// group, ceil(N / RED_ROWS) blocks of RED_ROWS rows, the ungrouped sums; with groups, per group (group_block, eskf_math.cuh),
+// and the final kernels add the blocks of each group in order.  The same fixed trees either way.
 constexpr int RED_ROWS = 4096;  // rows per block
-__global__ void stats_partial_kernel(const double* __restrict__ rows, const int32_t* __restrict__ status, int64_t n,
+struct GroupMap {
+  int64_t N, id0, g;  // filters, global id of the first one, group size (0: one group)
+  int64_t G, nblk;    // local groups, reduction blocks
+};
+__host__ __device__ inline GroupMap group_map(int64_t N, int64_t id0, int64_t g) {
+  return GroupMap{N, id0, g, g > 0 ? (id0 + N - 1) / g - id0 / g + 1 : 1, group_blocks(N, id0, g, RED_ROWS)};
+}
+// the blocks b0 .. b1 - 1 of local group k
+__device__ __forceinline__ void group_range(const GroupMap& m, int64_t k, int64_t& b0, int64_t& b1) {
+  b0 = group_blocks(group_row0(k, m.N, m.id0, m.g), m.id0, m.g, RED_ROWS);
+  b1 = group_blocks(group_row0(k + 1, m.N, m.id0, m.g), m.id0, m.g, RED_ROWS);
+}
+__global__ void stats_partial_kernel(const double* __restrict__ rows, const int32_t* __restrict__ status, const GroupMap m,
                                      double* __restrict__ partial) {
   __shared__ double sh[256][13];
-  const int64_t r0 = (int64_t)blockIdx.x * RED_ROWS;
+  int64_t r0, r1, k;
+  group_block(blockIdx.x, m.N, m.id0, m.g, RED_ROWS, r0, r1, k);
   double acc[13];
 #pragma unroll
   for (int i = 0; i < 13; ++i) acc[i] = 0.0;
-  for (int64_t r = r0 + threadIdx.x; r < r0 + RED_ROWS && r < n; r += 256) {
+  for (int64_t r = r0 + threadIdx.x; r < r1; r += 256) {
     const double* row = rows + r * ESKF_NSTAT;
     double v[10], chk = 0.0;
 #pragma unroll
@@ -321,11 +337,15 @@ __global__ void stats_partial_kernel(const double* __restrict__ rows, const int3
   }
   if (threadIdx.x < ESKF_NSTAT) partial[(int64_t)blockIdx.x * ESKF_NSTAT + threadIdx.x] = threadIdx.x < 13 ? sh[0][threadIdx.x] : 0.0;
 }
-__global__ void stats_final_kernel(const double* __restrict__ partial, int64_t nblk, double* __restrict__ out) {
-  if (threadIdx.x >= ESKF_NSTAT) return;
+// out [G][ESKF_NSTAT]: the blocks of each group added in order
+__global__ void stats_final_kernel(const double* __restrict__ partial, const GroupMap m, double* __restrict__ out) {
+  const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x, k = idx / ESKF_NSTAT, i = idx - k * ESKF_NSTAT;
+  if (k >= m.G) return;
+  int64_t b0, b1;
+  group_range(m, k, b0, b1);
   double a = 0.0;
-  for (int64_t b = 0; b < nblk; ++b) a += partial[b * ESKF_NSTAT + threadIdx.x];
-  out[threadIdx.x] = a;
+  for (int64_t b = b0; b < b1; ++b) a += partial[b * ESKF_NSTAT + i];
+  out[idx] = a;
 }
 
 // ---- filter consistency (eskf_keep_consistency): post-pass over the records the export instantiation filed ------------
@@ -358,19 +378,20 @@ __global__ void cons_eval_kernel(double* __restrict__ rec, double* __restrict__ 
   r[CONS_NEES * p.N] = ve;
 }
 
-// epoch_sum [E][ESKF_NCONS], deterministically like stats_sum: block b of epoch e sums the finite values of filters
-// b RED_ROWS .. (b + 1) RED_ROWS - 1 through a fixed tree, cons_final_kernel adds the blocks of an epoch in order.
+// epoch_sum [E][ESKF_NCONS], deterministically like stats_sum: block b of epoch e sums the finite values of the filters of
+// block b of the map through a fixed tree, cons_final_kernel adds the blocks of an epoch (of each group) in order.
 // [0] finite NIS, [1] sum, [2] sum of squares, [3..5] the same for the NEES, [6] filters whose NIS or (d > 0) NEES is NaN.
-__global__ void cons_partial_kernel(const double* __restrict__ rec, int64_t N, int64_t nblk, int with_nees,
-                                    double* __restrict__ partial) {
+__global__ void cons_partial_kernel(const double* __restrict__ rec, const GroupMap m, int with_nees, double* __restrict__ partial) {
   __shared__ double sh[256][7];
-  const int64_t e = blockIdx.x / nblk, b = blockIdx.x - e * nblk;
+  const int64_t N = m.N, e = blockIdx.x / m.nblk, b = blockIdx.x - e * m.nblk;
+  int64_t r0, r1, k;
+  group_block(b, N, m.id0, m.g, RED_ROWS, r0, r1, k);
   const double* vn = rec + e * CONS_SIZE * N + CONS_NIS * N;
   const double* ve = rec + e * CONS_SIZE * N + CONS_NEES * N;
   double acc[7];
 #pragma unroll
   for (int i = 0; i < 7; ++i) acc[i] = 0.0;
-  for (int64_t r = b * RED_ROWS + threadIdx.x; r < (b + 1) * RED_ROWS && r < N; r += 256) {
+  for (int64_t r = r0 + threadIdx.x; r < r1; r += 256) {
     const double a = vn[r], c = ve[r];
     const bool fa = isfinite(a), fc = isfinite(c);
     if (fa) {
@@ -395,16 +416,18 @@ __global__ void cons_partial_kernel(const double* __restrict__ rec, int64_t N, i
     }
     __syncthreads();
   }
-  if (threadIdx.x < ESKF_NCONS) partial[blockIdx.x * ESKF_NCONS + threadIdx.x] = threadIdx.x < 7 ? sh[0][threadIdx.x] : 0.0;
+  if (threadIdx.x < ESKF_NCONS) partial[(int64_t)blockIdx.x * ESKF_NCONS + threadIdx.x] = threadIdx.x < 7 ? sh[0][threadIdx.x] : 0.0;
 }
-// out [E][width] from the partial rows [E][nblk][width] of cons_partial_kernel (width ESKF_NCONS) or dof_partial_kernel
-// (ESKF_NDOFSUM): the blocks of an epoch added in order
-__global__ void cons_final_kernel(const double* __restrict__ partial, int64_t nblk, int64_t E, int width, double* __restrict__ out) {
+// out [G][E][width] from the partial rows [E][nblk][width] of cons_partial_kernel (width ESKF_NCONS) or dof_partial_kernel
+// (ESKF_NDOFSUM): the blocks of an epoch and group added in order
+__global__ void cons_final_kernel(const double* __restrict__ partial, const GroupMap m, int64_t E, int width, double* __restrict__ out) {
   const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (idx >= E * width) return;
-  const int64_t e = idx / width, i = idx - e * width;
+  if (idx >= m.G * E * width) return;
+  const int64_t k = idx / (E * width), e = (idx - k * E * width) / width, i = idx - (k * E + e) * width;
+  int64_t b0, b1;
+  group_range(m, k, b0, b1);
   double a = 0.0;
-  for (int64_t b = 0; b < nblk; ++b) a += partial[(e * nblk + b) * width + i];
+  for (int64_t b = b0; b < b1; ++b) a += partial[(e * m.nblk + b) * width + i];
   out[idx] = a;
 }
 
@@ -444,30 +467,32 @@ __global__ void __launch_bounds__(256) dof_history_kernel(const double* __restri
 }
 
 // dof_partial_kernel: the envelope rows [E][ESKF_NDOFSUM] deterministically, as cons_partial_kernel does the epoch sums:
-// block b of epoch e takes filters b RED_ROWS .. (b + 1) RED_ROWS - 1.  Each filter's DSUM_USED terms (dof_terms) do not fit
+// block b of epoch e takes the filters of block b of the map.  Each filter's DSUM_USED terms (dof_terms) do not fit
 // a per-thread accumulator, so every warp reduces the terms of its 32 filters at once, over fixed trees: recursive halving
 // over the lanes for each full group of 32 columns (after five exchange steps lane l holds the warp's sum of column
 // 32 g + l), an xor butterfly for each of the remaining columns (lane c - 64 keeps column c).  Every lane accumulates its
 // columns over the warp's rows in order, and the eight warps are added in order at the end.  cons_final_kernel adds the
 // blocks.
-__global__ void __launch_bounds__(256) dof_partial_kernel(const double* __restrict__ rec, const ConsArgs p, int64_t nblk,
+__global__ void __launch_bounds__(256) dof_partial_kernel(const double* __restrict__ rec, const ConsArgs p, const GroupMap m,
                                                           double* __restrict__ partial) {
   constexpr int NG = DSUM_USED / 32;  // full column groups; the tail DSUM_USED - 32 NG < 32 columns
   static_assert(DSUM_USED - 32 * NG < 32, "tail");
   __shared__ double sh[8][32 * (NG + 1)];
-  const int64_t e = blockIdx.x / nblk, b = blockIdx.x - e * nblk;
+  const int64_t e = blockIdx.x / m.nblk, b = blockIdx.x - e * m.nblk;
   const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-  const int64_t r1 = (b + 1) * RED_ROWS < p.N ? (b + 1) * RED_ROWS : p.N;
-  const double* re = rec + e * CONS_SIZE * p.N;
+  int64_t rb, r1, k;
+  group_block(b, m.N, m.id0, m.g, RED_ROWS, rb, r1, k);
+  const double* re = rec + e * CONS_SIZE * p.N + rb;  // (rows counted from the block's first one)
+  const int nr = (int)(r1 - rb);
   double acc[NG + 1];
 #pragma unroll
   for (int g = 0; g <= NG; ++g) acc[g] = 0.0;
-  for (int64_t r0 = b * RED_ROWS + 32 * w; r0 < r1; r0 += 256) {  // (warp-uniform)
-    const int64_t r = r0 + lane;
+  for (int r0 = 32 * w; r0 < nr; r0 += 256) {  // (warp-uniform)
+    const int r = r0 + lane;
     double t[DSUM_USED];
 #pragma unroll
     for (int c = 0; c < DSUM_USED; ++c) t[c] = 0.0;
-    if (r < r1) {
+    if (r < nr) {
       double eps[6];
 #pragma unroll
       for (int i = 0; i < 6; ++i) eps[i] = re[(CONS_DOFS + i) * p.N + r] - p.gt[i];
@@ -503,7 +528,7 @@ __global__ void __launch_bounds__(256) dof_partial_kernel(const double* __restri
     double a = 0.0;
     if (threadIdx.x < DSUM_USED)
       for (int k = 0; k < 8; ++k) a += sh[k][threadIdx.x];
-    partial[blockIdx.x * ESKF_NDOFSUM + threadIdx.x] = a;
+    partial[(int64_t)blockIdx.x * ESKF_NDOFSUM + threadIdx.x] = a;
   }
 }
 static_assert(DSUM_USED <= ESKF_NDOFSUM && ESKF_NDOFSUM <= 256, "envelope row");
@@ -568,8 +593,8 @@ struct NvtxRange {
 
 // ---------------------------------------------------------------------------------------------
 // 0..8: arguments / results of the calls; 9..11: pre- / post-pass buffers of eskf_run; 12: partial sums; 13: first steps of a
-// segment (seg_base_kernel); 14, 15: host carry of eskf_run_epochs
-constexpr int N_STAGE = 16;
+// segment (seg_base_kernel); 14, 15: host carry of eskf_run_epochs; 16: partial sums of the grouped statistics
+constexpr int N_STAGE = 17;
 struct eskf_handle {
   int device = 0;
   cudaStream_t stream = nullptr;
@@ -595,6 +620,14 @@ struct eskf_handle {
   double *cons_rec = nullptr, *cons_out = nullptr;
   size_t cons_rec_sz = 0, cons_out_sz = 0;
   ConsArgs cons_args{};  // gt_dofs and frozen mask of the last run that filed them
+  // filter groups (eskf_set_groups): the group size of the next run, and the block map of the last run's filters, with
+  // which eskf_get_group_sums reduces its results.  grp_stats [G][ESKF_NSTAT]: the last run's statistics per group (valid
+  // when grp_stats_ok); grp_buf: partial sums and host staging of eskf_get_group_sums
+  int64_t groups = 0;
+  GroupMap run_groups{};
+  bool grp_stats_ok = false;
+  double *grp_stats = nullptr, *grp_buf = nullptr;
+  size_t grp_stats_sz = 0, grp_buf_sz = 0;
 };
 
 #define CK(call)                                                  \
@@ -628,6 +661,24 @@ static int stage_in(eskf_t* h, int slot, const void* src, size_t bytes, int mem,
   if (rc) return rc;
   CK(cudaMemcpyAsync(h->stage[slot], src, bytes, cudaMemcpyHostToDevice, h->stream));
   *out = h->stage[slot];
+  return ESKF_OK;
+}
+
+// grow-only device buffer *p of *sz bytes: the new one is allocated before the old one is released, so that a request that
+// does not fit (ESKF_ENOMEM) leaves the old content readable
+static int grow(double** p, size_t* sz, size_t bytes, const char* what) {
+  if (*sz >= bytes) return ESKF_OK;
+  void* n = nullptr;
+  const cudaError_t err = cudaMalloc(&n, bytes);
+  if (err != cudaSuccess) {
+    cudaGetLastError();  // (an allocation failure is not sticky: clear it for the launches of later calls)
+    g_err = std::string(what) + ": " + std::to_string((unsigned long long)bytes) + " bytes do not fit in device memory: " +
+            cudaGetErrorString(err);
+    return err == cudaErrorMemoryAllocation ? ESKF_ENOMEM : ESKF_ECUDA;
+  }
+  CK(cudaFree(*p));
+  *p = (double*)n;
+  *sz = bytes;
   return ESKF_OK;
 }
 
@@ -790,6 +841,7 @@ static int create_alloc(eskf_t* h, const eskf_model_t* model, int64_t n_filters,
   CK(cudaDeviceGetAttribute(&smc, cudaDevAttrMultiProcessorCount, device));
   h->sm_count = smc > 0 ? smc : 148;
   h->pp_budget = pp_budget_bytes();
+  h->run_groups = group_map(n_filters, 0, 0);
   const size_t n = (size_t)n_filters;
   CK(cudaMalloc(&h->x, n * NX * sizeof(double)));
   CK(cudaMalloc(&h->P, n * 576 * sizeof(double)));
@@ -821,6 +873,8 @@ int eskf_destroy(eskf_t* h) {
   cudaFree(h->fxrec);
   cudaFree(h->cons_rec);
   cudaFree(h->cons_out);
+  cudaFree(h->grp_stats);
+  cudaFree(h->grp_buf);
   for (int i = 0; i < N_STAGE; ++i)
     if (h->stage[i]) cudaFree(h->stage[i]);
   delete h;
@@ -1026,6 +1080,8 @@ static int run_epochs(eskf_t* h, const eskf_streams_t* sp, int64_t e0, int64_t e
       }
     }
     if (h->cons_on) h->cons_E = 0;
+    h->run_groups = group_map(h->N, sp->filter_id0, h->groups);  // (a run of no epochs: its groups, and no statistics rows)
+    h->grp_stats_ok = false;
     return ESKF_OK;
   }
   const int64_t Es = e1 - e0;  // epochs of this launch
@@ -1056,6 +1112,16 @@ static int run_epochs(eskf_t* h, const eskf_streams_t* sp, int64_t e0, int64_t e
       if ((rc = stage_reserve(h, 7, sb))) return rc;
       dstats = (double*)h->stage[7];
     }
+  }
+  // with groups (eskf_set_groups), the statistics rows are also reduced per group: the buffers are reserved before anything
+  // is launched
+  const GroupMap gm = group_map(h->N, sp->filter_id0, h->groups);
+  const bool grp_stats = h->groups > 0 && dstats;
+  if (grp_stats) {
+    if ((rc = stage_reserve(h, 16, (size_t)gm.nblk * ESKF_NSTAT * sizeof(double)))) return rc;
+    const double* old = h->grp_stats;
+    if ((rc = grow(&h->grp_stats, &h->grp_stats_sz, (size_t)gm.G * ESKF_NSTAT * sizeof(double), fn.c_str()))) return rc;
+    if (h->grp_stats != old) h->grp_stats_ok = false;  // (the last run's rows went with the old buffer)
   }
   double* dtrace = nullptr;
   const size_t tb = (size_t)h->N * (size_t)T * NX * sizeof(double);
@@ -1194,6 +1260,8 @@ static int run_epochs(eskf_t* h, const eskf_streams_t* sp, int64_t e0, int64_t e
     }
   }
 #endif
+  h->run_groups = gm;  // (the results of this run are reduced with its groups, whatever eskf_set_groups says later)
+  h->grp_stats_ok = false;
   {
     NvtxRange nvtx_k("eskf_run: persistent kernel");
     if ((rc = launch(h, a, fpt, nt > 1))) return rc;
@@ -1207,13 +1275,22 @@ static int run_epochs(eskf_t* h, const eskf_streams_t* sp, int64_t e0, int64_t e
     h->launches += 2;
   }
   if (dsum) {
-    const int64_t nblk = (h->N + RED_ROWS - 1) / RED_ROWS;
-    if ((rc = stage_reserve(h, 12, (size_t)nblk * ESKF_NSTAT * sizeof(double)))) return rc;
+    const GroupMap one = group_map(h->N, 0, 0);
+    if ((rc = stage_reserve(h, 12, (size_t)one.nblk * ESKF_NSTAT * sizeof(double)))) return rc;
     NvtxRange nvtx_red("eskf_run: statistics reduction");
-    stats_partial_kernel<<<(unsigned)nblk, 256, 0, h->stream>>>(dstats, h->status, h->N, (double*)h->stage[12]);
-    stats_final_kernel<<<1, 32, 0, h->stream>>>((const double*)h->stage[12], nblk, dsum);
+    stats_partial_kernel<<<(unsigned)one.nblk, 256, 0, h->stream>>>(dstats, h->status, one, (double*)h->stage[12]);
+    stats_final_kernel<<<1, 32, 0, h->stream>>>((const double*)h->stage[12], one, dsum);
     CK(cudaGetLastError());
     h->launches += 2;
+  }
+  if (grp_stats) {
+    NvtxRange nvtx_red("eskf_run: statistics reduction per group");
+    stats_partial_kernel<<<(unsigned)gm.nblk, 256, 0, h->stream>>>(dstats, h->status, gm, (double*)h->stage[16]);
+    stats_final_kernel<<<(unsigned)((gm.G * ESKF_NSTAT + 127) / 128), 128, 0, h->stream>>>((const double*)h->stage[16], gm,
+                                                                                          h->grp_stats);
+    CK(cudaGetLastError());
+    h->launches += 2;
+    h->grp_stats_ok = true;
   }
   if (h->cons_on) {
     const int64_t E = a.E;  // (a segment's records: its epochs only)
@@ -1228,10 +1305,11 @@ static int run_epochs(eskf_t* h, const eskf_streams_t* sp, int64_t e0, int64_t e
       ca.E = E;
       for (int i = 0; i < 6; ++i) ca.gt[i] = sp->gt_dofs[i];
       ca.frozen_mask = h->model.frozen_mask & 63;
-      const int64_t n2 = h->N * E, nblk = cons_nblk(h);
+      const int64_t n2 = h->N * E;
+      const GroupMap one = group_map(h->N, 0, 0);
       cons_eval_kernel<<<(unsigned)((n2 + 127) / 128), 128, 0, h->stream>>>(h->cons_rec, nis, nees, ca);
-      cons_partial_kernel<<<(unsigned)(nblk * E), 256, 0, h->stream>>>(h->cons_rec, h->N, nblk, ca.frozen_mask != 63, part);
-      cons_final_kernel<<<(unsigned)((E * ESKF_NCONS + 127) / 128), 128, 0, h->stream>>>(part, nblk, E, ESKF_NCONS, esum);
+      cons_partial_kernel<<<(unsigned)(one.nblk * E), 256, 0, h->stream>>>(h->cons_rec, one, ca.frozen_mask != 63, part);
+      cons_final_kernel<<<(unsigned)((E * ESKF_NCONS + 127) / 128), 128, 0, h->stream>>>(part, one, E, ESKF_NCONS, esum);
       CK(cudaGetLastError());
       h->launches += 3;
       h->cons_args = ca;  // (for the envelope of eskf_get_dof_envelope)
@@ -1498,16 +1576,82 @@ int eskf_get_dof_envelope(eskf_t* h, double* dof_sum, int64_t* n_epochs, int mem
   int rc = cons_epochs(h, "eskf_get_dof_envelope", mem, n_epochs, &E);
   if (rc || E == 0 || !dof_sum) return rc;
   CK(cudaSetDevice(h->device));
-  const int64_t nblk = cons_nblk(h);
-  double* row = h->cons_out + 2 * h->N * E + (E + nblk * E) * ESKF_NCONS;  // (the layout of cons_reserve)
+  const GroupMap one = group_map(h->N, 0, 0);
+  double* row = h->cons_out + 2 * h->N * E + (E + one.nblk * E) * ESKF_NCONS;  // (the layout of cons_reserve)
   double* part = row + E * ESKF_NDOFSUM;
-  dof_partial_kernel<<<(unsigned)(nblk * E), 256, 0, h->stream>>>(h->cons_rec, h->cons_args, nblk, part);
-  cons_final_kernel<<<(unsigned)((E * ESKF_NDOFSUM + 127) / 128), 128, 0, h->stream>>>(part, nblk, E, ESKF_NDOFSUM, row);
+  dof_partial_kernel<<<(unsigned)(one.nblk * E), 256, 0, h->stream>>>(h->cons_rec, h->cons_args, one, part);
+  cons_final_kernel<<<(unsigned)((E * ESKF_NDOFSUM + 127) / 128), 128, 0, h->stream>>>(part, one, E, ESKF_NDOFSUM, row);
   CK(cudaGetLastError());
   h->launches += 2;
   const cudaMemcpyKind kd = (mem == ESKF_MEM_HOST) ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice;
   CK(cudaMemcpyAsync(dof_sum, row, (size_t)E * ESKF_NDOFSUM * sizeof(double), kd, h->stream));
   if (mem == ESKF_MEM_HOST) CK(cudaStreamSynchronize(h->stream));
+  return ESKF_OK;
+}
+
+int eskf_set_groups(eskf_t* h, int64_t group_size) {
+  if (!h || group_size < 0) {
+    g_err = "eskf_set_groups: group_size must be 0 (no groups) or positive";
+    return ESKF_EINVAL;
+  }
+  h->groups = group_size;
+  return ESKF_OK;
+}
+
+int eskf_get_group_sums(eskf_t* h, double* stats_sum, double* epoch_sum, double* dof_sum, int64_t* group0, int64_t* n_groups,
+                        int64_t* n_epochs, int mem) {
+  if (!h || (mem != ESKF_MEM_HOST && mem != ESKF_MEM_DEVICE)) {
+    g_err = "eskf_get_group_sums: bad argument";
+    return ESKF_EINVAL;
+  }
+  const GroupMap m = h->run_groups;
+  if (stats_sum && !h->grp_stats_ok) {
+    g_err = "eskf_get_group_sums: the last eskf_run produced no statistics rows or ran without groups (eskf_set_groups)";
+    return ESKF_EINVAL;
+  }
+  int64_t E = 0;
+  if (epoch_sum || dof_sum) {
+    const int rc = cons_epochs(h, "eskf_get_group_sums", mem, nullptr, &E);
+    if (rc) return rc;
+  }
+  if (group0) *group0 = m.g > 0 ? m.id0 / m.g : 0;
+  if (n_groups) *n_groups = m.G;
+  if (n_epochs) *n_epochs = h->cons_E > 0 ? h->cons_E : 0;
+  if (!stats_sum && !((epoch_sum || dof_sum) && E > 0)) return ESKF_OK;
+  CK(cudaSetDevice(h->device));
+  const bool host = mem == ESKF_MEM_HOST;
+  const cudaMemcpyKind kd = host ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice;
+  // scratch: the partial sums of the rows asked for ([E][nblk][width]) and, for a host destination, their [G][E][width]
+  const size_t wc = epoch_sum && E > 0 ? ESKF_NCONS : 0, wd = dof_sum && E > 0 ? ESKF_NDOFSUM : 0;
+  const size_t pb = (size_t)E * m.nblk, ob = host ? (size_t)m.G * E : 0;
+  if (pb > (size_t)INT32_MAX) {  // (one block per epoch and reduction block: the grid's x dimension)
+    g_err = "eskf_get_group_sums: " + std::to_string((unsigned long long)pb) + " reduction blocks (epochs x blocks of the groups) " +
+            "exceed the grid limit of 2^31 - 1: take larger groups, or fewer epochs per segment";
+    return ESKF_EINVAL;
+  }
+  int rc = grow(&h->grp_buf, &h->grp_buf_sz, ((pb + ob) * (wc + wd)) * sizeof(double), "eskf_get_group_sums");
+  if (rc) return rc;
+  double* part = h->grp_buf;
+  double* stage = part + pb * (wc + wd);
+  if (stats_sum) CK(cudaMemcpyAsync(stats_sum, h->grp_stats, (size_t)m.G * ESKF_NSTAT * sizeof(double), kd, h->stream));
+  if (wc) {
+    double* out = host ? stage : epoch_sum;
+    cons_partial_kernel<<<(unsigned)pb, 256, 0, h->stream>>>(h->cons_rec, m, h->cons_args.frozen_mask != 63, part);
+    cons_final_kernel<<<(unsigned)((m.G * E * ESKF_NCONS + 127) / 128), 128, 0, h->stream>>>(part, m, E, ESKF_NCONS, out);
+    CK(cudaGetLastError());
+    h->launches += 2;
+    if (host) CK(cudaMemcpyAsync(epoch_sum, out, ob * ESKF_NCONS * sizeof(double), kd, h->stream));
+  }
+  if (wd) {
+    double* p = part + pb * wc;
+    double* out = host ? stage + ob * wc : dof_sum;
+    dof_partial_kernel<<<(unsigned)pb, 256, 0, h->stream>>>(h->cons_rec, h->cons_args, m, p);
+    cons_final_kernel<<<(unsigned)((m.G * E * ESKF_NDOFSUM + 127) / 128), 128, 0, h->stream>>>(p, m, E, ESKF_NDOFSUM, out);
+    CK(cudaGetLastError());
+    h->launches += 2;
+    if (host) CK(cudaMemcpyAsync(dof_sum, out, ob * ESKF_NDOFSUM * sizeof(double), kd, h->stream));
+  }
+  if (host) CK(cudaStreamSynchronize(h->stream));
   return ESKF_OK;
 }
 

@@ -1225,6 +1225,44 @@ ESKF_HD void stacked_cta(int64_t block, int64_t N, int64_t fpt, int F, int64_t& 
   nf = (int)(left < F ? left : F);
 }
 
+// ---- block map of the grouped reductions (eskf_set_groups) ------------------------------------------------------------
+// Filter f of a handle whose run had filter_id0 = id0 belongs to global group (id0 + f) / g, the global-id rule of the
+// trajectories and the noise ids: local group k = (id0 + f) / g - id0 / g.  The first and last local groups may be partial.
+// g = 0 is one group, the whole handle.  A reduction block never straddles a group: every group is cut into blocks of at
+// most rpb rows from its first local row, and the blocks are numbered group after group, in row order.  With one group
+// (g = 0, or every filter in one group with id0 % g = 0) the blocks are ceil(N / rpb) blocks of rows b rpb .. (b + 1) rpb
+// - 1: the layout of the ungrouped reduction.
+// group_row0: the first local row of local group k (k = number of groups: N), so that group k has blocks
+// group_blocks(group_row0(k)) .. group_blocks(group_row0(k + 1)) - 1.
+ESKF_HD int64_t group_row0(int64_t k, int64_t N, int64_t id0, int64_t g) {
+  if (k <= 0) return 0;
+  if (g <= 0) return N;
+  const int64_t r = g - id0 % g + (k - 1) * g;  // the first group holds g - id0 % g rows
+  return r < N ? r : N;
+}
+ESKF_HD int64_t group_blocks(int64_t N, int64_t id0, int64_t g, int64_t rpb) {
+  if (g <= 0) return (N + rpb - 1) / rpb;
+  const int64_t first = g - id0 % g < N ? g - id0 % g : N, rest = N - first;
+  return (first + rpb - 1) / rpb + (rest / g) * ((g + rpb - 1) / rpb) + ((rest % g) + rpb - 1) / rpb;
+}
+// block b -> rows row0 .. row1 - 1 (1..rpb of them) and local group k
+ESKF_HD void group_block(int64_t b, int64_t N, int64_t id0, int64_t g, int64_t rpb, int64_t& row0, int64_t& row1, int64_t& k) {
+  int64_t start = 0, end = N;  // rows of the block's group
+  k = 0;
+  if (g > 0) {
+    end = group_row0(1, N, id0, g);
+    const int64_t b0 = (end + rpb - 1) / rpb, cpg = (g + rpb - 1) / rpb;  // blocks of the first group, of a whole one
+    if (b >= b0) {
+      k = 1 + (b - b0) / cpg;
+      b -= b0 + (k - 1) * cpg;
+      start = end + (k - 1) * g;
+      end = start + g < N ? start + g : N;
+    }
+  }
+  row0 = start + b * rpb;
+  row1 = row0 + rpb < end ? row0 + rpb : end;
+}
+
 // ---- filter consistency of eskf_run (eskf_keep_consistency) ------------------------------------------------------------
 // Record of one (epoch e, filter f), element-major so that the filters of a warp store and the post-pass reads coalesced:
 // element j at cons[(e * CONS_SIZE + j) * N + f].  The export instantiation of eskf_kernel3 files it, cons_eval_kernel

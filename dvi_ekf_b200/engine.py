@@ -416,6 +416,44 @@ class BatchFilter:
         CUDA tensor with ``device``."""
         return self._cons_outputs(self._lib.eskf_get_dof_envelope, "eskf_get_dof_envelope", lambda E: ((E, NDOFSUM),), device)[0]
 
+    def set_groups(self, group_size: int):
+        """Filter groups of the next ``run`` (eskf_set_groups, include/eskf.h): filter f of a handle whose run has
+        ``filter_id0 = id0`` belongs to global group ``(id0 + f) // group_size``; ``group_size = filters_per_traj`` gives one
+        group per trajectory, ``noise_id_modulus`` one per tuning candidate; 0 (the default) is one group, the whole
+        handle.  A run with groups also reduces its statistics rows per group (``get_group_sums``)."""
+        if isinstance(group_size, bool) or int(group_size) != group_size:
+            raise TypeError(f"group_size must be an integer, not {group_size!r}")
+        if group_size < 0:
+            raise ValueError(f"group_size must be 0 (no groups) or positive, not {group_size}")
+        check(self._lib.eskf_set_groups(self._h, int(group_size)), "eskf_set_groups")
+
+    def get_group_sums(self, stats: bool = True, consistency: bool = False, dof_envelope: bool = False, device: bool = False):
+        """(group0, stats_sum [G,16], epoch_sum [G,E,8], dof_sum [G,E,80]) of the last ``run`` (eskf_get_group_sums,
+        include/eskf.h): row k is global group ``group0 + k``, with the layout and meaning of ``run``'s ``stats_sum``,
+        ``get_consistency``'s ``epoch_sum`` and ``get_dof_envelope``'s ``dof_sum``.  Each array is None unless asked for;
+        ``stats`` needs a run with statistics and groups, ``consistency`` / ``dof_envelope`` the records of a run since
+        ``keep_consistency()``.  numpy arrays, or CUDA tensors with ``device``.  A shard's rows go into the job's with
+        ``sharding.place_group_rows``."""
+        g0, G, E = C.c_int64(), C.c_int64(), C.c_int64()
+        fn = self._lib.eskf_get_group_sums
+        check(fn(self._h, None, None, None, C.byref(g0), C.byref(G), C.byref(E), MEM_HOST), "eskf_get_group_sums")
+        G, E = int(G.value), int(E.value)
+        shapes = ((G, NSTAT) if stats else None, (G, E, NCONS) if consistency else None,
+                  (G, E, NDOFSUM) if dof_envelope else None)
+        if device:
+            import torch
+
+            dev = torch.device("cuda", self.device)
+            out = [None if s is None else torch.empty(s, dtype=torch.float64, device=dev) for s in shapes]
+            ptrs, mem = [None if t is None else C.c_void_p(t.data_ptr()) for t in out], MEM_DEVICE
+        else:
+            out = [None if s is None else np.empty(s) for s in shapes]
+            ptrs, mem = [None if a is None else a.ctypes.data_as(C.c_void_p) for a in out], MEM_HOST
+        check(fn(self._h, *ptrs, None, None, None, mem), "eskf_get_group_sums")
+        if device:
+            self.sync()  # (the kernels and copies ran on the handle's stream)
+        return (int(g0.value), *out)
+
     def set_prepass_budget(self, n_bytes: int):
         """Memory ``run`` may use to keep the Monte-Carlo generator and the update-MSE statistics out of the persistent kernel
         (include/eskf.h, eskf_set_prepass_budget); 0 = everything inside the kernel.  Both ways give the same bits."""

@@ -9,7 +9,7 @@ from __future__ import annotations
 
 import os
 from dataclasses import dataclass
-from typing import List, Optional
+from typing import List, Optional, Tuple
 
 import numpy as np
 
@@ -19,6 +19,7 @@ from .config import Config
 from .consistency import NIS_DIM, candidate_objective, summarise_consistency, summarise_dofs
 from .engine import BatchFilter
 from .probe import GT_IMU_DOFS
+from .sharding import summarise_stats
 
 
 @dataclass(frozen=True)
@@ -350,21 +351,25 @@ class Simulator:
         self.config.meas_noise_std = val[7:8]
         self.kf.update_noise_matrices()
 
-    def _update_config(self, cfg: Config) -> None:
-        t, xyz, q, i0 = load_trajectory(str(cfg.traj_fp), max_vals=cfg.max_vals, start_frame=cfg.camera.start_frame,
-                                        with_start_index=True)
+    def _trajectory(self, cfg: Config, traj_fp: str, max_vals: Optional[int]) -> Tuple[Camera, Streams]:
+        """(Camera, Streams) of one camera trajectory (a path, or a name of data/trajs.npz) cut to ``max_vals`` frames"""
+        t, xyz, q, i0 = load_trajectory(str(traj_fp), max_vals=max_vals, start_frame=cfg.camera.start_frame, with_start_index=True)
         mode = "zyx_legacy" if self.legacy_golden else "xyz"
         # with_notch: true (SURVEY 8f rank 4; unrunnable at the reference's HEAD, quirk Q12): the notch rows are cut like the
         # camera rows (VisualTrajectory.py:66-70) and the camera generates its rotated twin (Camera.py:131-134)
         notch = load_notch(str(cfg.notch_fp), max_vals=len(t), start_index=i0) if cfg.with_notch else None
         if notch is not None and len(notch) != len(t):
             raise ValueError(f"notch trajectory has {len(notch)} rows for {len(t)} camera frames")  # VisualTrajectory.py:70
-        self.camera = Camera(t, xyz, q, scale=cfg.camera.scale, euler_mode=mode, notch=notch)
+        camera = Camera(t, xyz, q, scale=cfg.camera.scale, euler_mode=mode, notch=notch)
+        streams = build_streams(camera, cfg.interframe_vals, cfg.model.length, cfg.model.angle, gt_dofs=cfg.gt_imu_dofs,
+                                ic_dofs=cfg.ic_imu_dofs)
+        return camera, streams
+
+    def _update_config(self, cfg: Config) -> None:
+        self.camera, self.streams = self._trajectory(cfg, cfg.traj_fp, cfg.max_vals)
         cfg.max_vals, cfg.min_t, cfg.max_t = self.camera.max_vals, self.camera.min_t, self.camera.max_t
         cfg.total_data_pts = (self.camera.max_vals - 1) * cfg.interframe_vals + 1
         self.camera_interp = (self.camera.rotated or self.camera).interpolate(cfg.interframe_vals)  # Imu.create (Imu.py:87-90)
-        self.streams: Streams = build_streams(self.camera, cfg.interframe_vals, cfg.model.length, cfg.model.angle,
-                                              gt_dofs=cfg.gt_imu_dofs, ic_dofs=cfg.ic_imu_dofs)
         self.x0 = State.from_vector(self.streams.x0)
         self._cov0 = cfg.cov0_matrix
 
@@ -450,6 +455,96 @@ class Simulator:
     def reset_kf(self) -> None:
         self.kf = Filter(self)
 
+    def _mc_x0(self, x0_row, n: int):
+        """[n, 26] initial states of Monte-Carlo runs 0 .. n-1: run 0 nominal, run i's DOFs perturbed by the draws of
+        (batch seed, i)"""
+        b = self.config.batch
+        x0 = np.repeat(np.asarray(x0_row)[None], n, 0)
+        for i in range(1, n):
+            rng = np.random.default_rng([b.seed, i])
+            x0[i, 10:13] += rng.normal(0.0, np.deg2rad(b.dof_ic_std_deg), 3)
+            x0[i, 13:16] += rng.normal(0.0, b.dof_ic_std_cm, 3)
+        return x0
+
+    def _batch(self, n: int, x0, u0, consistency: bool, groups: int = 0) -> BatchFilter:
+        """a BatchFilter of n filters with the filter's noise matrices, cov0, the given x0 / u0 rows, consistency on or off
+        and filter groups of ``groups``"""
+        cfg = self.config
+        bf = BatchFilter(n, scope_length=cfg.model.length, cam_angle_rad=cfg.model.angle, frozen_dofs=cfg.frozen_dofs,
+                         zero_frozen_dofs=not self.legacy_golden, device=self.device)
+        try:
+            bf.set_noise(np.diag(self.kf.Q)[None].copy(), np.diag(self.kf.R)[None].copy(), self.kf.stdev_nom[None].copy())
+            bf.set_state(x0, self._cov0[None], u0, None)
+            if consistency:
+                bf.keep_consistency()
+            if groups:
+                bf.set_groups(groups)
+        except Exception:
+            bf.close()
+            raise
+        return bf
+
+    def _run_kwargs(self, cam_ref, imu_ref) -> dict:
+        """the keyword arguments of BatchFilter.run for a Monte-Carlo run (``batch:`` section)"""
+        cfg, b = self.config, self.config.batch
+        imu_std = np.hstack((cfg.imu.stdev_omega, cfg.imu.stdev_accel)) if b.imu_noise else None
+        cam_std = np.array(cfg.meas_noise_std) if b.cam_noise else None
+        return dict(cam_ref=cam_ref, imu_ref=imu_ref, gt_dofs=cfg.gt_imu_dofs, seed=b.seed, imu_noise_std=imu_std,
+                    cam_noise_std=cam_std)
+
+    def _stacked_trajectories(self, names, n_filters: int, frames: Optional[int] = None, consistency: bool = False):
+        """(BatchFilter, run keyword arguments) of the stacked launch of ``run_trajectories``: the named trajectories built as
+        ``__init__`` builds ``config.traj_name``, cut to ``frames`` frames (None: the shortest one's), ``n_filters`` filters
+        each, groups of ``n_filters``.  ``bf.run(**kw)`` runs it; the caller closes the handle.  (Also the hook through which
+        tools/trajectory_study.py times the launch and the getters.)"""
+        names = [str(nm) for nm in names]
+        if not names or len(set(names)) != len(names):
+            raise ValueError("names must be one or more distinct trajectory names")
+        n = int(n_filters)
+        if n <= 0:
+            raise ValueError("n_filters must be positive")
+        cfg = self.config
+        avail = min(len(load_trajectory(nm, start_frame=cfg.camera.start_frame)[0]) for nm in names)
+        frames = avail if frames is None else int(frames)
+        if not 2 <= frames <= avail:
+            raise ValueError(f"frames must be 2 .. {avail} (the shortest trajectory's frame count), not {frames}")
+        ss = [self._trajectory(cfg, nm, frames)[1] for nm in names]
+        T = max(len(s.dt) for s in ss)
+        pad = lambda a: np.concatenate((a, np.zeros((T - len(a), *a.shape[1:]))))  # (steps past sum(n_prop): never read)
+        cat = lambda f: np.ascontiguousarray(np.concatenate([f(s) for s in ss]))
+        bf = self._batch(n * len(names), cat(lambda s: self._mc_x0(s.x0, n)), cat(lambda s: np.repeat(s.u0[None], n, 0)),
+                         consistency, groups=n)
+        kw = self._run_kwargs(cat(lambda s: s.cam_ref), cat(lambda s: s.imu_ref))
+        kw.update(dt=cat(lambda s: pad(s.dt)), om_acc=cat(lambda s: pad(s.om_acc)), n_prop=cat(lambda s: s.n_prop),
+                  cam=cat(lambda s: s.cam), notch=cat(lambda s: s.notch), n_traj=len(names), filters_per_traj=n,
+                  noise_free_filter0=True, noise_id_modulus=n)
+        return bf, kw
+
+    def run_trajectories(self, names, n_filters: int, frames: Optional[int] = None, consistency: bool = False) -> dict:
+        """One Monte-Carlo study over several trajectories (names as ``load_trajectory`` takes them, e.g. ``trans_x``), in ONE
+        stacked launch: every trajectory cut to ``frames`` camera frames (None: the shortest one's), ``n_filters`` filters
+        each.  Filter j of every trajectory is run j of ``run``: the same perturbed initial DOFs and the noise of id j
+        (run 0 noise free), so trajectories are compared on common random numbers, and each trajectory's filters give the
+        bits ``run(n_filters)`` of a simulator configured with it alone gives.  Returns, and keeps as
+        ``trajectory_results``, per name: ``stats`` (``sharding.summarise_stats`` of its filters) and, with ``consistency``,
+        ``consistency`` and ``dof_envelope`` (``summarise_consistency`` / ``summarise_dofs`` of its filters).  The
+        per-filter statistics rows are kept as ``stats`` ([len(names) * n_filters, 16], trajectory-major)."""
+        cfg = self.config
+        bf, kw = self._stacked_trajectories(names, n_filters, frames, consistency)
+        with bf:
+            st, _ = bf.run(**kw)
+            _, gst, gcons, gdof = bf.get_group_sums(stats=True, consistency=consistency, dof_envelope=consistency)
+        dim = 6 - sum(1 for f in cfg.frozen_dofs if f)
+        res = {}
+        for k, nm in enumerate(str(v) for v in names):
+            res[nm] = {"stats": summarise_stats(gst[k])}
+            if consistency:
+                res[nm]["consistency"] = summarise_consistency(gcons[k], dim)
+                res[nm]["dof_envelope"] = summarise_dofs(gdof[k], cfg.frozen_dofs)
+        self.stats = st
+        self.trajectory_results = res
+        return res
+
     def run(self, disp_config=False, save_best=False, verbose=True, n_filters: Optional[int] = None, consistency: bool = False,
             segment_epochs: Optional[int] = None):
         """Simulator.run (Simulator.py:121-158) as ONE batched launch: ``num_kf_runs`` (or ``n_filters``)
@@ -462,22 +557,8 @@ class Simulator:
         consistency records then take the memory of k epochs, not of the whole run, and their per-epoch rows are joined."""
         cfg, s = self.config, self.streams
         n = int(n_filters or self.num_kf_runs)
-        b = cfg.batch
-        x0 = np.repeat(s.x0[None], n, 0)
-        for i in range(1, n):
-            rng = np.random.default_rng([b.seed, i])
-            x0[i, 10:13] += rng.normal(0.0, np.deg2rad(b.dof_ic_std_deg), 3)
-            x0[i, 13:16] += rng.normal(0.0, b.dof_ic_std_cm, 3)
-        with BatchFilter(n, scope_length=cfg.model.length, cam_angle_rad=cfg.model.angle, frozen_dofs=cfg.frozen_dofs,
-                         zero_frozen_dofs=not self.legacy_golden, device=self.device) as bf:
-            bf.set_noise(np.diag(self.kf.Q)[None].copy(), np.diag(self.kf.R)[None].copy(), self.kf.stdev_nom[None].copy())
-            bf.set_state(x0, self._cov0[None], s.u0[None], None)
-            if consistency:
-                bf.keep_consistency()
-            imu_std = np.hstack((cfg.imu.stdev_omega, cfg.imu.stdev_accel)) if b.imu_noise else None
-            cam_std = np.array(cfg.meas_noise_std) if b.cam_noise else None
-            kw = dict(cam_ref=s.cam_ref, imu_ref=s.imu_ref, gt_dofs=cfg.gt_imu_dofs, seed=b.seed, imu_noise_std=imu_std,
-                      cam_noise_std=cam_std)
+        with self._batch(n, self._mc_x0(s.x0, n), s.u0[None], consistency) as bf:
+            kw = self._run_kwargs(s.cam_ref, s.imu_ref)
             E = len(s.n_prop)
             if segment_epochs and E:
                 k = int(segment_epochs)

@@ -38,7 +38,8 @@ def allreduce_stats(stats_sum, group=None):
     """Sum of the per-rank statistics vectors (eskf_run's stats_sum), in place; a torch tensor on the device the
     process group works on (NCCL: the GPU; gloo: the CPU).  No-op without an initialised process group.  It serves any
     per-rank sum the same way: the consistency epoch sums (``get_consistency``) and the per-DOF envelope ``dof_sum``
-    (``get_dof_envelope``, for ``consistency.summarise_dofs``) as well."""
+    (``get_dof_envelope``, for ``consistency.summarise_dofs``) as well, and the per-group sums of ``get_group_sums`` once
+    ``place_group_rows`` has put every rank's rows at their global groups."""
     import torch.distributed as dist
 
     if dist.is_available() and dist.is_initialized():
@@ -53,6 +54,25 @@ def allreduce_stats(stats_sum, group=None):
             if nvtx:
                 torch.cuda.nvtx.range_pop()
     return stats_sum
+
+
+def place_group_rows(rows, group0: int, n_groups_total: int):
+    """A shard's per-group rows (``BatchFilter.get_group_sums``: row k is global group ``group0 + k``) scattered into a zero
+    array of the job's ``n_groups_total`` groups, ``[n_groups_total, ...]``, so that ``allreduce_stats`` adds the ranks'
+    arrays.  A group cut by a shard boundary is a partial row in both shards; the addition gives its sums.  numpy in, numpy
+    out; a torch tensor gives a tensor on its device."""
+    n, g0, total = len(rows), int(group0), int(n_groups_total)
+    if g0 < 0 or g0 + n > total:
+        raise ValueError(f"rows of groups [{g0}, {g0 + n}) do not fit in {total} groups")
+    if type(rows).__module__.startswith("torch"):
+        import torch
+
+        out = torch.zeros((total, *rows.shape[1:]), dtype=rows.dtype, device=rows.device)
+    else:
+        rows = np.asarray(rows)
+        out = np.zeros((total, *rows.shape[1:]), dtype=rows.dtype)
+    out[g0:g0 + n] = rows
+    return out
 
 
 def summarise_stats(stats_sum):

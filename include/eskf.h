@@ -151,7 +151,7 @@ int eskf_run(eskf_t* h, const eskf_streams_t* streams, double* stats_out, double
  *     (a small copy that makes the call synchronous); only when noise is on and a pre-pass is possible.
  * Rules: 0 <= epoch_begin <= epoch_end <= n_epochs, otherwise ESKF_EINVAL; variant 1 (eskf_kernel): ESKF_EINVAL.  An empty
  * range (epoch_begin == epoch_end) launches nothing and changes nothing on the handle except that the consistency getters
- * then report zero epochs (with eskf_keep_consistency on); it copies carry_in to carry_out (zeros without carry_in) and does
+ * then report zero epochs (with eskf_keep_consistency on) and eskf_get_group_sums reports its groups and no statistics; it copies carry_in to carry_out (zeros without carry_in) and does
  * NOT write stats_out / stats_sum.  A refused call leaves the handle unchanged.  eskf_run(h, s, ...) with n_epochs > 0 is
  * eskf_run_epochs(h, s, 0, n_epochs, NULL, NULL, ...). */
 int eskf_run_epochs(eskf_t* h, const eskf_streams_t* streams, int64_t epoch_begin, int64_t epoch_end, const double* carry_in,
@@ -218,6 +218,40 @@ int eskf_get_consistency(eskf_t* h, double* nis, double* nees, double* epoch_sum
  * row and its partial sums with the records (ESKF_ENOMEM before launch covers them). */
 int eskf_get_dof_history(eskf_t* h, double* dofs, double* var, int64_t* n_epochs, int mem);
 int eskf_get_dof_envelope(eskf_t* h, double* dof_sum, int64_t* n_epochs, int mem);
+
+/* Filter groups (no reference counterpart): the sums of eskf_run (stats_sum), eskf_get_consistency (epoch_sum) and
+ * eskf_get_dof_envelope (dof_sum) per group of filters instead of over the whole handle, for batches whose filters are not
+ * exchangeable: stacked trajectories, tuning candidates.
+ *
+ * eskf_set_groups: group size g of the NEXT eskf_run / eskf_run_epochs; 0 (the default) is no grouping, a negative value
+ * ESKF_EINVAL.  Filter f of a handle whose run had filter_id0 = id0 belongs to GLOBAL group (id0 + f) / g, the rule of the
+ * trajectories and of noise_id_modulus: g = filters_per_traj gives one group per trajectory, g = noise_id_modulus one per
+ * candidate.  The handle's filters cover groups group0 = id0 / g .. (id0 + N - 1) / g; the first and the last may be
+ * partial.  A run records its g and filter_id0 with its results: eskf_set_groups between a run and a getter changes nothing
+ * the getter returns.  With g > 0, a run that produces statistics rows (stats_out or stats_sum non-NULL) also reduces them
+ * per group into the handle (two more small launches; none without groups), masked as stats_sum; a segment's are
+ * accumulated over epochs [0, epoch_end) like its stats_sum.  Everything else a run returns is the same with or without
+ * groups.
+ *
+ * eskf_get_group_sums: stats_sum [G,ESKF_NSTAT], epoch_sum [G,E,ESKF_NCONS], dof_sum [G,E,ESKF_NDOFSUM] of the last run;
+ * row k is global group *group0 + k and has the layout and meaning of the ungrouped vector.  G = 1 and *group0 = 0 for a run
+ * without groups.  Any pointer may be NULL (query G and E first).  epoch_sum and dof_sum follow the rules of
+ * eskf_get_consistency / eskf_get_dof_envelope: the records of the last run since eskf_keep_consistency(h, 1), ESKF_EINVAL
+ * otherwise and with variant 1, a segment's epochs only; they are computed by the call from the records, which it does not
+ * change, nor anything else a run returned.  A non-NULL stats_sum is ESKF_EINVAL when the last run produced no statistics
+ * rows or ran without groups (an empty eskf_run_epochs range produces none).  *n_epochs = E (0 without records).
+ * ESKF_EINVAL when E x blocks, the grid of the consistency or envelope reduction, exceeds 2^31 - 1 (tiny groups over many
+ * epochs): take larger groups or shorter segments.  The call allocates its partial sums (E * blocks * 88
+ * doubles, blocks = G + N / 4096 at most, plus the outputs for a host destination); ESKF_ENOMEM when they do not fit,
+ * leaving every result readable.  mem: as for eskf_get_dof_envelope.
+ * Reduction: every group is cut into blocks of at most 4096 filters from its first one, each block summed over a fixed
+ * tree, the blocks of a group added in order: the same records give the same bits, and a group's row is bit-identical to the
+ * ungrouped sum of a handle holding exactly that group's filters.  Shards: a group cut by a shard boundary appears as a
+ * partial row in both shards; adding the rows gives the group's sums (dvi_ekf_b200.sharding.place_group_rows puts a shard's
+ * rows at their global groups for the all-reduce). */
+int eskf_set_groups(eskf_t* h, int64_t group_size);
+int eskf_get_group_sums(eskf_t* h, double* stats_sum, double* epoch_sum, double* dof_sum, int64_t* group0, int64_t* n_groups,
+                        int64_t* n_epochs, int mem);
 
 /* blocks until everything queued on the handle's stream has finished */
 int eskf_sync(eskf_t* h);
