@@ -96,7 +96,10 @@ class Config:
         self.batch = SimpleNamespace(
             seed=int(b.get("seed", 1234)), imu_noise=bool(b.get("imu_noise", True)), cam_noise=bool(b.get("cam_noise", True)),
             dof_ic_std_deg=float(b.get("dof_ic_std_deg", 3.0)), dof_ic_std_cm=float(b.get("dof_ic_std_cm", 3.0)),
-            legacy_golden=bool(b.get("legacy_golden", False)), device=int(b.get("device", 0)))
+            legacy_golden=bool(b.get("legacy_golden", False)), device=int(b.get("device", 0)),
+            cam_dropout=float(b.get("cam_dropout", 0.0)))  # probability that a Monte-Carlo filter loses a camera frame
+        if not 0.0 <= self.batch.cam_dropout <= 1.0:
+            raise ValueError(f"batch.cam_dropout must be a probability in [0, 1], not {self.batch.cam_dropout}")
 
     @property
     def dofs_updated(self) -> bool:

@@ -36,13 +36,16 @@ def summarise_consistency(epoch_sum, dim_dofs: int, alpha: float = 0.05) -> dict
       ``[chi2.ppf(alpha/2, M n), chi2.ppf(1 - alpha/2, M n)] / M`` with M the epoch's count and n = 7 or d;
     - ``nis_inside``, ``nees_inside``: fraction of the epochs with a count whose average lies inside its interval (NaN if
       there is no such epoch);
-    - ``n_nis``, ``n_nees`` [E]: the counts; ``skipped`` [E]: filters whose value is NaN at the epoch; ``skipped_total``.
+    - ``n_nis``, ``n_nees`` [E]: the counts; ``skipped`` [E]: filters whose value is NaN at the epoch (a dropped measurement
+      is not counted); ``skipped_total``;
+    - ``dropped`` [E]: filters whose measurement was dropped (``BatchFilter.run(drop_prob=...)``; 0 without dropout).
     """
     s = np.asarray(epoch_sum, dtype=float).reshape(-1, 8)
     d = int(dim_dofs)
     if not 0 <= d <= 6:
         raise ValueError("dim_dofs must be 0..6")
-    out = {"n_nis": s[:, 0].copy(), "n_nees": s[:, 3].copy(), "skipped": s[:, 6].copy(), "skipped_total": float(s[:, 6].sum())}
+    out = {"n_nis": s[:, 0].copy(), "n_nees": s[:, 3].copy(), "skipped": s[:, 6].copy(), "skipped_total": float(s[:, 6].sum()),
+           "dropped": s[:, 7].copy()}
     for key, cnt, tot, dim in (("nis", s[:, 0], s[:, 1], NIS_DIM), ("nees", s[:, 3], s[:, 4], d)):
         avg = np.full(len(s), np.nan)
         if dim > 0:
@@ -90,7 +93,8 @@ def summarise_dofs(dof_sum, frozen_dofs, alpha: float = 0.05) -> dict:
       ``[binom.ppf(alpha/2, M, p_k), binom.ppf(1 - alpha/2, M, p_k)] / M``;
     - ``err_second_moment`` [E,6,6] = sum eps eps^T / M (the ensemble's error correlation, bias included) and
       ``filter_cov`` [E,6,6] = sum B / M (the filter's claimed one, symmetrised);
-    - ``count`` [E] = M and ``excluded`` [E], the filters left out at the epoch.
+    - ``count`` [E] = M and ``excluded`` [E], the filters left out at the epoch; ``dropped`` [E], the filters whose measurement
+      was dropped (they contribute their prior).
     """
     from scipy.special import erf
     from scipy.stats import binom, chi2
@@ -109,7 +113,7 @@ def summarise_dofs(dof_sum, frozen_dofs, alpha: float = 0.05) -> dict:
     with np.errstate(invalid="ignore", divide="ignore"):
         var = np.where(m[:, None] >= 2, np.maximum(s2 - s1 * s1 / mm, 0.0) / np.maximum(mm - 1, 1.0), np.nan) * est
     sig = np.sqrt(sb / mm) * est
-    out = {"count": m, "excluded": s[:, 1].copy(), "bias": bias, "rmse": np.sqrt(msq), "std": np.sqrt(var), "sigma_filter": sig}
+    out = {"count": m, "excluded": s[:, 1].copy(), "dropped": s[:, 74].copy(), "bias": bias, "rmse": np.sqrt(msq), "std": np.sqrt(var), "sigma_filter": sig}
     with np.errstate(invalid="ignore", divide="ignore"):
         out["inflation"] = out["rmse"] / sig
     out["anees_dof"] = sr / mm * est

@@ -70,14 +70,18 @@ __global__ void dfma_peak_kernel(double* out, int iters, double a, double b) {
   if (s == 123.456) out[0] = s;  // keeps the chain alive without a store in the common case
 }
 
-// eskf_noise_dump: the standard normals of (filter, step, kind), exactly as the persistent kernels draw them
+// eskf_noise_dump: the standard normals of (filter, step, kind), exactly as the persistent kernels draw them; for
+// RNG_KIND_DROP the dropout uniform of (filter, epoch) in z[0] and zeros
 __global__ void noise_dump_kernel(double* out, uint64_t seed, int64_t filter_id0, int64_t n_filters, int64_t step0, int64_t n_steps,
                                   uint32_t kind) {
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n_filters * n_steps) return;
   const int64_t f = i / n_steps, k = i - f * n_steps;
-  double z[8];
-  normal8(seed, (uint64_t)(filter_id0 + f), (uint64_t)(step0 + k), kind, z);
+  double z[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+  if (kind == RNG_KIND_DROP)
+    z[0] = drop_uniform(seed, (uint64_t)(filter_id0 + f), (uint64_t)(step0 + k));
+  else
+    normal8(seed, (uint64_t)(filter_id0 + f), (uint64_t)(step0 + k), kind, z);
   for (int j = 0; j < 8; ++j) out[i * 8 + j] = z[j];
 }
 
@@ -362,7 +366,8 @@ __global__ void cons_eval_kernel(double* __restrict__ rec, double* __restrict__ 
   if (idx >= p.E * p.N) return;
   const int64_t e = idx / p.N, f = idx - e * p.N;
   double* r = rec + e * CONS_SIZE * p.N + f;  // element j at r[j N]
-  const bool applied = r[CONS_NEES * p.N] != 0.0;
+  const double flag = r[CONS_NEES * p.N];
+  const bool applied = flag == 1.0, dropped = flag == 2.0;  // (a dropped measurement: the NEES of the prior)
   double eps[6], B[36];
 #pragma unroll
   for (int i = 0; i < 6; ++i) eps[i] = r[(CONS_DOFS + i) * p.N] - p.gt[i];
@@ -371,29 +376,30 @@ __global__ void cons_eval_kernel(double* __restrict__ rec, double* __restrict__ 
   double vn = r[CONS_NIS * p.N];
   double ve = nees_dofs(B, eps, p.frozen_mask);
   if (!applied || !isfinite(vn)) vn = NAN;
-  if (!applied || !isfinite(ve)) ve = NAN;
+  if (!(applied || dropped) || !isfinite(ve)) ve = NAN;
   nis[f * p.E + e] = vn;
   nees[f * p.E + e] = ve;
-  r[CONS_NIS * p.N] = vn;
+  r[CONS_NIS * p.N] = dropped ? -INFINITY : vn;  // (-inf marks the dropped ones for the reductions: a NIS is never infinite)
   r[CONS_NEES * p.N] = ve;
 }
 
 // epoch_sum [E][ESKF_NCONS], deterministically like stats_sum: block b of epoch e sums the finite values of the filters of
 // block b of the map through a fixed tree, cons_final_kernel adds the blocks of an epoch (of each group) in order.
-// [0] finite NIS, [1] sum, [2] sum of squares, [3..5] the same for the NEES, [6] filters whose NIS or (d > 0) NEES is NaN.
+// [0] finite NIS, [1] sum, [2] sum of squares, [3..5] the same for the NEES, [6] filters whose NIS (measurement not dropped) or
+// (d > 0) NEES is NaN, [7] filters whose measurement was dropped.
 __global__ void cons_partial_kernel(const double* __restrict__ rec, const GroupMap m, int with_nees, double* __restrict__ partial) {
-  __shared__ double sh[256][7];
+  __shared__ double sh[256][8];
   const int64_t N = m.N, e = blockIdx.x / m.nblk, b = blockIdx.x - e * m.nblk;
   int64_t r0, r1, k;
   group_block(b, N, m.id0, m.g, RED_ROWS, r0, r1, k);
   const double* vn = rec + e * CONS_SIZE * N + CONS_NIS * N;
   const double* ve = rec + e * CONS_SIZE * N + CONS_NEES * N;
-  double acc[7];
+  double acc[8];
 #pragma unroll
-  for (int i = 0; i < 7; ++i) acc[i] = 0.0;
+  for (int i = 0; i < 8; ++i) acc[i] = 0.0;
   for (int64_t r = r0 + threadIdx.x; r < r1; r += 256) {
     const double a = vn[r], c = ve[r];
-    const bool fa = isfinite(a), fc = isfinite(c);
+    const bool fa = isfinite(a), fc = isfinite(c), dr = a == -INFINITY;
     if (fa) {
       acc[0] += 1.0;
       acc[1] += a;
@@ -404,19 +410,20 @@ __global__ void cons_partial_kernel(const double* __restrict__ rec, const GroupM
       acc[4] += c;
       acc[5] += c * c;
     }
-    if (!fa || (with_nees && !fc)) acc[6] += 1.0;
+    if ((!fa && !dr) || (with_nees && !fc)) acc[6] += 1.0;
+    if (dr) acc[7] += 1.0;
   }
 #pragma unroll
-  for (int i = 0; i < 7; ++i) sh[threadIdx.x][i] = acc[i];
+  for (int i = 0; i < 8; ++i) sh[threadIdx.x][i] = acc[i];
   __syncthreads();
   for (int o = 128; o > 0; o >>= 1) {
     if ((int)threadIdx.x < o) {
 #pragma unroll
-      for (int i = 0; i < 7; ++i) sh[threadIdx.x][i] += sh[threadIdx.x + o][i];
+      for (int i = 0; i < 8; ++i) sh[threadIdx.x][i] += sh[threadIdx.x + o][i];
     }
     __syncthreads();
   }
-  if (threadIdx.x < ESKF_NCONS) partial[(int64_t)blockIdx.x * ESKF_NCONS + threadIdx.x] = threadIdx.x < 7 ? sh[0][threadIdx.x] : 0.0;
+  if (threadIdx.x < ESKF_NCONS) partial[(int64_t)blockIdx.x * ESKF_NCONS + threadIdx.x] = sh[0][threadIdx.x];
 }
 // out [G][E][width] from the partial rows [E][nblk][width] of cons_partial_kernel (width ESKF_NCONS) or dof_partial_kernel
 // (ESKF_NDOFSUM): the blocks of an epoch and group added in order
@@ -473,10 +480,12 @@ __global__ void __launch_bounds__(256) dof_history_kernel(const double* __restri
 // 32 g + l), an xor butterfly for each of the remaining columns (lane c - 64 keeps column c).  Every lane accumulates its
 // columns over the warp's rows in order, and the eight warps are added in order at the end.  cons_final_kernel adds the
 // blocks.
+// A dropped measurement (CONS_NIS = -inf, cons_eval_kernel) lets the filter contribute its prior and counts in column DSUM_DROP.
 __global__ void __launch_bounds__(256) dof_partial_kernel(const double* __restrict__ rec, const ConsArgs p, const GroupMap m,
                                                           double* __restrict__ partial) {
-  constexpr int NG = DSUM_USED / 32;  // full column groups; the tail DSUM_USED - 32 NG < 32 columns
-  static_assert(DSUM_USED - 32 * NG < 32, "tail");
+  constexpr int W = DSUM_DROP + 1;  // reduced columns
+  constexpr int NG = W / 32;  // full column groups; the tail W - 32 NG < 32 columns
+  static_assert(W - 32 * NG < 32 && DSUM_DROP >= DSUM_USED, "tail");
   __shared__ double sh[8][32 * (NG + 1)];
   const int64_t e = blockIdx.x / m.nblk, b = blockIdx.x - e * m.nblk;
   const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
@@ -489,18 +498,21 @@ __global__ void __launch_bounds__(256) dof_partial_kernel(const double* __restri
   for (int g = 0; g <= NG; ++g) acc[g] = 0.0;
   for (int r0 = 32 * w; r0 < nr; r0 += 256) {  // (warp-uniform)
     const int r = r0 + lane;
-    double t[DSUM_USED];
+    double t[W];
 #pragma unroll
-    for (int c = 0; c < DSUM_USED; ++c) t[c] = 0.0;
+    for (int c = 0; c < W; ++c) t[c] = 0.0;
     if (r < nr) {
       double eps[6];
 #pragma unroll
       for (int i = 0; i < 6; ++i) eps[i] = re[(CONS_DOFS + i) * p.N + r] - p.gt[i];
-      dof_terms(re[CONS_NIS * p.N + r], eps, re + CONS_B * p.N + r, p.N, p.frozen_mask, t);
+      const double vn = re[CONS_NIS * p.N + r];
+      const bool dr = vn == -INFINITY;
+      dof_terms(dr ? 0.0 : vn, eps, re + CONS_B * p.N + r, p.N, p.frozen_mask, t);
+      t[DSUM_DROP] = dr ? 1.0 : 0.0;
     }
     // (the tail first, then the groups from the last: fewer terms live at once)
 #pragma unroll
-    for (int c = 32 * NG; c < DSUM_USED; ++c) {
+    for (int c = 32 * NG; c < W; ++c) {
       double v = t[c];
 #pragma unroll
       for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
@@ -526,7 +538,7 @@ __global__ void __launch_bounds__(256) dof_partial_kernel(const double* __restri
   __syncthreads();
   if (threadIdx.x < ESKF_NDOFSUM) {
     double a = 0.0;
-    if (threadIdx.x < DSUM_USED)
+    if (threadIdx.x < W)
       for (int k = 0; k < 8; ++k) a += sh[k][threadIdx.x];
     partial[(int64_t)blockIdx.x * ESKF_NDOFSUM + threadIdx.x] = a;
   }
@@ -628,6 +640,10 @@ struct eskf_handle {
   bool grp_stats_ok = false;
   double *grp_stats = nullptr, *grp_buf = nullptr;
   size_t grp_stats_sz = 0, grp_buf_sz = 0;
+  // simulated frame loss (eskf_set_meas_dropout): drop probabilities [drop_nt][drop_E] of every later run, on (drop_nt > 0) or off
+  double* drop_p = nullptr;
+  size_t drop_sz = 0;
+  int64_t drop_nt = 0, drop_E = 0;
 };
 
 #define CK(call)                                                  \
@@ -875,6 +891,7 @@ int eskf_destroy(eskf_t* h) {
   cudaFree(h->cons_out);
   cudaFree(h->grp_stats);
   cudaFree(h->grp_buf);
+  cudaFree(h->drop_p);
   for (int i = 0; i < N_STAGE; ++i)
     if (h->stage[i]) cudaFree(h->stage[i]);
   delete h;
@@ -1067,6 +1084,18 @@ static int run_epochs(eskf_t* h, const eskf_streams_t* sp, int64_t e0, int64_t e
       return ESKF_EINVAL;
     }
   }
+  if (h->drop_nt > 0) {
+    if (kernel_of(h) != 3) {
+      g_err = fn + ": measurement dropout needs the default kernel (eskf_set_variant(h, 1) selects the first one)";
+      return ESKF_EINVAL;
+    }
+    if (h->drop_nt != nt || h->drop_E != E) {
+      g_err = fn + ": the dropout probabilities are [" + std::to_string((long long)h->drop_nt) + ", " +
+              std::to_string((long long)h->drop_E) + "], the streams [n_traj = " + std::to_string((long long)nt) +
+              ", n_epochs = " + std::to_string((long long)E) + "]";
+      return ESKF_EINVAL;
+    }
+  }
   const size_t cb = (size_t)h->N * ESKF_NCARRY * sizeof(double);
   if (!whole && e0 == e1) {  // an empty range launches nothing: the carry passes through, the statistics are not written
     if (carry_out && carry_out != carry_in) {
@@ -1183,6 +1212,7 @@ static int run_epochs(eskf_t* h, const eskf_streams_t* sp, int64_t e0, int64_t e
   a.stats_sum = nullptr;  // (the kernels' own atomic sums are not used any more: see stats_partial_kernel)
   a.trace = dtrace;
   a.cons = (h->cons_on && E > 0) ? h->cons_rec : nullptr;
+  a.drop_p = h->drop_nt > 0 ? h->drop_p : nullptr;
   a.seed = sp->seed;
   a.noise_free0 = sp->noise_free_filter0;
   a.noise_mod = sp->noise_id_modulus;
@@ -1401,7 +1431,8 @@ int eskf_fp64_peak(int device, void* cuda_stream, int repeats, double* tflops_ou
 
 int eskf_noise_dump(int device, void* cuda_stream, uint64_t seed, int64_t filter_id0, int64_t n_filters, int64_t step0,
                     int64_t n_steps, int kind, double* out, int mem) {
-  if (!out || n_filters <= 0 || n_steps <= 0 || (kind != (int)RNG_KIND_IMU && kind != (int)RNG_KIND_CAM)) {
+  if (!out || n_filters <= 0 || n_steps <= 0 ||
+      (kind != (int)RNG_KIND_IMU && kind != (int)RNG_KIND_CAM && kind != (int)RNG_KIND_DROP)) {
     g_err = "eskf_noise_dump: bad argument";
     return ESKF_EINVAL;
   }
@@ -1423,6 +1454,46 @@ int eskf_noise_dump(int device, void* cuda_stream, uint64_t seed, int64_t filter
   const int rc = body();
   if (mem == ESKF_MEM_HOST) cudaFree(d);
   return rc;
+}
+
+int eskf_set_meas_dropout(eskf_t* h, const double* prob, int64_t n_traj, int64_t n_epochs, int mem) {
+  if (!h || (mem != ESKF_MEM_HOST && mem != ESKF_MEM_DEVICE)) {
+    g_err = "eskf_set_meas_dropout: bad argument";
+    return ESKF_EINVAL;
+  }
+  if (!prob) {
+    h->drop_nt = h->drop_E = 0;
+    return ESKF_OK;
+  }
+  if (n_traj < 1 || n_epochs < 0) {
+    g_err = "eskf_set_meas_dropout: n_traj must be positive and n_epochs non-negative";
+    return ESKF_EINVAL;
+  }
+  CK(cudaSetDevice(h->device));
+  const size_t n = (size_t)n_traj * (size_t)n_epochs, bytes = n * sizeof(double);
+  std::vector<double> hp;
+  const double* v = prob;
+  if (mem == ESKF_MEM_DEVICE && n > 0) {  // (read back to validate: a synchronous call, not a hot path)
+    hp.resize(n);
+    CK(cudaMemcpyAsync(hp.data(), prob, bytes, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    v = hp.data();
+  }
+  for (size_t i = 0; i < n; ++i)
+    if (!(v[i] >= 0.0 && v[i] <= 1.0)) {  // (false for NaN)
+      g_err = "eskf_set_meas_dropout: entry " + std::to_string((unsigned long long)i) + " = " + std::to_string(v[i]) +
+              " is not a probability in [0, 1]";
+      return ESKF_EINVAL;
+    }
+  int rc = grow(&h->drop_p, &h->drop_sz, bytes > 0 ? bytes : sizeof(double), "eskf_set_meas_dropout");
+  if (rc) return rc;
+  if (n > 0) {  // (from the validated host values; the source may go away on return)
+    CK(cudaMemcpyAsync(h->drop_p, v, bytes, cudaMemcpyHostToDevice, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+  }
+  h->drop_nt = n_traj;
+  h->drop_E = n_epochs;
+  return ESKF_OK;
 }
 
 int64_t eskf_launch_count(const eskf_t* h) { return h ? h->launches : 0; }

@@ -79,6 +79,9 @@ struct KArgs {
   int64_t e_base, E_all;
   const double* carry_in;
   double* carry_out;
+  // simulated frame loss (eskf_set_meas_dropout; eskf_kernel3 export instantiations only): [n_traj][E_all] (E_all = E outside a
+  // segment) drop probabilities of every epoch, indexed like the per-epoch streams, or nullptr
+  const double* drop_p;
 };
 
 // one FilterTraj row's worth of nominal state in the layout of x (include/eskf.h)

@@ -738,7 +738,10 @@ __device__ __forceinline__ void role3_cam(const KArgs& a, const Ctx3& c, int lan
     // ---- U0: residual (Filter.py:363-375) ----
     if (lane < F) {
       bool ok = false;
-      if (act) {
+      // export mode, simulated frame loss (eskf_set_meas_dropout): the STAGER decided with the measurement; a dropped one is
+      // not evaluated and SX3_OK stays -1 for the covariance warps (no update: the tile keeps P-) and for U2 below (no status bit)
+      const bool drop = EX && act && a.drop_p && sx[SX3_OK * F] < 0.0;
+      if (act && !drop) {
         double cam[7], res[7];
 #pragma unroll
         for (int i = 0; i < 7; ++i) cam[i] = sx[(SX3_MEAS + i) * F];
@@ -755,7 +758,7 @@ __device__ __forceinline__ void role3_cam(const KArgs& a, const Ctx3& c, int lan
         for (int i = 0; i < 7; ++i) sx[(SX3_RES + i) * F] = res[i];
         if (!ok) st |= ESKF_STATUS_ASIN_DOMAIN;
       }
-      sx[SX3_OK * F] = ok ? 1.0 : 0.0;
+      sx[SX3_OK * F] = drop ? -1.0 : ok ? 1.0 : 0.0;
     }
     PT_MARK(5);
     PT_MARK(5);
@@ -780,7 +783,7 @@ __device__ __forceinline__ void role3_cam(const KArgs& a, const Ctx3& c, int lan
         for (int i = 0; i < 4; ++i) qc[i] = qn[i];
         n_upd += 1.0;
         if (EX && a.trace && k0_of<SG>(c) + k > 0) trace_cam(a.trace + ((c.f0 + lane) * a.T + k0_of<SG>(c) + k - 1) * NX, pc, qc);
-      } else {
+      } else if (!EX || sx[SX3_OK * F] >= 0.0) {  // (a dropped measurement is not a skipped update)
         st |= ESKF_STATUS_UPDATE_SKIPPED;
       }
 #if ESKF_OPT_PP
@@ -1156,6 +1159,9 @@ __device__ __forceinline__ void role3_stage(const KArgs& a, const Ctx3& c, int l
 #endif
   };
   auto stage_meas = [&](int64_t e) {
+    if (EX && a.drop_p)  // simulated frame loss: SX3_OK = -1 marks the epoch's measurement as dropped
+      sx[SX3_OK * F] = meas_dropped(a.drop_p[erow3<SG>(a, c, e)], a.seed, (uint64_t)gid, (uint64_t)((SG ? a.e_base : 0) + e),
+                                    a.noise_free0 && gid == 0) ? -1.0 : 0.0;
 #if ESKF_OPT_PP
     if (a.meas_pf) {
       const double* m = a.meas_pf + (e * a.N + c.f0 + lane) * 8;
@@ -1656,7 +1662,8 @@ __device__ __forceinline__ void role3_cov(const KArgs& a, const Ctx3& c, int ct)
     __syncthreads();  // U0 | U1
     JIT();
     PT_MARK(6);
-    const bool upd_c = inv_ok && (sxc[SX3_OK * F] != 0.0);
+    // (SX3_OK: 1 valid residual, 0 none, -1 a measurement dropped by eskf_set_meas_dropout, export mode only)
+    const bool upd_c = inv_ok && (EX ? sxc[SX3_OK * F] > 0.0 : sxc[SX3_OK * F] != 0.0);
     double nis = NAN;  // (export mode: consistency record)
     if (upd_c) {
       double K[3][7], res[7], dl[3];
@@ -1680,7 +1687,7 @@ __device__ __forceinline__ void role3_cov(const KArgs& a, const Ctx3& c, int ct)
       if (a.cons && cg == 0 && cf < c.nf) {
         double* r = a.cons + e * CONS_SIZE * a.N + c.f0 + cf;
         r[CONS_NIS * a.N] = nis;
-        r[CONS_NEES * a.N] = upd_c ? 1.0 : 0.0;
+        r[CONS_NEES * a.N] = upd_c ? 1.0 : sxc[SX3_OK * F] < 0.0 ? 2.0 : 0.0;  // applied / not applied / dropped
       }
     }
     PT_MARK(7);

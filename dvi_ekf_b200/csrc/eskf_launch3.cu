@@ -33,8 +33,9 @@ cudaError_t launch_eskf_kernel3<ESKF_F>(const KArgs& a, cudaStream_t stream) {
   // export mode (FilterTraj rows, eskf_streams_t.trace_x; Jacobian record of the last step, eskf_keep_jacobians; consistency
   // records, eskf_keep_consistency) and the CTA mapping of stacked trajectories are separate instantiations: the production
   // kernel of a single-trajectory batch carries none of their code (the dump alone cost 10 % through register allocation).
-  // A segment of the trajectory (eskf_run_epochs) is a third bit: eskf_run keeps the kernels it had.
-  const int mode = ((a.trace || a.fx_dump || a.cons) ? 1 : 0) | (a.n_traj > 1 ? 2 : 0) | (a.k_base ? 4 : 0);
+  // A segment of the trajectory (eskf_run_epochs) is a third bit: eskf_run keeps the kernels it had.  Simulated frame loss
+  // (eskf_set_meas_dropout) is export code too.
+  const int mode = ((a.trace || a.fx_dump || a.cons || a.drop_p) ? 1 : 0) | (a.n_traj > 1 ? 2 : 0) | (a.k_base ? 4 : 0);
   auto kern = mode == 0   ? eskf_kernel3<F, ESKF_REG_S, ESKF_REG_C, 0>
               : mode == 1 ? eskf_kernel3<F, ESKF_REG_S, ESKF_REG_C, 1>
               : mode == 2 ? eskf_kernel3<F, ESKF_REG_S, ESKF_REG_C, 2>

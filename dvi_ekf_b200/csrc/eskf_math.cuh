@@ -1269,7 +1269,8 @@ ESKF_HD void group_block(int64_t b, int64_t N, int64_t id0, int64_t g, int64_t r
 // (eskf_api.cu) turns it into the NIS / NEES outputs.
 constexpr int CONS_NIS = 0;    // r^T inv(S) r of the update, NaN if it was not applied (covariance lane 0)
 constexpr int CONS_DOFS = 1;   // 6: dofs after the update (JACOB role)
-constexpr int CONS_NEES = 7;   // kernel: 1 if the update was applied, else 0; cons_eval_kernel overwrites it with the NEES
+constexpr int CONS_NEES = 7;   // kernel: 1 if the update was applied, 2 if its measurement was dropped (eskf_set_meas_dropout),
+                               // else 0; cons_eval_kernel overwrites it with the NEES (and CONS_NIS of a dropped one with -inf)
 constexpr int CONS_B = 8;      // 36: covariance block of error-state rows / columns 9..14 after the update, as the tile holds
                                // it (the transpose of the reference's, which a quadratic form does not see; lanes 3 and 4)
 constexpr int CONS_SIZE = 44;  // doubles
@@ -1326,7 +1327,8 @@ constexpr int DSUM_EXCL = 1;   // excluded filters
 constexpr int DSUM_DOF = 2;    // 7 per DOF i at DSUM_DOF + 7 i: eps, eps^2, B_ii, eps^2 / B_ii, eps^2 <= k^2 B_ii (k = 1, 2, 3)
 constexpr int DSUM_EE = 44;    // 15: eps_i eps_j, pairs i < j row-major (0,1), (0,2), ..., (4,5)
 constexpr int DSUM_BB = 59;    // 15: (B_ij + B_ji) / 2, the same pairs
-constexpr int DSUM_USED = 74;  // the rest of the row is reserved (0)
+constexpr int DSUM_USED = 74;  // the terms of dof_terms
+constexpr int DSUM_DROP = 74;  // filters whose measurement was dropped (dof_partial_kernel); the rest of the row is reserved (0)
 
 // The terms of one record for that row, t[0 .. DSUM_USED - 1]: nis as cons_eval_kernel left it, eps = dofs - gt_dofs,
 // B the 6x6 DOF block (row-major, element (i, j) at B[(6 i + j) ld]: ld = N reads it in place from a record).  The filter

@@ -110,4 +110,28 @@ ESKF_HD void normal8(uint64_t seed, uint64_t filter, uint64_t step, uint32_t kin
   box_muller32(b[2], b[3], z + 6);
 }
 
+// ---- simulated frame loss (eskf_set_meas_dropout, include/eskf.h) ----
+// One uniform per (noise id, GLOBAL epoch): word 0 of the Philox block with normal4's counter layout, kind RNG_KIND_DROP and
+// draw 0.  u = (x + 1/2) 2^-32 is exact in double precision and lies strictly inside (0, 1): 2^-33 <= u <= 1 - 2^-33.  It
+// depends on nothing but (seed, id, epoch), so segments, shards and noise_id_modulus see the draws of one whole-batch run,
+// and the other kinds' draws do not move.  eskf_noise_dump(kind = ESKF_NOISE_DROP) reads it back.
+constexpr uint32_t RNG_KIND_DROP = 3;
+
+ESKF_HD double unit_open32(uint32_t x) { return ((double)x + 0.5) * 2.3283064365386963e-10; }  // (x + 1/2) 2^-32
+
+ESKF_HD double drop_uniform(uint64_t seed, uint64_t id, uint64_t epoch) {
+  uint32_t c[4] = {(uint32_t)epoch, RNG_KIND_DROP * 16u + ((uint32_t)(epoch >> 32) << 8), (uint32_t)id, (uint32_t)(id >> 32)};
+  philox4x32_10(c, (uint32_t)seed, (uint32_t)(seed >> 32));
+  return unit_open32(c[0]);
+}
+
+// The measurement of epoch `epoch` is dropped for noise id `id` iff u < p: p = 0 never drops, p = 1 always does.  Within one
+// id the masks nest (p1 <= p2: every epoch dropped at p1 is dropped at p2, both compare the same u), which a sweep over p
+// relies on.  A noise-free reference filter (nf0: noise_free_filter0 and id 0) makes no random drop: it loses exactly the
+// epochs with p == 1.
+ESKF_HD bool meas_dropped(double p, uint64_t seed, uint64_t id, uint64_t epoch, bool nf0) {
+  if (!(p > 0.0)) return false;
+  return nf0 ? p == 1.0 : drop_uniform(seed, id, epoch) < p;
+}
+
 }  // namespace eskf

@@ -96,6 +96,32 @@ def check_run_geometry(n_filters: int, n_traj: int, filters_per_traj: int, filte
             raise ValueError(f"sum(n_prop) = {int(tot.max())} exceeds n_steps = {n_steps}")
 
 
+def drop_prob_array(prob, n_traj: int, n_epochs: int) -> np.ndarray:
+    """The drop probabilities of ``BatchFilter.run(drop_prob=...)`` as the C-contiguous float64 [n_traj, n_epochs] array
+    eskf_set_meas_dropout takes: ``prob`` is a scalar, [n_epochs] (every trajectory) or [n_traj, n_epochs], every entry
+    finite and in [0, 1].  Raises ``ValueError`` otherwise."""
+    p = np.asarray(prob, dtype=np.float64)
+    if p.ndim > 2 or (p.ndim >= 1 and p.shape[-1] != n_epochs) or (p.ndim == 2 and p.shape[0] != n_traj):
+        raise ValueError(f"drop_prob must be a scalar, [{n_epochs}] or [{n_traj}, {n_epochs}] (n_traj, n_epochs of the streams), "
+                         f"not of shape {p.shape}")
+    if not np.isfinite(p).all():
+        raise ValueError("drop_prob must be finite (NaN or infinite entry)")
+    if (p < 0).any() or (p > 1).any():
+        raise ValueError(f"drop_prob entries are probabilities in [0, 1], not {float(p.min())} .. {float(p.max())}")
+    return np.ascontiguousarray(np.broadcast_to(p, (n_traj, n_epochs)))
+
+
+def mask_from_uniforms(u, p, noise_free) -> np.ndarray:
+    """The dropout rule of eskf_set_meas_dropout (include/eskf.h) on given uniforms: ``u`` and ``p`` [n, E] (the filters'
+    uniforms and drop probabilities), ``noise_free`` [n] (noise-free reference filters, which lose only the epochs with
+    p == 1).  Returns bool [n, E]: dropped iff u < p."""
+    u, p = np.asarray(u, dtype=np.float64), np.asarray(p, dtype=np.float64)
+    m = u < p
+    nf = np.asarray(noise_free, dtype=bool)
+    m[nf] = p[nf] == 1.0
+    return m
+
+
 def segment_steps(n_prop, n_steps: int, e0: int, e1: int):
     """(k0, k1), each [n_traj]: the global steps at which every trajectory's epochs e0 and e1 start, as the kernels count
     them -- the running sum of n_prop with every epoch clamped to what is left of the n_steps-long stream (a negative entry
@@ -231,7 +257,7 @@ class BatchFilter:
     def run(self, dt, om_acc, n_prop, cam, notch, cam_ref=None, imu_ref=None, gt_dofs=(0, 0, 0, 0, 0, 20.0),
             n_traj: int = 1, filters_per_traj: Optional[int] = None, seed: int = 0, filter_id0: int = 0,
             imu_noise_std=None, cam_noise_std=None, noise_free_filter0: bool = True, want_stats: bool = True,
-            stats_on_device: bool = False, trace=None, noise_id_modulus: int = 0, epochs=None, carry=None):
+            stats_on_device: bool = False, trace=None, noise_id_modulus: int = 0, epochs=None, carry=None, drop_prob=None):
         """``Filter.run`` (Filter.py:144-185) for every filter, in one persistent kernel.
         Returns (stats [N,16], stats_sum [16]) (see include/eskf.h) or None.
         ``trace``: optional [N,T,26] float64 array (numpy for host streams, CUDA tensor for device streams) that
@@ -243,7 +269,9 @@ class BatchFilter:
         without ``want_stats`` and for an empty range (which runs nothing).  ``carry`` [N,4] (the running update-MSE sums, applied updates and status word) comes
         from the previous segment's return value, None to start fresh; it and the returned one live where the statistics
         do (numpy, or CUDA tensors with ``stats_on_device``), and the returned one is also kept as ``last_carry``.  Segments
-        run back to back give bit for bit what one run gives; a checkpoint is ``get_state()``, the carry and e1."""
+        run back to back give bit for bit what one run gives; a checkpoint is ``get_state()``, the carry and e1.
+        ``drop_prob``: simulated frame loss (``set_meas_dropout``): a scalar, [E] or [n_traj, E] (numpy, or a CUDA tensor) of
+        per-epoch probabilities that a filter loses the camera measurement; None runs without dropout."""
         adt = _Arg(dt, None, name="dt")
         anp = _Arg(n_prop, None, dtype=np.int32, name="n_prop")
         T = adt.rows // n_traj
@@ -275,6 +303,7 @@ class BatchFilter:
             if atr.mem != mem:
                 raise ValueError("trace must live where the streams live (host numpy / CUDA tensor)")
             s.trace_x = atr.ptr
+        self.set_meas_dropout(drop_prob, n_traj, E)
         if epochs is not None:
             return self._run_epochs(s, int(epochs[0]), int(epochs[1]), carry, want_stats, stats_on_device)
         if not want_stats:
@@ -331,6 +360,30 @@ class BatchFilter:
         for e0, e1 in zip(b, b[1:]):
             st, sm, carry = self.run(dt, om_acc, n_prop, cam, notch, epochs=(e0, e1), carry=carry, **kw)
             yield e0, e1, st, sm
+
+    def set_meas_dropout(self, prob, n_traj: int = 1, n_epochs: Optional[int] = None):
+        """Simulated frame loss of every later ``run`` (eskf_set_meas_dropout, include/eskf.h): filter g loses the camera
+        measurement of epoch e with probability prob[trajectory, e], decided on the device from the run's seed and the
+        filter's noise id (``dropout_mask`` gives the mask).  ``prob``: a scalar, [n_epochs] or [n_traj, n_epochs] (numpy, or a
+        CUDA tensor), broadcast to [n_traj, n_epochs] (the streams' shape, which a run checks); None switches it off."""
+        if prob is None:
+            check(self._lib.eskf_set_meas_dropout(self._h, None, 0, 0, MEM_HOST), "eskf_set_meas_dropout")
+            return
+        if n_epochs is None:
+            if np.ndim(prob) == 0:
+                raise ValueError("n_epochs is needed for a scalar probability")
+            n_epochs = int(prob.shape[-1]) if _is_torch(prob) else np.shape(prob)[-1]
+        if _is_torch(prob) and prob.is_cuda:
+            import torch
+
+            drop_prob_array(prob.detach().cpu().numpy(), n_traj, n_epochs)  # (the shape and value checks, on a host copy)
+            t = torch.broadcast_to(prob.to(torch.float64), (n_traj, n_epochs)).contiguous()
+            check(self._lib.eskf_set_meas_dropout(self._h, C.c_void_p(t.data_ptr()), n_traj, n_epochs, MEM_DEVICE),
+                  "eskf_set_meas_dropout")
+            return
+        p = drop_prob_array(prob.numpy() if _is_torch(prob) else prob, n_traj, n_epochs)
+        check(self._lib.eskf_set_meas_dropout(self._h, p.ctypes.data_as(C.c_void_p), n_traj, n_epochs, MEM_HOST),
+              "eskf_set_meas_dropout")
 
     def sync(self):
         check(self._lib.eskf_sync(self._h), "eskf_sync")
@@ -464,7 +517,7 @@ class BatchFilter:
         check(self._lib.eskf_set_variant(self._h, int(variant)), "eskf_set_variant")
 
 
-NOISE_IMU, NOISE_CAM = 1, 2
+NOISE_IMU, NOISE_CAM, NOISE_DROP = 1, 2, 3
 
 
 def noise_samples(seed: int, filter_id0: int, n_filters: int, step0: int, n_steps: int, kind: int, device: int = 0):
@@ -474,6 +527,26 @@ def noise_samples(seed: int, filter_id0: int, n_filters: int, step0: int, n_step
     check(lib.eskf_noise_dump(int(device), None, int(seed), int(filter_id0), int(n_filters), int(step0), int(n_steps), int(kind),
                               out.ctypes.data_as(C.c_void_p), MEM_HOST), "eskf_noise_dump")
     return out
+
+
+def dropout_mask(prob, seed: int, filter_id0: int, n_filters: int, epochs, n_traj: int = 1, filters_per_traj: Optional[int] = None,
+                 noise_id_modulus: int = 0, noise_free_filter0: bool = True, device: int = 0) -> np.ndarray:
+    """bool [n_filters, e1 - e0]: which of global epochs ``epochs = (e0, e1)`` filters ``filter_id0 ..`` lose in a run with
+    ``drop_prob = prob`` (a scalar, [E] or [n_traj, E]) and these run arguments, from the uniforms the device draws
+    (``eskf_noise_dump`` with ESKF_NOISE_DROP: the definition of the draw)."""
+    e0, e1 = (int(v) for v in epochs)
+    E = int(np.shape(prob)[-1]) if np.ndim(prob) else e1
+    p = drop_prob_array(prob, n_traj, E)
+    if not 0 <= e0 <= e1 <= E:
+        raise ValueError(f"epochs [{e0}, {e1}) is not within [0, {E}]")
+    g = int(filter_id0) + np.arange(int(n_filters))
+    traj = g // int(filters_per_traj or n_filters) if n_traj > 1 else np.zeros_like(g)
+    gid = g % noise_id_modulus if noise_id_modulus > 0 else g
+    if e1 == e0:
+        return np.zeros((len(g), 0), dtype=bool)
+    lo = int(gid.min())
+    u = noise_samples(seed, lo, int(gid.max()) - lo + 1, e0, e1 - e0, NOISE_DROP, device)[:, :, 0]
+    return mask_from_uniforms(u[gid - lo], p[traj, e0:e1], (gid == 0) & bool(noise_free_filter0))
 
 
 def fp64_peak_tflops(device: int = 0, repeats: int = 5) -> float:

@@ -419,7 +419,7 @@ class Simulator:
             # r noise realisations, so candidates differ only by their parameters
             st, _ = bf.run(s.dt, s.om_acc, s.n_prop, s.cam, s.notch, cam_ref=s.cam_ref, imu_ref=s.imu_ref,
                            gt_dofs=cfg.gt_imu_dofs, seed=b.seed, imu_noise_std=imu_std, cam_noise_std=cam_std,
-                           noise_free_filter0=True, noise_id_modulus=r)
+                           noise_free_filter0=True, noise_id_modulus=r, **self._dropout_kwargs())
             if metric in ("nis", "nees"):
                 nis, nees, _ = bf.get_consistency()
                 return candidate_objective(nis if metric == "nis" else nees, m, NIS_DIM if metric == "nis" else dim_dofs)
@@ -484,13 +484,21 @@ class Simulator:
             raise
         return bf
 
-    def _run_kwargs(self, cam_ref, imu_ref) -> dict:
+    def _dropout_kwargs(self, cam_dropout: Optional[float] = None) -> dict:
+        """``drop_prob`` of BatchFilter.run for the frame-loss probability ``cam_dropout`` (None: ``batch.cam_dropout``); nothing
+        at 0, so that a run without frame loss keeps the production kernel"""
+        p = self.config.batch.cam_dropout if cam_dropout is None else float(cam_dropout)
+        if not 0.0 <= p <= 1.0:
+            raise ValueError(f"cam_dropout must be a probability in [0, 1], not {p}")
+        return {"drop_prob": p} if p > 0 else {}
+
+    def _run_kwargs(self, cam_ref, imu_ref, cam_dropout: Optional[float] = None) -> dict:
         """the keyword arguments of BatchFilter.run for a Monte-Carlo run (``batch:`` section)"""
         cfg, b = self.config, self.config.batch
         imu_std = np.hstack((cfg.imu.stdev_omega, cfg.imu.stdev_accel)) if b.imu_noise else None
         cam_std = np.array(cfg.meas_noise_std) if b.cam_noise else None
         return dict(cam_ref=cam_ref, imu_ref=imu_ref, gt_dofs=cfg.gt_imu_dofs, seed=b.seed, imu_noise_std=imu_std,
-                    cam_noise_std=cam_std)
+                    cam_noise_std=cam_std, **self._dropout_kwargs(cam_dropout))
 
     def _stacked_trajectories(self, names, n_filters: int, frames: Optional[int] = None, consistency: bool = False):
         """(BatchFilter, run keyword arguments) of the stacked launch of ``run_trajectories``: the named trajectories built as
@@ -546,7 +554,7 @@ class Simulator:
         return res
 
     def run(self, disp_config=False, save_best=False, verbose=True, n_filters: Optional[int] = None, consistency: bool = False,
-            segment_epochs: Optional[int] = None):
+            segment_epochs: Optional[int] = None, cam_dropout: Optional[float] = None):
         """Simulator.run (Simulator.py:121-158) as ONE batched launch: ``num_kf_runs`` (or ``n_filters``)
         independent filters, run 0 noise free (the reference's deterministic run), the others with
         Monte-Carlo IMU / camera noise and DOF initial-condition perturbations (``batch:`` section).
@@ -554,11 +562,13 @@ class Simulator:
         epoch and their chi-square intervals), ``self.dof_envelope`` ``consistency.summarise_dofs`` of it (bias, RMSE,
         claimed sigma, inflation, per-DOF ANEES and coverage per DOF and epoch).
         ``segment_epochs`` k: the same run in launches of k epochs (``BatchFilter.run_segments``), with the same results; the
-        consistency records then take the memory of k epochs, not of the whole run, and their per-epoch rows are joined."""
+        consistency records then take the memory of k epochs, not of the whole run, and their per-epoch rows are joined.
+        ``cam_dropout``: the probability that a filter loses a camera frame (``BatchFilter.run(drop_prob=...)``; run 0, the
+        noise-free one, loses none); None takes ``batch.cam_dropout`` (default 0: no frame loss)."""
         cfg, s = self.config, self.streams
         n = int(n_filters or self.num_kf_runs)
         with self._batch(n, self._mc_x0(s.x0, n), s.u0[None], consistency) as bf:
-            kw = self._run_kwargs(s.cam_ref, s.imu_ref)
+            kw = self._run_kwargs(s.cam_ref, s.imu_ref, cam_dropout)
             E = len(s.n_prop)
             if segment_epochs and E:
                 k = int(segment_epochs)

@@ -177,10 +177,12 @@ int eskf_get_jacobians(eskf_t* h, double* Fx, double* Fi, int mem);
  *               of them): eps = dofs+ - gt_dofs after the update (rad / cm, the units of x[10:16]), B the block of error-state
  *               rows / columns 9..14 of the covariance after the update (Joseph form and reset), solved by LU with partial
  *               pivoting; d in expectation; NaN when d = 0.
- * Both are NaN where the update was not applied (ESKF_STATUS_* cases) and where the value is not finite.
+ * Both are NaN where the update was not applied (ESKF_STATUS_* cases) and where the value is not finite.  Where the
+ * measurement was dropped (eskf_set_meas_dropout) nis is NaN and nees is that of the PRIOR DOFs and DOF block (no update).
  * epoch_sum[e, 0:8] sums over the handle's filters, FINITE values only (a diverged filter is counted, never propagates):
  *   [0] number of finite NIS, [1] sum of NIS, [2] sum of NIS^2, [3] number of finite NEES, [4] sum, [5] sum of squares,
- *   [6] filters whose NIS, or NEES when d > 0, is NaN at e, [7] reserved (0).
+ *   [6] filters whose NIS is NaN although their measurement was not dropped, or whose NEES is NaN (d > 0), at e,
+ *   [7] filters whose measurement was dropped at e (0 without dropout).
  * Fixed reduction tree, no atomics: the same inputs give the same bits; plain sums, so shards combine by all-reduce.
  * eskf_get_consistency returns those of the LAST such run: nis, nees [N,E]; epoch_sum [E,ESKF_NCONS]; *n_epochs = E.
  * Any pointer may be NULL (query E first).  The run files the records through the export instantiation of the persistent
@@ -206,13 +208,14 @@ int eskf_get_consistency(eskf_t* h, double* nis, double* nees, double* epoch_sum
  *
  * eskf_get_dof_envelope: dof_sum [E,ESKF_NDOFSUM], per epoch sums over the handle's filters, computed by the call from the
  * records.  With eps_i = dofs_i - gt_dofs[i] (the gt_dofs of that run) and B the 6x6 DOF block of the record, filter f
- * CONTRIBUTES at epoch e when its nis is finite and, for every estimated DOF i (bit i of frozen_mask clear), eps_i and B_ii
+ * CONTRIBUTES at epoch e when its nis is finite or its measurement was dropped (its prior then) and, for every estimated DOF i (bit i of frozen_mask clear), eps_i and B_ii
  * are finite and B_ii > 0 and, for every pair of estimated DOFs, B_ij and B_ji are finite.  Row e:
  *   [0]  M, the contributing filters;  [1]  N - M, the excluded ones;
  *   [2 + 7 i .. 2 + 7 i + 6] for DOF i = 0..5: sum eps_i, sum eps_i^2, sum B_ii, sum eps_i^2 / B_ii, and the number of
  *        filters with eps_i^2 <= B_ii, eps_i^2 <= 4 B_ii, eps_i^2 <= 9 B_ii (compared as written: no square root);
  *   [44 .. 58] sum eps_i eps_j over the 15 pairs i < j, row-major (0,1), (0,2), ..., (4,5);
- *   [59 .. 73] sum (B_ij + B_ji) / 2 over the same pairs;   [74 .. 79] reserved (0).
+ *   [59 .. 73] sum (B_ij + B_ji) / 2 over the same pairs;   [74] filters whose measurement was dropped (eskf_set_meas_dropout);
+ *   [75 .. 79] reserved (0).
  * Sums over contributing filters only; entries of frozen DOFs, and of pairs that involve one, are 0.  Fixed reduction tree,
  * no atomics: the same records give the same bits.  Plain sums: shards combine them by all-reduce.  The run reserves the
  * row and its partial sums with the records (ESKF_ENOMEM before launch covers them). */
@@ -253,6 +256,26 @@ int eskf_set_groups(eskf_t* h, int64_t group_size);
 int eskf_get_group_sums(eskf_t* h, double* stats_sum, double* epoch_sum, double* dof_sum, int64_t* group0, int64_t* n_groups,
                         int64_t* n_epochs, int mem);
 
+/* Simulated frame loss (no reference counterpart): per-filter, per-epoch measurement dropout of eskf_run / eskf_run_epochs, drawn
+ * on the device.  prob [n_traj, n_epochs] in `mem` space (the whole trajectory's epochs, as the streams) is copied into the
+ * handle and applies to every later run until it is changed; NULL switches dropout off (the default).  Every entry must be
+ * finite and in [0, 1], else ESKF_EINVAL and the handle is unchanged; a device array is read back to check it (the call is
+ * synchronous).  A run returns ESKF_EINVAL, before anything is launched and with the handle unchanged, when (n_traj, n_epochs)
+ * differ from its streams' or with variant 1.  eskf_propagate / eskf_update ignore the setting.
+ * Rule: filter g (global id) with noise id gid (g % noise_id_modulus when the modulus is > 0, else g) loses the measurement of
+ * global epoch e iff u < prob[trajectory of g, e], u = (x + 1/2) 2^-32 in (0, 1) and x word 0 of Philox4x32-10(key = seed,
+ * counter = (e lo, 3 * 16 + (e hi << 8), gid lo, gid hi)) -- the layout of the noise draws with kind ESKF_NOISE_DROP
+ * (eskf_noise_dump reads u back).  prob = 0 never drops, prob = 1 always drops; with noise_free_filter0, noise id 0 makes no
+ * random drop and loses exactly the epochs with prob = 1.  Within one noise id the masks nest: prob1 <= prob2 drops a subset
+ * of the epochs prob2 drops.  The draw depends on neither noise std, and no other draw moves: segments, shards and
+ * noise_id_modulus see the masks of one whole run.
+ * A dropped measurement: the update is not applied (state and covariance stay at the prior; the trace row of the epoch's last
+ * step keeps the propagated state), no status bit is set and the residual is not evaluated; statistics row [9] does not count
+ * it; the update MSE of the epoch is evaluated as always, from the state at the frame instant.  Consistency: see
+ * eskf_get_consistency and eskf_get_dof_envelope (nis NaN, nees of the prior, epoch_sum[7] and dof_sum[74] the dropped count).
+ * A run with dropout runs the export instantiation of the persistent kernel. */
+int eskf_set_meas_dropout(eskf_t* h, const double* prob, int64_t n_traj, int64_t n_epochs, int mem);
+
 /* blocks until everything queued on the handle's stream has finished */
 int eskf_sync(eskf_t* h);
 
@@ -275,8 +298,9 @@ int eskf_set_variant(eskf_t* h, int variant);
  * out[n_filters][n_steps][8].  kind = ESKF_NOISE_IMU: z[0..5] scale om(3), acc(3) of IMU sample `step`;
  * kind = ESKF_NOISE_CAM: z[0..2] camera position, z[3..5] small body rotation of the measured quaternion,
  * z[6] notch angle of camera epoch `step`.  The generator uses the device's SFU approximations, so THIS is
- * the definition of the noise a run saw: parity tests feed these samples to the oracle. */
-enum { ESKF_NOISE_IMU = 1, ESKF_NOISE_CAM = 2 };
+ * the definition of the noise a run saw: parity tests feed these samples to the oracle.  kind = ESKF_NOISE_DROP: z[0] is the
+ * dropout uniform u of filter id `filter_id0 + f` and epoch `step` (eskf_set_meas_dropout), z[1..7] are 0. */
+enum { ESKF_NOISE_IMU = 1, ESKF_NOISE_CAM = 2, ESKF_NOISE_DROP = 3 };
 int eskf_noise_dump(int device, void* cuda_stream, uint64_t seed, int64_t filter_id0, int64_t n_filters, int64_t step0,
                     int64_t n_steps, int kind, double* out, int mem);
 
