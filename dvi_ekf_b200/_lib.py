@@ -25,7 +25,7 @@ EXPORTS = (
     "eskf_version", "eskf_fp64_peak", "eskf_set_variant", "eskf_noise_dump", "eskf_prepass", "eskf_prepass_last_error",
     "eskf_set_prepass_budget", "eskf_keep_jacobians", "eskf_get_jacobians", "eskf_keep_consistency", "eskf_get_consistency",
     "eskf_get_dof_history", "eskf_get_dof_envelope", "eskf_run_epochs", "eskf_set_groups", "eskf_get_group_sums",
-    "eskf_set_meas_dropout",
+    "eskf_set_meas_dropout", "eskf_set_meas_outliers", "eskf_set_innovation_gate",
 )
 
 
@@ -125,6 +125,8 @@ def load():
     lib.eskf_get_dof_envelope.argtypes = [vp, vp, C.POINTER(i64), i32]
     lib.eskf_set_groups.argtypes = [vp, i64]
     lib.eskf_set_meas_dropout.argtypes = [vp, vp, i64, i64, i32]
+    lib.eskf_set_meas_outliers.argtypes = [vp, vp, i64, i64, vp, i32]
+    lib.eskf_set_innovation_gate.argtypes = [vp, vp, i64, i32]
     lib.eskf_get_group_sums.argtypes = [vp, vp, vp, vp, C.POINTER(i64), C.POINTER(i64), C.POINTER(i64), i32]
     lib.eskf_fp64_peak.argtypes = [i32, vp, i32, C.POINTER(C.c_double), C.POINTER(C.c_double)]
     lib.eskf_noise_dump.argtypes = [i32, vp, C.c_uint64, i64, i64, i64, i64, i32, vp, i32]

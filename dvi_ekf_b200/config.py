@@ -97,9 +97,23 @@ class Config:
             seed=int(b.get("seed", 1234)), imu_noise=bool(b.get("imu_noise", True)), cam_noise=bool(b.get("cam_noise", True)),
             dof_ic_std_deg=float(b.get("dof_ic_std_deg", 3.0)), dof_ic_std_cm=float(b.get("dof_ic_std_cm", 3.0)),
             legacy_golden=bool(b.get("legacy_golden", False)), device=int(b.get("device", 0)),
-            cam_dropout=float(b.get("cam_dropout", 0.0)))  # probability that a Monte-Carlo filter loses a camera frame
+            cam_dropout=float(b.get("cam_dropout", 0.0)),  # probability that a Monte-Carlo filter loses a camera frame
+            # innovation gate: NIS threshold of every camera update (absent or null: no gate)
+            nis_gate=None if b.get("nis_gate") is None else float(b.get("nis_gate")),
+            # simulated outlier frames: probability per frame and the offsets' 7 standard deviations (units of meas_noise_std)
+            cam_outlier_prob=float(b.get("cam_outlier_prob", 0.0)),
+            cam_outlier_std=None if b.get("cam_outlier_std") is None else [float(v) for v in b.get("cam_outlier_std")])
         if not 0.0 <= self.batch.cam_dropout <= 1.0:
             raise ValueError(f"batch.cam_dropout must be a probability in [0, 1], not {self.batch.cam_dropout}")
+        if self.batch.nis_gate is not None and not self.batch.nis_gate >= 0.0:
+            raise ValueError(f"batch.nis_gate must be a NIS threshold >= 0 (or null for no gate), not {self.batch.nis_gate}")
+        if not 0.0 <= self.batch.cam_outlier_prob <= 1.0:
+            raise ValueError(f"batch.cam_outlier_prob must be a probability in [0, 1], not {self.batch.cam_outlier_prob}")
+        sd = self.batch.cam_outlier_std
+        if sd is not None and not (len(sd) == 7 and all(v >= 0.0 and v != float("inf") for v in sd)):
+            raise ValueError(f"batch.cam_outlier_std must be 7 finite values >= 0, not {sd}")
+        if self.batch.cam_outlier_prob > 0 and sd is None:
+            raise ValueError("batch.cam_outlier_prob > 0 requires batch.cam_outlier_std (7 values)")
 
     @property
     def dofs_updated(self) -> bool:

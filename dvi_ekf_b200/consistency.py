@@ -26,6 +26,16 @@ def _interval(count, dim, alpha):
     return np.stack([lo, hi], axis=1)
 
 
+def nis_gate_threshold(prob: float, dim: int = NIS_DIM) -> float:
+    """The chi-square innovation gate at confidence ``prob``: ``chi2.ppf(prob, dim)``, the NIS a consistent filter exceeds
+    with probability 1 - prob (``BatchFilter.run(nis_gate=...)``; dim = 7, the camera measurement)."""
+    from scipy.stats import chi2
+
+    if not 0.0 <= prob <= 1.0:
+        raise ValueError(f"prob must be in [0, 1], not {prob}")
+    return float(chi2.ppf(prob, dim))
+
+
 def summarise_consistency(epoch_sum, dim_dofs: int, alpha: float = 0.05) -> dict:
     """Summary of ``epoch_sum`` [E, 8] (one handle's, or the all-reduced sum of several shards'), ``dim_dofs`` the number of
     estimated DOFs d.  Returns a dict of numpy arrays / floats:
@@ -94,7 +104,8 @@ def summarise_dofs(dof_sum, frozen_dofs, alpha: float = 0.05) -> dict:
     - ``err_second_moment`` [E,6,6] = sum eps eps^T / M (the ensemble's error correlation, bias included) and
       ``filter_cov`` [E,6,6] = sum B / M (the filter's claimed one, symmetrised);
     - ``count`` [E] = M and ``excluded`` [E], the filters left out at the epoch; ``dropped`` [E], the filters whose measurement
-      was dropped (they contribute their prior).
+      was dropped (they contribute their prior); ``rejected`` [E], the filters whose update the innovation gate rejected
+      (``BatchFilter.run(nis_gate=...)``; they contribute their prior too).
     """
     from scipy.special import erf
     from scipy.stats import binom, chi2
@@ -113,7 +124,7 @@ def summarise_dofs(dof_sum, frozen_dofs, alpha: float = 0.05) -> dict:
     with np.errstate(invalid="ignore", divide="ignore"):
         var = np.where(m[:, None] >= 2, np.maximum(s2 - s1 * s1 / mm, 0.0) / np.maximum(mm - 1, 1.0), np.nan) * est
     sig = np.sqrt(sb / mm) * est
-    out = {"count": m, "excluded": s[:, 1].copy(), "dropped": s[:, 74].copy(), "bias": bias, "rmse": np.sqrt(msq), "std": np.sqrt(var), "sigma_filter": sig}
+    out = {"count": m, "excluded": s[:, 1].copy(), "dropped": s[:, 74].copy(), "rejected": s[:, 75].copy(), "bias": bias, "rmse": np.sqrt(msq), "std": np.sqrt(var), "sigma_filter": sig}
     with np.errstate(invalid="ignore", divide="ignore"):
         out["inflation"] = out["rmse"] / sig
     out["anees_dof"] = sr / mm * est

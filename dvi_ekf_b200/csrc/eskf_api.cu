@@ -71,17 +71,24 @@ __global__ void dfma_peak_kernel(double* out, int iters, double a, double b) {
 }
 
 // eskf_noise_dump: the standard normals of (filter, step, kind), exactly as the persistent kernels draw them; for
-// RNG_KIND_DROP the dropout uniform of (filter, epoch) in z[0] and zeros
+// RNG_KIND_DROP the dropout uniform of (filter, epoch) in z[0] and zeros; for RNG_KIND_OUTLIER the outlier uniform in z[0]
+// and the seven offset normals in z[1..7]
 __global__ void noise_dump_kernel(double* out, uint64_t seed, int64_t filter_id0, int64_t n_filters, int64_t step0, int64_t n_steps,
                                   uint32_t kind) {
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n_filters * n_steps) return;
   const int64_t f = i / n_steps, k = i - f * n_steps;
   double z[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-  if (kind == RNG_KIND_DROP)
+  if (kind == RNG_KIND_DROP) {
     z[0] = drop_uniform(seed, (uint64_t)(filter_id0 + f), (uint64_t)(step0 + k));
-  else
+  } else if (kind == RNG_KIND_OUTLIER) {
+    double w[8];
+    normal8(seed, (uint64_t)(filter_id0 + f), (uint64_t)(step0 + k), kind, w);
+    z[0] = outlier_uniform(seed, (uint64_t)(filter_id0 + f), (uint64_t)(step0 + k));
+    for (int j = 0; j < 7; ++j) z[1 + j] = w[j];
+  } else {
     normal8(seed, (uint64_t)(filter_id0 + f), (uint64_t)(step0 + k), kind, z);
+  }
   for (int j = 0; j < 8; ++j) out[i * 8 + j] = z[j];
 }
 
@@ -356,10 +363,13 @@ __global__ void stats_final_kernel(const double* __restrict__ partial, const Gro
 // cons_eval_kernel, one thread per (epoch, filter): NIS as filed, NEES of the estimated DOFs from the posterior DOFs and DOF
 // block (nees_dofs, eskf_math.cuh); NaN for an update that was not applied and for any non-finite value.  Writes the
 // filter-major outputs [N, E] and both values back into the record (CONS_NIS, CONS_NEES) for the epoch reduction.
+// An update rejected by the innovation gate keeps the NIS the gate compared and, like a dropped measurement, the NEES of
+// the prior.
 struct ConsArgs {
   int64_t N, E;
   double gt[6];
   int frozen_mask;
+  const double* gate;  // [N] the innovation-gate thresholds of the run that filed the records (a snapshot), or nullptr
 };
 __global__ void cons_eval_kernel(double* __restrict__ rec, double* __restrict__ nis, double* __restrict__ nees, const ConsArgs p) {
   const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -367,7 +377,8 @@ __global__ void cons_eval_kernel(double* __restrict__ rec, double* __restrict__ 
   const int64_t e = idx / p.N, f = idx - e * p.N;
   double* r = rec + e * CONS_SIZE * p.N + f;  // element j at r[j N]
   const double flag = r[CONS_NEES * p.N];
-  const bool applied = flag == 1.0, dropped = flag == 2.0;  // (a dropped measurement: the NEES of the prior)
+  // (a dropped measurement or a rejected update: the NEES of the prior)
+  const bool applied = flag == 1.0, dropped = flag == 2.0, rejected = flag == 3.0;
   double eps[6], B[36];
 #pragma unroll
   for (int i = 0; i < 6; ++i) eps[i] = r[(CONS_DOFS + i) * p.N] - p.gt[i];
@@ -375,8 +386,8 @@ __global__ void cons_eval_kernel(double* __restrict__ rec, double* __restrict__ 
   for (int i = 0; i < 36; ++i) B[i] = r[(CONS_B + i) * p.N];
   double vn = r[CONS_NIS * p.N];
   double ve = nees_dofs(B, eps, p.frozen_mask);
-  if (!applied || !isfinite(vn)) vn = NAN;
-  if (!(applied || dropped) || !isfinite(ve)) ve = NAN;
+  if (!rejected && (!applied || !isfinite(vn))) vn = NAN;
+  if (!(applied || dropped || rejected) || !isfinite(ve)) ve = NAN;
   nis[f * p.E + e] = vn;
   nees[f * p.E + e] = ve;
   r[CONS_NIS * p.N] = dropped ? -INFINITY : vn;  // (-inf marks the dropped ones for the reductions: a NIS is never infinite)
@@ -481,11 +492,13 @@ __global__ void __launch_bounds__(256) dof_history_kernel(const double* __restri
 // columns over the warp's rows in order, and the eight warps are added in order at the end.  cons_final_kernel adds the
 // blocks.
 // A dropped measurement (CONS_NIS = -inf, cons_eval_kernel) lets the filter contribute its prior and counts in column DSUM_DROP.
+// So does an update rejected by the innovation gate, in column DSUM_REJ: its NIS exceeds the threshold of the run that filed
+// the record (ConsArgs::gate, the kernel's own comparison of the same values), an applied update's does not.
 __global__ void __launch_bounds__(256) dof_partial_kernel(const double* __restrict__ rec, const ConsArgs p, const GroupMap m,
                                                           double* __restrict__ partial) {
-  constexpr int W = DSUM_DROP + 1;  // reduced columns
+  constexpr int W = DSUM_REJ + 1;  // reduced columns
   constexpr int NG = W / 32;  // full column groups; the tail W - 32 NG < 32 columns
-  static_assert(W - 32 * NG < 32 && DSUM_DROP >= DSUM_USED, "tail");
+  static_assert(W - 32 * NG < 32 && DSUM_DROP >= DSUM_USED && DSUM_REJ == DSUM_DROP + 1, "tail");
   __shared__ double sh[8][32 * (NG + 1)];
   const int64_t e = blockIdx.x / m.nblk, b = blockIdx.x - e * m.nblk;
   const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
@@ -509,6 +522,7 @@ __global__ void __launch_bounds__(256) dof_partial_kernel(const double* __restri
       const bool dr = vn == -INFINITY;
       dof_terms(dr ? 0.0 : vn, eps, re + CONS_B * p.N + r, p.N, p.frozen_mask, t);
       t[DSUM_DROP] = dr ? 1.0 : 0.0;
+      t[DSUM_REJ] = (p.gate && vn > p.gate[rb + r]) ? 1.0 : 0.0;
     }
     // (the tail first, then the groups from the last: fewer terms live at once)
 #pragma unroll
@@ -644,6 +658,16 @@ struct eskf_handle {
   double* drop_p = nullptr;
   size_t drop_sz = 0;
   int64_t drop_nt = 0, drop_E = 0;
+  // simulated outlier frames (eskf_set_meas_outliers): probabilities [out_nt][out_E] and offset std of every later run, on
+  // (out_nt > 0) or off
+  double* out_p = nullptr;
+  size_t out_sz = 0;
+  int64_t out_nt = 0, out_E = 0;
+  double out_std[7] = {0, 0, 0, 0, 0, 0, 0};
+  // innovation gate (eskf_set_innovation_gate): gate[0, N) the thresholds of every later run, on (gate_on) or off;
+  // gate[N, 2N) a snapshot of those the last run with consistency records used (ConsArgs::gate, read by the getters)
+  double* gate = nullptr;
+  bool gate_on = false;
 };
 
 #define CK(call)                                                  \
@@ -892,6 +916,8 @@ int eskf_destroy(eskf_t* h) {
   cudaFree(h->grp_stats);
   cudaFree(h->grp_buf);
   cudaFree(h->drop_p);
+  cudaFree(h->out_p);
+  cudaFree(h->gate);
   for (int i = 0; i < N_STAGE; ++i)
     if (h->stage[i]) cudaFree(h->stage[i]);
   delete h;
@@ -1096,6 +1122,22 @@ static int run_epochs(eskf_t* h, const eskf_streams_t* sp, int64_t e0, int64_t e
       return ESKF_EINVAL;
     }
   }
+  if (h->out_nt > 0) {
+    if (kernel_of(h) != 3) {
+      g_err = fn + ": simulated outlier frames need the default kernel (eskf_set_variant(h, 1) selects the first one)";
+      return ESKF_EINVAL;
+    }
+    if (h->out_nt != nt || h->out_E != E) {
+      g_err = fn + ": the outlier probabilities are [" + std::to_string((long long)h->out_nt) + ", " +
+              std::to_string((long long)h->out_E) + "], the streams [n_traj = " + std::to_string((long long)nt) +
+              ", n_epochs = " + std::to_string((long long)E) + "]";
+      return ESKF_EINVAL;
+    }
+  }
+  if (h->gate_on && kernel_of(h) != 3) {
+    g_err = fn + ": the innovation gate needs the default kernel (eskf_set_variant(h, 1) selects the first one)";
+    return ESKF_EINVAL;
+  }
   const size_t cb = (size_t)h->N * ESKF_NCARRY * sizeof(double);
   if (!whole && e0 == e1) {  // an empty range launches nothing: the carry passes through, the statistics are not written
     if (carry_out && carry_out != carry_in) {
@@ -1213,6 +1255,9 @@ static int run_epochs(eskf_t* h, const eskf_streams_t* sp, int64_t e0, int64_t e
   a.trace = dtrace;
   a.cons = (h->cons_on && E > 0) ? h->cons_rec : nullptr;
   a.drop_p = h->drop_nt > 0 ? h->drop_p : nullptr;
+  a.out_p = h->out_nt > 0 ? h->out_p : nullptr;
+  for (int i = 0; i < 7; ++i) a.out_std[i] = h->out_std[i];
+  a.nis_gate = h->gate_on ? h->gate : nullptr;
   a.seed = sp->seed;
   a.noise_free0 = sp->noise_free_filter0;
   a.noise_mod = sp->noise_id_modulus;
@@ -1335,6 +1380,11 @@ static int run_epochs(eskf_t* h, const eskf_streams_t* sp, int64_t e0, int64_t e
       ca.E = E;
       for (int i = 0; i < 6; ++i) ca.gt[i] = sp->gt_dofs[i];
       ca.frozen_mask = h->model.frozen_mask & 63;
+      ca.gate = nullptr;
+      if (h->gate_on) {  // (the getters answer from the thresholds this run compared, whatever is set later)
+        CK(cudaMemcpyAsync(h->gate + h->N, h->gate, (size_t)h->N * sizeof(double), cudaMemcpyDeviceToDevice, h->stream));
+        ca.gate = h->gate + h->N;
+      }
       const int64_t n2 = h->N * E;
       const GroupMap one = group_map(h->N, 0, 0);
       cons_eval_kernel<<<(unsigned)((n2 + 127) / 128), 128, 0, h->stream>>>(h->cons_rec, nis, nees, ca);
@@ -1432,7 +1482,7 @@ int eskf_fp64_peak(int device, void* cuda_stream, int repeats, double* tflops_ou
 int eskf_noise_dump(int device, void* cuda_stream, uint64_t seed, int64_t filter_id0, int64_t n_filters, int64_t step0,
                     int64_t n_steps, int kind, double* out, int mem) {
   if (!out || n_filters <= 0 || n_steps <= 0 ||
-      (kind != (int)RNG_KIND_IMU && kind != (int)RNG_KIND_CAM && kind != (int)RNG_KIND_DROP)) {
+      (kind != (int)RNG_KIND_IMU && kind != (int)RNG_KIND_CAM && kind != (int)RNG_KIND_DROP && kind != (int)RNG_KIND_OUTLIER)) {
     g_err = "eskf_noise_dump: bad argument";
     return ESKF_EINVAL;
   }
@@ -1493,6 +1543,101 @@ int eskf_set_meas_dropout(eskf_t* h, const double* prob, int64_t n_traj, int64_t
   }
   h->drop_nt = n_traj;
   h->drop_E = n_epochs;
+  return ESKF_OK;
+}
+
+int eskf_set_meas_outliers(eskf_t* h, const double* prob, int64_t n_traj, int64_t n_epochs, const double* std_, int mem) {
+  if (!h || (mem != ESKF_MEM_HOST && mem != ESKF_MEM_DEVICE)) {
+    g_err = "eskf_set_meas_outliers: bad argument";
+    return ESKF_EINVAL;
+  }
+  if (!prob) {
+    h->out_nt = h->out_E = 0;
+    return ESKF_OK;
+  }
+  if (n_traj < 1 || n_epochs < 0) {
+    g_err = "eskf_set_meas_outliers: n_traj must be positive and n_epochs non-negative";
+    return ESKF_EINVAL;
+  }
+  if (!std_) {
+    g_err = "eskf_set_meas_outliers: std (7 values) is required with a probability table";
+    return ESKF_EINVAL;
+  }
+  for (int i = 0; i < 7; ++i)
+    if (!(std_[i] >= 0.0 && std_[i] < INFINITY)) {  // (false for NaN)
+      g_err = "eskf_set_meas_outliers: std[" + std::to_string(i) + "] = " + std::to_string(std_[i]) +
+              " is not finite and non-negative";
+      return ESKF_EINVAL;
+    }
+  CK(cudaSetDevice(h->device));
+  const size_t n = (size_t)n_traj * (size_t)n_epochs, bytes = n * sizeof(double);
+  std::vector<double> hp;
+  const double* v = prob;
+  if (mem == ESKF_MEM_DEVICE && n > 0) {  // (read back to validate: a synchronous call, not a hot path)
+    hp.resize(n);
+    CK(cudaMemcpyAsync(hp.data(), prob, bytes, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    v = hp.data();
+  }
+  for (size_t i = 0; i < n; ++i)
+    if (!(v[i] >= 0.0 && v[i] <= 1.0)) {  // (false for NaN)
+      g_err = "eskf_set_meas_outliers: entry " + std::to_string((unsigned long long)i) + " = " + std::to_string(v[i]) +
+              " is not a probability in [0, 1]";
+      return ESKF_EINVAL;
+    }
+  int rc = grow(&h->out_p, &h->out_sz, bytes > 0 ? bytes : sizeof(double), "eskf_set_meas_outliers");
+  if (rc) return rc;
+  if (n > 0) {  // (from the validated host values; the source may go away on return)
+    CK(cudaMemcpyAsync(h->out_p, v, bytes, cudaMemcpyHostToDevice, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+  }
+  h->out_nt = n_traj;
+  h->out_E = n_epochs;
+  for (int i = 0; i < 7; ++i) h->out_std[i] = std_[i];
+  return ESKF_OK;
+}
+
+int eskf_set_innovation_gate(eskf_t* h, const double* nis_max, int64_t n, int mem) {
+  if (!h || (mem != ESKF_MEM_HOST && mem != ESKF_MEM_DEVICE)) {
+    g_err = "eskf_set_innovation_gate: bad argument";
+    return ESKF_EINVAL;
+  }
+  if (!nis_max) {
+    h->gate_on = false;
+    return ESKF_OK;
+  }
+  if (n != 1 && n != h->N) {
+    g_err = "eskf_set_innovation_gate: n must be 1 or n_filters";
+    return ESKF_EINVAL;
+  }
+  CK(cudaSetDevice(h->device));
+  std::vector<double> hv((size_t)n);
+  if (mem == ESKF_MEM_DEVICE) {  // (read back to validate: a synchronous call, not a hot path)
+    CK(cudaMemcpyAsync(hv.data(), nis_max, (size_t)n * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+  } else {
+    memcpy(hv.data(), nis_max, (size_t)n * sizeof(double));
+  }
+  for (int64_t i = 0; i < n; ++i)
+    if (!(hv[i] >= 0.0)) {  // (false for NaN; +inf passes: that filter is never gated)
+      g_err = "eskf_set_innovation_gate: entry " + std::to_string((long long)i) + " = " + std::to_string(hv[i]) +
+              " is not a threshold >= 0";
+      return ESKF_EINVAL;
+    }
+  if (n == 1) hv.assign((size_t)h->N, hv[0]);
+  if (!h->gate) {  // (thresholds and the snapshot of the last run's; allocated once, kept when the gate is switched off)
+    void* g = nullptr;
+    const cudaError_t err = cudaMalloc(&g, (size_t)h->N * 2 * sizeof(double));
+    if (err != cudaSuccess) {
+      cudaGetLastError();
+      g_err = std::string("eskf_set_innovation_gate: ") + cudaGetErrorString(err);
+      return err == cudaErrorMemoryAllocation ? ESKF_ENOMEM : ESKF_ECUDA;
+    }
+    h->gate = (double*)g;
+  }
+  CK(cudaMemcpyAsync(h->gate, hv.data(), (size_t)h->N * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+  CK(cudaStreamSynchronize(h->stream));
+  h->gate_on = true;
   return ESKF_OK;
 }
 

@@ -82,6 +82,12 @@ struct KArgs {
   // simulated frame loss (eskf_set_meas_dropout; eskf_kernel3 export instantiations only): [n_traj][E_all] (E_all = E outside a
   // segment) drop probabilities of every epoch, indexed like the per-epoch streams, or nullptr
   const double* drop_p;
+  // simulated outlier frames (eskf_set_meas_outliers; export instantiations only): [n_traj][E_all] outlier probabilities, laid
+  // out like drop_p, or nullptr, and the offsets' standard deviations (position 3, body rotation 3, notch 1)
+  const double* out_p;
+  double out_std[7];
+  // innovation gate (eskf_set_innovation_gate; export instantiations only): [N] NIS thresholds of the launch's filters, or nullptr
+  const double* nis_gate;
 };
 
 // one FilterTraj row's worth of nominal state in the layout of x (include/eskf.h)

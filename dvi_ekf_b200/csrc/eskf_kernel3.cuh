@@ -540,7 +540,7 @@ __device__ __forceinline__ void role3_imu(const KArgs& a, const Ctx3& c, int lan
     JIT();
     PT_MARK(3);
     if (act) {
-      if (sx[SX3_OK2 * F] != 0.0) {  // state (+) error state, IMU part (state.py:46-53,116-121)
+      if (EX ? sx[SX3_OK2 * F] > 0.0 : sx[SX3_OK2 * F] != 0.0) {  // state (+) error state, IMU part (state.py:46-53,116-121)
         const double th[3] = {sx[(SX3_DELTA + 6) * F], sx[(SX3_DELTA + 7) * F], sx[(SX3_DELTA + 8) * F]};
         double dq[4], qn[4];
         quat_about_axis(sqrt(th[0] * th[0] + th[1] * th[1] + th[2] * th[2]), th, dq);
@@ -771,7 +771,9 @@ __device__ __forceinline__ void role3_cam(const KArgs& a, const Ctx3& c, int lan
     PT_MARK(3);
     PT_MARK(3);
     if (act) {
-      if (sx[SX3_OK2 * F] != 0.0) {  // camera part of the injection, incl. the dqc axis slip (quirk Q4, state.py:124)
+      // (SX3_OK2 = -1 in export mode: rejected by the innovation gate -- not applied, and like a dropped measurement not a
+      // skipped update)
+      if (EX ? sx[SX3_OK2 * F] > 0.0 : sx[SX3_OK2 * F] != 0.0) {  // camera part of the injection, incl. the dqc axis slip (quirk Q4, state.py:124)
         const double th[3] = {sx[(SX3_DELTA + 6) * F], sx[(SX3_DELTA + 7) * F], sx[(SX3_DELTA + 8) * F]};
         const double thc[3] = {sx[(SX3_DELTA + 21) * F], sx[(SX3_DELTA + 22) * F], sx[(SX3_DELTA + 23) * F]};
         double dqc[4], qn[4];
@@ -783,7 +785,7 @@ __device__ __forceinline__ void role3_cam(const KArgs& a, const Ctx3& c, int lan
         for (int i = 0; i < 4; ++i) qc[i] = qn[i];
         n_upd += 1.0;
         if (EX && a.trace && k0_of<SG>(c) + k > 0) trace_cam(a.trace + ((c.f0 + lane) * a.T + k0_of<SG>(c) + k - 1) * NX, pc, qc);
-      } else if (!EX || sx[SX3_OK * F] >= 0.0) {  // (a dropped measurement is not a skipped update)
+      } else if (!EX || (sx[SX3_OK * F] >= 0.0 && sx[SX3_OK2 * F] == 0.0)) {  // (a dropped measurement is not a skipped update)
         st |= ESKF_STATUS_UPDATE_SKIPPED;
       }
 #if ESKF_OPT_PP
@@ -992,7 +994,7 @@ __device__ __forceinline__ void role3_jac(const KArgs& a, const Ctx3& c, int lan
     JIT();
     PT_MARK(3);
     if (act) {
-      if (sx[SX3_OK2 * F] != 0.0) {
+      if (EX ? sx[SX3_OK2 * F] > 0.0 : sx[SX3_OK2 * F] != 0.0) {  // (-1: rejected by the innovation gate, export mode)
 #pragma unroll
         for (int i = 0; i < 6; ++i)
           if (!((a.model.frozen_mask >> i) & 1)) dofs[i] += sx[(SX3_DELTA + 9 + i) * F];  // Filter.py:377-379
@@ -1159,39 +1161,60 @@ __device__ __forceinline__ void role3_stage(const KArgs& a, const Ctx3& c, int l
 #endif
   };
   auto stage_meas = [&](int64_t e) {
-    if (EX && a.drop_p)  // simulated frame loss: SX3_OK = -1 marks the epoch's measurement as dropped
-      sx[SX3_OK * F] = meas_dropped(a.drop_p[erow3<SG>(a, c, e)], a.seed, (uint64_t)gid, (uint64_t)((SG ? a.e_base : 0) + e),
-                                    a.noise_free0 && gid == 0) ? -1.0 : 0.0;
+    bool drop = false;
+    if (EX && a.drop_p) {  // simulated frame loss: SX3_OK = -1 marks the epoch's measurement as dropped
+      drop = meas_dropped(a.drop_p[erow3<SG>(a, c, e)], a.seed, (uint64_t)gid, (uint64_t)((SG ? a.e_base : 0) + e),
+                          a.noise_free0 && gid == 0);
+      sx[SX3_OK * F] = drop ? -1.0 : 0.0;
+    }
+    // simulated outlier frames: decided after the dropout (a dropped frame is not corrupted) and applied below to the
+    // measurement as staged, noise included, on both statistics paths alike
+    const bool outl = EX && a.out_p && !drop;
+    double cam[7], notch;
 #if ESKF_OPT_PP
     if (a.meas_pf) {
       const double* m = a.meas_pf + (e * a.N + c.f0 + lane) * 8;
+      if (!outl) {
 #pragma unroll
-      for (int i = 0; i < 8; ++i) sx[(SX3_MEAS + i) * F] = m[i];
-      return;
-    }
-#endif
-    const int64_t mrow = a.meas_per_filter ? (c.f0 + lane) : erow3<SG>(a, c, e);
-    double cam[7];
-#pragma unroll
-    for (int i = 0; i < 7; ++i) cam[i] = a.cam[mrow * 7 + i];
-    double notch = a.notch[mrow];
-    if (noisy) {
-      double z[8];
-      normal8(a.seed, (uint64_t)gid, (uint64_t)((SG ? a.e_base : 0) + e), RNG_KIND_CAM, z);
-      double dth[3];
-#pragma unroll
-      for (int i = 0; i < 3; ++i) {
-        cam[i] += a.cam_noise[i] * z[i];
-        dth[i] = a.cam_noise[3 + i] * z[3 + i];
+        for (int i = 0; i < 8; ++i) sx[(SX3_MEAS + i) * F] = m[i];
+        return;
       }
-      // orientation noise: small body rotation of the measured quaternion (its norm is kept)
-      double dq[4], qn[4];
-      quat_about_axis(sqrt(dth[0] * dth[0] + dth[1] * dth[1] + dth[2] * dth[2]), dth, dq);
-      const double nq = sqrt(cam[3] * cam[3] + cam[4] * cam[4] + cam[5] * cam[5] + cam[6] * cam[6]);
-      quat_mul(cam + 3, dq, qn);
 #pragma unroll
-      for (int i = 0; i < 4; ++i) cam[3 + i] = qn[i] * nq;
-      notch += a.cam_noise[6] * z[6];
+      for (int i = 0; i < 7; ++i) cam[i] = m[i];
+      notch = m[7];
+    } else
+#endif
+    {
+      const int64_t mrow = a.meas_per_filter ? (c.f0 + lane) : erow3<SG>(a, c, e);
+#pragma unroll
+      for (int i = 0; i < 7; ++i) cam[i] = a.cam[mrow * 7 + i];
+      notch = a.notch[mrow];
+      if (noisy) {
+        double z[8];
+        normal8(a.seed, (uint64_t)gid, (uint64_t)((SG ? a.e_base : 0) + e), RNG_KIND_CAM, z);
+        double dth[3];
+#pragma unroll
+        for (int i = 0; i < 3; ++i) {
+          cam[i] += a.cam_noise[i] * z[i];
+          dth[i] = a.cam_noise[3 + i] * z[3 + i];
+        }
+        // orientation noise: small body rotation of the measured quaternion (its norm is kept)
+        double dq[4], qn[4];
+        quat_about_axis(sqrt(dth[0] * dth[0] + dth[1] * dth[1] + dth[2] * dth[2]), dth, dq);
+        const double nq = sqrt(cam[3] * cam[3] + cam[4] * cam[4] + cam[5] * cam[5] + cam[6] * cam[6]);
+        quat_mul(cam + 3, dq, qn);
+#pragma unroll
+        for (int i = 0; i < 4; ++i) cam[3 + i] = qn[i] * nq;
+        notch += a.cam_noise[6] * z[6];
+      }
+    }
+    if (outl) {
+      const uint64_t ge = (uint64_t)((SG ? a.e_base : 0) + e);
+      if (meas_outlier(a.out_p[erow3<SG>(a, c, e)], a.seed, (uint64_t)gid, ge, a.noise_free0 && gid == 0)) {
+        double z[8];
+        normal8(a.seed, (uint64_t)gid, ge, RNG_KIND_OUTLIER, z);
+        cam_offset(cam, notch, a.out_std, z);
+      }
     }
 #pragma unroll
     for (int i = 0; i < 7; ++i) sx[(SX3_MEAS + i) * F] = cam[i];
@@ -1663,16 +1686,22 @@ __device__ __forceinline__ void role3_cov(const KArgs& a, const Ctx3& c, int ct)
     JIT();
     PT_MARK(6);
     // (SX3_OK: 1 valid residual, 0 none, -1 a measurement dropped by eskf_set_meas_dropout, export mode only)
-    const bool upd_c = inv_ok && (EX ? sxc[SX3_OK * F] > 0.0 : sxc[SX3_OK * F] != 0.0);
-    double nis = NAN;  // (export mode: consistency record)
-    if (upd_c) {
+    const bool ok_c = inv_ok && (EX ? sxc[SX3_OK * F] > 0.0 : sxc[SX3_OK * F] != 0.0);
+    double nis = NAN;  // (export mode: consistency record, innovation gate)
+    bool rej = false;  // (export mode: rejected by the innovation gate, eskf_set_innovation_gate)
+    if (ok_c) {
       double K[3][7], res[7], dl[3];
 #pragma unroll
       for (int m = 0; m < 7; ++m) res[m] = sxc[(SX3_RES + m) * F];
       upd3_gain<4>(cg, rec, res, K, dl);
       if constexpr (EX) {
-        if (a.cons && cg == 0) nis = upd3_nis<4>(rec, res);
+        // every lane of the filter evaluates the NIS from the shared record (same inputs, same bits) and so takes the gate's
+        // decision itself; a NaN NIS is never rejected.  (Evaluated after the gain, which a rejected update discards: before
+        // it the NIS cost the export instantiations up to 500 bytes of spills.)
+        if (a.cons || a.nis_gate) nis = upd3_nis<4>(rec, res);
+        rej = a.nis_gate && nis > a.nis_gate[c.f0 + cf];
       }
+      // (the scalar roles read the increments only when SX3_OK2 > 0)
 #pragma unroll
       for (int v = 0; v < 3; ++v) sxw[(SX3_DELTA + 3 * cg + v) * F] = dl[v];
       if (a.K_out && cf < c.nf) {
@@ -1682,12 +1711,15 @@ __device__ __forceinline__ void role3_cov(const KArgs& a, const Ctx3& c, int ct)
           for (int m = 0; m < 7; ++m) a.K_out[((c.f0 + cf) * 24 + 3 * cg + v) * 7 + m] = K[v][m];
       }
     }
-    if (cg == 0) sxw[SX3_OK2 * F] = upd_c ? 1.0 : 0.0;
+    const bool upd_c = ok_c && !rej;
+    // (SX3_OK2: 1 applied, 0 not applied, -1 rejected by the innovation gate, export mode only)
+    if (cg == 0) sxw[SX3_OK2 * F] = upd_c ? 1.0 : rej ? -1.0 : 0.0;
     if constexpr (EX) {
       if (a.cons && cg == 0 && cf < c.nf) {
         double* r = a.cons + e * CONS_SIZE * a.N + c.f0 + cf;
-        r[CONS_NIS * a.N] = nis;
-        r[CONS_NEES * a.N] = upd_c ? 1.0 : sxc[SX3_OK * F] < 0.0 ? 2.0 : 0.0;  // applied / not applied / dropped
+        r[CONS_NIS * a.N] = nis;  // (a rejected update keeps the NIS the gate compared)
+        // applied / not applied / dropped / rejected
+        r[CONS_NEES * a.N] = upd_c ? 1.0 : rej ? 3.0 : sxc[SX3_OK * F] < 0.0 ? 2.0 : 0.0;
       }
     }
     PT_MARK(7);

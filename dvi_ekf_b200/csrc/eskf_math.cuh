@@ -213,6 +213,25 @@ ESKF_HD void quat_about_axis(double angle, const double* axis, double* q) {
   quat_normalise(q);
 }
 
+// Offset of a camera measurement cam = (p 3, raw q 4) and its notch by the normals z[0..6] scaled by sd[7], as the camera
+// noise is applied: p += sd z, a small body rotation of q by sd[3..5] z[3..5] that keeps the raw quaternion's norm, and
+// notch += sd[6] z[6].  (Simulated outlier frames, eskf_set_meas_outliers.)
+ESKF_HD void cam_offset(double* cam, double& notch, const double* sd, const double* z) {
+  double dth[3];
+#pragma unroll
+  for (int i = 0; i < 3; ++i) {
+    cam[i] += sd[i] * z[i];
+    dth[i] = sd[3 + i] * z[3 + i];
+  }
+  double dq[4], qn[4];
+  quat_about_axis(sqrt(dth[0] * dth[0] + dth[1] * dth[1] + dth[2] * dth[2]), dth, dq);
+  const double nq = sqrt(cam[3] * cam[3] + cam[4] * cam[4] + cam[5] * cam[5] + cam[6] * cam[6]);
+  quat_mul(cam + 3, dq, qn);
+#pragma unroll
+  for (int i = 0; i < 4; ++i) cam[3 + i] = qn[i] * nq;
+  notch += sd[6] * z[6];
+}
+
 // ---- probe kinematics -----------------------------------------------------------
 // Closed form of the 8-joint DH chain (Probe.py:147-167) with q8 = 0:
 //   triad  e_a(t) = (s1 s2 st - c1 ct,  s1 ct + c1 s2 st,  c2 st)
@@ -1267,10 +1286,11 @@ ESKF_HD void group_block(int64_t b, int64_t N, int64_t id0, int64_t g, int64_t r
 // Record of one (epoch e, filter f), element-major so that the filters of a warp store and the post-pass reads coalesced:
 // element j at cons[(e * CONS_SIZE + j) * N + f].  The export instantiation of eskf_kernel3 files it, cons_eval_kernel
 // (eskf_api.cu) turns it into the NIS / NEES outputs.
-constexpr int CONS_NIS = 0;    // r^T inv(S) r of the update, NaN if it was not applied (covariance lane 0)
+constexpr int CONS_NIS = 0;    // r^T inv(S) r of the update, NaN if it was not applied and not rejected (covariance lane 0)
 constexpr int CONS_DOFS = 1;   // 6: dofs after the update (JACOB role)
 constexpr int CONS_NEES = 7;   // kernel: 1 if the update was applied, 2 if its measurement was dropped (eskf_set_meas_dropout),
-                               // else 0; cons_eval_kernel overwrites it with the NEES (and CONS_NIS of a dropped one with -inf)
+                               // 3 if the innovation gate rejected it (eskf_set_innovation_gate), else 0; cons_eval_kernel
+                               // overwrites it with the NEES (and CONS_NIS of a dropped one with -inf)
 constexpr int CONS_B = 8;      // 36: covariance block of error-state rows / columns 9..14 after the update, as the tile holds
                                // it (the transpose of the reference's, which a quadratic form does not see; lanes 3 and 4)
 constexpr int CONS_SIZE = 44;  // doubles
@@ -1328,7 +1348,8 @@ constexpr int DSUM_DOF = 2;    // 7 per DOF i at DSUM_DOF + 7 i: eps, eps^2, B_i
 constexpr int DSUM_EE = 44;    // 15: eps_i eps_j, pairs i < j row-major (0,1), (0,2), ..., (4,5)
 constexpr int DSUM_BB = 59;    // 15: (B_ij + B_ji) / 2, the same pairs
 constexpr int DSUM_USED = 74;  // the terms of dof_terms
-constexpr int DSUM_DROP = 74;  // filters whose measurement was dropped (dof_partial_kernel); the rest of the row is reserved (0)
+constexpr int DSUM_DROP = 74;  // filters whose measurement was dropped (dof_partial_kernel)
+constexpr int DSUM_REJ = 75;   // filters whose update the innovation gate rejected (dof_partial_kernel); the rest is reserved (0)
 
 // The terms of one record for that row, t[0 .. DSUM_USED - 1]: nis as cons_eval_kernel left it, eps = dofs - gt_dofs,
 // B the 6x6 DOF block (row-major, element (i, j) at B[(6 i + j) ld]: ld = N reads it in place from a record).  The filter

@@ -134,4 +134,26 @@ ESKF_HD bool meas_dropped(double p, uint64_t seed, uint64_t id, uint64_t epoch, 
   return nf0 ? p == 1.0 : drop_uniform(seed, id, epoch) < p;
 }
 
+// ---- simulated outlier frames (eskf_set_meas_outliers, include/eskf.h) ----
+// One uniform and one set of offsets per (noise id, GLOBAL epoch), kind RNG_KIND_OUTLIER: the offsets are normal8 (draws 0
+// and 1), u = unit_open32 of word 0 of draw 2 with drop_uniform's counter layout.  Like the dropout draw it depends on
+// nothing but (seed, id, epoch): segments, shards and noise_id_modulus see the outliers of one whole-batch run, and no other
+// kind's draw moves.  eskf_noise_dump(kind = ESKF_NOISE_OUTLIER) reads u and the offsets back.
+constexpr uint32_t RNG_KIND_OUTLIER = 4;
+
+ESKF_HD double outlier_uniform(uint64_t seed, uint64_t id, uint64_t epoch) {
+  uint32_t c[4] = {(uint32_t)epoch, RNG_KIND_OUTLIER * 16u + 2u + ((uint32_t)(epoch >> 32) << 8), (uint32_t)id,
+                   (uint32_t)(id >> 32)};
+  philox4x32_10(c, (uint32_t)seed, (uint32_t)(seed >> 32));
+  return unit_open32(c[0]);
+}
+
+// The measurement of epoch `epoch` is an outlier for noise id `id` iff u < p: p = 0 never, p = 1 always.  The masks nest over
+// p and the offsets do not depend on p, so a sweep over p corrupts a superset with the same offsets.  A noise-free reference
+// filter (nf0) is never corrupted.
+ESKF_HD bool meas_outlier(double p, uint64_t seed, uint64_t id, uint64_t epoch, bool nf0) {
+  if (nf0 || !(p > 0.0)) return false;
+  return outlier_uniform(seed, id, epoch) < p;
+}
+
 }  // namespace eskf

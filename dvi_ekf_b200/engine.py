@@ -96,18 +96,19 @@ def check_run_geometry(n_filters: int, n_traj: int, filters_per_traj: int, filte
             raise ValueError(f"sum(n_prop) = {int(tot.max())} exceeds n_steps = {n_steps}")
 
 
-def drop_prob_array(prob, n_traj: int, n_epochs: int) -> np.ndarray:
+def drop_prob_array(prob, n_traj: int, n_epochs: int, name: str = "drop_prob") -> np.ndarray:
     """The drop probabilities of ``BatchFilter.run(drop_prob=...)`` as the C-contiguous float64 [n_traj, n_epochs] array
     eskf_set_meas_dropout takes: ``prob`` is a scalar, [n_epochs] (every trajectory) or [n_traj, n_epochs], every entry
-    finite and in [0, 1].  Raises ``ValueError`` otherwise."""
+    finite and in [0, 1].  Raises ``ValueError`` otherwise.  (The outlier probabilities of eskf_set_meas_outliers are
+    checked the same way; ``name`` names the argument in the message.)"""
     p = np.asarray(prob, dtype=np.float64)
     if p.ndim > 2 or (p.ndim >= 1 and p.shape[-1] != n_epochs) or (p.ndim == 2 and p.shape[0] != n_traj):
-        raise ValueError(f"drop_prob must be a scalar, [{n_epochs}] or [{n_traj}, {n_epochs}] (n_traj, n_epochs of the streams), "
+        raise ValueError(f"{name} must be a scalar, [{n_epochs}] or [{n_traj}, {n_epochs}] (n_traj, n_epochs of the streams), "
                          f"not of shape {p.shape}")
     if not np.isfinite(p).all():
-        raise ValueError("drop_prob must be finite (NaN or infinite entry)")
+        raise ValueError(f"{name} must be finite (NaN or infinite entry)")
     if (p < 0).any() or (p > 1).any():
-        raise ValueError(f"drop_prob entries are probabilities in [0, 1], not {float(p.min())} .. {float(p.max())}")
+        raise ValueError(f"{name} entries are probabilities in [0, 1], not {float(p.min())} .. {float(p.max())}")
     return np.ascontiguousarray(np.broadcast_to(p, (n_traj, n_epochs)))
 
 
@@ -120,6 +121,30 @@ def mask_from_uniforms(u, p, noise_free) -> np.ndarray:
     nf = np.asarray(noise_free, dtype=bool)
     m[nf] = p[nf] == 1.0
     return m
+
+
+def outlier_std_array(std) -> np.ndarray:
+    """The offset standard deviations of eskf_set_meas_outliers: 7 finite values >= 0 (position 3, small body rotation 3,
+    notch 1, in the units of cam_noise_std) as a float64 array.  Raises ``ValueError`` otherwise."""
+    if std is None:
+        raise ValueError("outlier_std (7 values) is required with outlier probabilities")
+    s = np.asarray(std, dtype=np.float64)
+    if s.shape != (7,):
+        raise ValueError(f"outlier_std must have 7 entries (position 3, rotation 3, notch 1), not shape {s.shape}")
+    if not (np.isfinite(s).all() and (s >= 0).all()):
+        raise ValueError(f"outlier_std entries must be finite and >= 0, not {s.tolist()}")
+    return np.ascontiguousarray(s)
+
+
+def nis_gate_array(thr, n: int) -> np.ndarray:
+    """The thresholds of eskf_set_innovation_gate: a scalar (every filter) or [n] (one per filter), each >= 0 and not NaN
+    (+inf: never gated), as a C-contiguous float64 array of 1 or n entries.  Raises ``ValueError`` otherwise."""
+    t = np.asarray(thr, dtype=np.float64)
+    if t.ndim > 1 or (t.ndim == 1 and t.shape[0] not in (1, n)):
+        raise ValueError(f"nis_gate must be a scalar or [{n}] (one threshold per filter), not of shape {t.shape}")
+    if np.isnan(t).any() or (t < 0).any():
+        raise ValueError("nis_gate thresholds must be >= 0 and not NaN (+inf switches a filter's gate off)")
+    return np.ascontiguousarray(t.reshape(-1))
 
 
 def segment_steps(n_prop, n_steps: int, e0: int, e1: int):
@@ -257,7 +282,8 @@ class BatchFilter:
     def run(self, dt, om_acc, n_prop, cam, notch, cam_ref=None, imu_ref=None, gt_dofs=(0, 0, 0, 0, 0, 20.0),
             n_traj: int = 1, filters_per_traj: Optional[int] = None, seed: int = 0, filter_id0: int = 0,
             imu_noise_std=None, cam_noise_std=None, noise_free_filter0: bool = True, want_stats: bool = True,
-            stats_on_device: bool = False, trace=None, noise_id_modulus: int = 0, epochs=None, carry=None, drop_prob=None):
+            stats_on_device: bool = False, trace=None, noise_id_modulus: int = 0, epochs=None, carry=None, drop_prob=None,
+            nis_gate=None, outlier_prob=None, outlier_std=None):
         """``Filter.run`` (Filter.py:144-185) for every filter, in one persistent kernel.
         Returns (stats [N,16], stats_sum [16]) (see include/eskf.h) or None.
         ``trace``: optional [N,T,26] float64 array (numpy for host streams, CUDA tensor for device streams) that
@@ -271,7 +297,10 @@ class BatchFilter:
         do (numpy, or CUDA tensors with ``stats_on_device``), and the returned one is also kept as ``last_carry``.  Segments
         run back to back give bit for bit what one run gives; a checkpoint is ``get_state()``, the carry and e1.
         ``drop_prob``: simulated frame loss (``set_meas_dropout``): a scalar, [E] or [n_traj, E] (numpy, or a CUDA tensor) of
-        per-epoch probabilities that a filter loses the camera measurement; None runs without dropout."""
+        per-epoch probabilities that a filter loses the camera measurement; None runs without dropout.
+        ``nis_gate``: the innovation gate (``set_innovation_gate``): a scalar or [N] NIS threshold; an update whose NIS exceeds
+        it is rejected.  ``outlier_prob`` / ``outlier_std``: simulated outlier frames (``set_meas_outliers``): a scalar, [E] or
+        [n_traj, E] of per-epoch probabilities and the 7 offset standard deviations.  None runs without either."""
         adt = _Arg(dt, None, name="dt")
         anp = _Arg(n_prop, None, dtype=np.int32, name="n_prop")
         T = adt.rows // n_traj
@@ -304,6 +333,8 @@ class BatchFilter:
                 raise ValueError("trace must live where the streams live (host numpy / CUDA tensor)")
             s.trace_x = atr.ptr
         self.set_meas_dropout(drop_prob, n_traj, E)
+        self.set_innovation_gate(nis_gate)
+        self.set_meas_outliers(outlier_prob, outlier_std, n_traj, E)
         if epochs is not None:
             return self._run_epochs(s, int(epochs[0]), int(epochs[1]), carry, want_stats, stats_on_device)
         if not want_stats:
@@ -384,6 +415,52 @@ class BatchFilter:
         p = drop_prob_array(prob.numpy() if _is_torch(prob) else prob, n_traj, n_epochs)
         check(self._lib.eskf_set_meas_dropout(self._h, p.ctypes.data_as(C.c_void_p), n_traj, n_epochs, MEM_HOST),
               "eskf_set_meas_dropout")
+
+    def set_innovation_gate(self, thr):
+        """Innovation gate of every later ``run`` (eskf_set_innovation_gate, include/eskf.h): an update whose residual is
+        valid and whose NIS r^T inv(S) r exceeds the filter's threshold is rejected (state and covariance stay at the
+        prior, no status bit).  ``thr``: a scalar or [N] (numpy, or a CUDA tensor), each >= 0 and not NaN, +inf never
+        gates; None switches the gate off."""
+        if thr is None:
+            check(self._lib.eskf_set_innovation_gate(self._h, None, 0, MEM_HOST), "eskf_set_innovation_gate")
+            return
+        if _is_torch(thr) and thr.is_cuda:
+            import torch
+
+            nis_gate_array(thr.detach().cpu().numpy(), self.n)  # (the shape and value checks, on a host copy)
+            t = thr.to(torch.float64).reshape(-1).contiguous()
+            check(self._lib.eskf_set_innovation_gate(self._h, C.c_void_p(t.data_ptr()), int(t.numel()), MEM_DEVICE),
+                  "eskf_set_innovation_gate")
+            return
+        t = nis_gate_array(thr.numpy() if _is_torch(thr) else thr, self.n)
+        check(self._lib.eskf_set_innovation_gate(self._h, t.ctypes.data_as(C.c_void_p), int(t.size), MEM_HOST),
+              "eskf_set_innovation_gate")
+
+    def set_meas_outliers(self, prob, std=None, n_traj: int = 1, n_epochs: Optional[int] = None):
+        """Simulated outlier frames of every later ``run`` (eskf_set_meas_outliers, include/eskf.h): filter g's camera
+        measurement of epoch e is offset with probability prob[trajectory, e] by std * z (z standard normals drawn on the
+        device from the run's seed and the filter's noise id; ``outlier_mask`` gives the mask).  ``prob`` as for
+        ``set_meas_dropout``; ``std`` 7 values >= 0 (position 3, small body rotation 3, notch 1); None switches it off."""
+        if prob is None:
+            check(self._lib.eskf_set_meas_outliers(self._h, None, 0, 0, None, MEM_HOST), "eskf_set_meas_outliers")
+            return
+        sd = outlier_std_array(std)
+        if n_epochs is None:
+            if np.ndim(prob) == 0:
+                raise ValueError("n_epochs is needed for a scalar probability")
+            n_epochs = int(prob.shape[-1]) if _is_torch(prob) else np.shape(prob)[-1]
+        sdp = sd.ctypes.data_as(C.c_void_p)
+        if _is_torch(prob) and prob.is_cuda:
+            import torch
+
+            drop_prob_array(prob.detach().cpu().numpy(), n_traj, n_epochs, "outlier_prob")  # (the checks, on a host copy)
+            t = torch.broadcast_to(prob.to(torch.float64), (n_traj, n_epochs)).contiguous()
+            check(self._lib.eskf_set_meas_outliers(self._h, C.c_void_p(t.data_ptr()), n_traj, n_epochs, sdp, MEM_DEVICE),
+                  "eskf_set_meas_outliers")
+            return
+        p = drop_prob_array(prob.numpy() if _is_torch(prob) else prob, n_traj, n_epochs, "outlier_prob")
+        check(self._lib.eskf_set_meas_outliers(self._h, p.ctypes.data_as(C.c_void_p), n_traj, n_epochs, sdp, MEM_HOST),
+              "eskf_set_meas_outliers")
 
     def sync(self):
         check(self._lib.eskf_sync(self._h), "eskf_sync")
@@ -517,7 +594,7 @@ class BatchFilter:
         check(self._lib.eskf_set_variant(self._h, int(variant)), "eskf_set_variant")
 
 
-NOISE_IMU, NOISE_CAM, NOISE_DROP = 1, 2, 3
+NOISE_IMU, NOISE_CAM, NOISE_DROP, NOISE_OUTLIER = 1, 2, 3, 4
 
 
 def noise_samples(seed: int, filter_id0: int, n_filters: int, step0: int, n_steps: int, kind: int, device: int = 0):
@@ -547,6 +624,30 @@ def dropout_mask(prob, seed: int, filter_id0: int, n_filters: int, epochs, n_tra
     lo = int(gid.min())
     u = noise_samples(seed, lo, int(gid.max()) - lo + 1, e0, e1 - e0, NOISE_DROP, device)[:, :, 0]
     return mask_from_uniforms(u[gid - lo], p[traj, e0:e1], (gid == 0) & bool(noise_free_filter0))
+
+
+def outlier_mask(prob, seed: int, filter_id0: int, n_filters: int, epochs, n_traj: int = 1, filters_per_traj: Optional[int] = None,
+                 noise_id_modulus: int = 0, noise_free_filter0: bool = True, device: int = 0):
+    """(mask bool [n_filters, e1 - e0], offsets [n_filters, e1 - e0, 7]): which of global epochs ``epochs = (e0, e1)`` of
+    filters ``filter_id0 ..`` are outliers in a run with ``outlier_prob = prob`` (a scalar, [E] or [n_traj, E]) and these run
+    arguments, and the standard normals of their offsets (scale them by ``outlier_std``), from the draws of the device
+    (``eskf_noise_dump`` with ESKF_NOISE_OUTLIER: the definition).  The noise-free reference filter is never corrupted."""
+    e0, e1 = (int(v) for v in epochs)
+    E = int(np.shape(prob)[-1]) if np.ndim(prob) else e1
+    p = drop_prob_array(prob, n_traj, E, "outlier_prob")
+    if not 0 <= e0 <= e1 <= E:
+        raise ValueError(f"epochs [{e0}, {e1}) is not within [0, {E}]")
+    g = int(filter_id0) + np.arange(int(n_filters))
+    traj = g // int(filters_per_traj or n_filters) if n_traj > 1 else np.zeros_like(g)
+    gid = g % noise_id_modulus if noise_id_modulus > 0 else g
+    if e1 == e0:
+        return np.zeros((len(g), 0), dtype=bool), np.zeros((len(g), 0, 7))
+    lo = int(gid.min())
+    d = noise_samples(seed, lo, int(gid.max()) - lo + 1, e0, e1 - e0, NOISE_OUTLIER, device)[gid - lo]
+    nf = (gid == 0) & bool(noise_free_filter0)
+    m = mask_from_uniforms(d[:, :, 0], p[traj, e0:e1], np.zeros(len(g), dtype=bool))
+    m[nf] = False  # (unlike a dropout, the noise-free reference filter is never corrupted, even at p = 1)
+    return m, d[:, :, 1:8]
 
 
 def fp64_peak_tflops(device: int = 0, repeats: int = 5) -> float:

@@ -17,7 +17,7 @@ from . import rotations as rot
 from .camera import Camera, Streams, build_streams, load_notch, load_trajectory
 from .config import Config
 from .consistency import NIS_DIM, candidate_objective, summarise_consistency, summarise_dofs
-from .engine import BatchFilter
+from .engine import BatchFilter, outlier_std_array
 from .probe import GT_IMU_DOFS
 from .sharding import summarise_stats
 
@@ -419,7 +419,7 @@ class Simulator:
             # r noise realisations, so candidates differ only by their parameters
             st, _ = bf.run(s.dt, s.om_acc, s.n_prop, s.cam, s.notch, cam_ref=s.cam_ref, imu_ref=s.imu_ref,
                            gt_dofs=cfg.gt_imu_dofs, seed=b.seed, imu_noise_std=imu_std, cam_noise_std=cam_std,
-                           noise_free_filter0=True, noise_id_modulus=r, **self._dropout_kwargs())
+                           noise_free_filter0=True, noise_id_modulus=r, **self._dropout_kwargs(), **self._gate_kwargs())
             if metric in ("nis", "nees"):
                 nis, nees, _ = bf.get_consistency()
                 return candidate_objective(nis if metric == "nis" else nees, m, NIS_DIM if metric == "nis" else dim_dofs)
@@ -492,13 +492,30 @@ class Simulator:
             raise ValueError(f"cam_dropout must be a probability in [0, 1], not {p}")
         return {"drop_prob": p} if p > 0 else {}
 
-    def _run_kwargs(self, cam_ref, imu_ref, cam_dropout: Optional[float] = None) -> dict:
+    def _gate_kwargs(self, nis_gate: Optional[float] = None, cam_outliers=None) -> dict:
+        """``nis_gate`` / ``outlier_prob`` / ``outlier_std`` of BatchFilter.run for the innovation gate ``nis_gate`` (None:
+        ``batch.nis_gate``) and the simulated outlier frames ``cam_outliers = (prob, std)`` (None: ``batch.cam_outlier_prob``
+        / ``batch.cam_outlier_std``); nothing for no gate and p = 0, so that such a run keeps the production kernel"""
+        b = self.config.batch
+        thr = b.nis_gate if nis_gate is None else float(nis_gate)
+        p, sd = (b.cam_outlier_prob, b.cam_outlier_std) if cam_outliers is None else (float(cam_outliers[0]), cam_outliers[1])
+        if thr is not None and not thr >= 0.0:
+            raise ValueError(f"nis_gate must be a NIS threshold >= 0, not {thr}")
+        if not 0.0 <= p <= 1.0:
+            raise ValueError(f"the outlier probability must be in [0, 1], not {p}")
+        kw = {} if thr is None else {"nis_gate": thr}
+        if p > 0:
+            kw.update(outlier_prob=p, outlier_std=outlier_std_array(sd))
+        return kw
+
+    def _run_kwargs(self, cam_ref, imu_ref, cam_dropout: Optional[float] = None, nis_gate: Optional[float] = None,
+                    cam_outliers=None) -> dict:
         """the keyword arguments of BatchFilter.run for a Monte-Carlo run (``batch:`` section)"""
         cfg, b = self.config, self.config.batch
         imu_std = np.hstack((cfg.imu.stdev_omega, cfg.imu.stdev_accel)) if b.imu_noise else None
         cam_std = np.array(cfg.meas_noise_std) if b.cam_noise else None
         return dict(cam_ref=cam_ref, imu_ref=imu_ref, gt_dofs=cfg.gt_imu_dofs, seed=b.seed, imu_noise_std=imu_std,
-                    cam_noise_std=cam_std, **self._dropout_kwargs(cam_dropout))
+                    cam_noise_std=cam_std, **self._dropout_kwargs(cam_dropout), **self._gate_kwargs(nis_gate, cam_outliers))
 
     def _stacked_trajectories(self, names, n_filters: int, frames: Optional[int] = None, consistency: bool = False):
         """(BatchFilter, run keyword arguments) of the stacked launch of ``run_trajectories``: the named trajectories built as
@@ -554,7 +571,8 @@ class Simulator:
         return res
 
     def run(self, disp_config=False, save_best=False, verbose=True, n_filters: Optional[int] = None, consistency: bool = False,
-            segment_epochs: Optional[int] = None, cam_dropout: Optional[float] = None):
+            segment_epochs: Optional[int] = None, cam_dropout: Optional[float] = None, nis_gate: Optional[float] = None,
+            cam_outliers=None):
         """Simulator.run (Simulator.py:121-158) as ONE batched launch: ``num_kf_runs`` (or ``n_filters``)
         independent filters, run 0 noise free (the reference's deterministic run), the others with
         Monte-Carlo IMU / camera noise and DOF initial-condition perturbations (``batch:`` section).
@@ -564,11 +582,15 @@ class Simulator:
         ``segment_epochs`` k: the same run in launches of k epochs (``BatchFilter.run_segments``), with the same results; the
         consistency records then take the memory of k epochs, not of the whole run, and their per-epoch rows are joined.
         ``cam_dropout``: the probability that a filter loses a camera frame (``BatchFilter.run(drop_prob=...)``; run 0, the
-        noise-free one, loses none); None takes ``batch.cam_dropout`` (default 0: no frame loss)."""
+        noise-free one, loses none); None takes ``batch.cam_dropout`` (default 0: no frame loss).
+        ``nis_gate``: the NIS threshold of the innovation gate (``BatchFilter.run(nis_gate=...)``); None takes
+        ``batch.nis_gate`` (default: no gate).  ``cam_outliers = (prob, std)``: simulated outlier frames
+        (``BatchFilter.run(outlier_prob=prob, outlier_std=std)``; run 0 gets none); None takes ``batch.cam_outlier_prob`` /
+        ``batch.cam_outlier_std`` (default p = 0: none)."""
         cfg, s = self.config, self.streams
         n = int(n_filters or self.num_kf_runs)
         with self._batch(n, self._mc_x0(s.x0, n), s.u0[None], consistency) as bf:
-            kw = self._run_kwargs(s.cam_ref, s.imu_ref, cam_dropout)
+            kw = self._run_kwargs(s.cam_ref, s.imu_ref, cam_dropout, nis_gate, cam_outliers)
             E = len(s.n_prop)
             if segment_epochs and E:
                 k = int(segment_epochs)

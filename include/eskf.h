@@ -177,8 +177,10 @@ int eskf_get_jacobians(eskf_t* h, double* Fx, double* Fi, int mem);
  *               of them): eps = dofs+ - gt_dofs after the update (rad / cm, the units of x[10:16]), B the block of error-state
  *               rows / columns 9..14 of the covariance after the update (Joseph form and reset), solved by LU with partial
  *               pivoting; d in expectation; NaN when d = 0.
- * Both are NaN where the update was not applied (ESKF_STATUS_* cases) and where the value is not finite.  Where the
- * measurement was dropped (eskf_set_meas_dropout) nis is NaN and nees is that of the PRIOR DOFs and DOF block (no update).
+ * Both are NaN where the update was not applied (ESKF_STATUS_* cases) and where the value is not finite, except for an
+ * update the innovation gate rejected (eskf_set_innovation_gate): its nis is the NIS the gate compared and its nees that of
+ * the PRIOR DOFs and DOF block.  Where the measurement was dropped (eskf_set_meas_dropout) nis is NaN and nees is that of
+ * the PRIOR too (no update).  epoch_sum[0..5] include the rejected updates' NIS and prior NEES.
  * epoch_sum[e, 0:8] sums over the handle's filters, FINITE values only (a diverged filter is counted, never propagates):
  *   [0] number of finite NIS, [1] sum of NIS, [2] sum of NIS^2, [3] number of finite NEES, [4] sum, [5] sum of squares,
  *   [6] filters whose NIS is NaN although their measurement was not dropped, or whose NEES is NaN (d > 0), at e,
@@ -208,14 +210,16 @@ int eskf_get_consistency(eskf_t* h, double* nis, double* nees, double* epoch_sum
  *
  * eskf_get_dof_envelope: dof_sum [E,ESKF_NDOFSUM], per epoch sums over the handle's filters, computed by the call from the
  * records.  With eps_i = dofs_i - gt_dofs[i] (the gt_dofs of that run) and B the 6x6 DOF block of the record, filter f
- * CONTRIBUTES at epoch e when its nis is finite or its measurement was dropped (its prior then) and, for every estimated DOF i (bit i of frozen_mask clear), eps_i and B_ii
+ * CONTRIBUTES at epoch e when its nis is finite or its measurement was dropped (its prior then; so does a filter whose update
+ * the innovation gate rejected) and, for every estimated DOF i (bit i of frozen_mask clear), eps_i and B_ii
  * are finite and B_ii > 0 and, for every pair of estimated DOFs, B_ij and B_ji are finite.  Row e:
  *   [0]  M, the contributing filters;  [1]  N - M, the excluded ones;
  *   [2 + 7 i .. 2 + 7 i + 6] for DOF i = 0..5: sum eps_i, sum eps_i^2, sum B_ii, sum eps_i^2 / B_ii, and the number of
  *        filters with eps_i^2 <= B_ii, eps_i^2 <= 4 B_ii, eps_i^2 <= 9 B_ii (compared as written: no square root);
  *   [44 .. 58] sum eps_i eps_j over the 15 pairs i < j, row-major (0,1), (0,2), ..., (4,5);
  *   [59 .. 73] sum (B_ij + B_ji) / 2 over the same pairs;   [74] filters whose measurement was dropped (eskf_set_meas_dropout);
- *   [75 .. 79] reserved (0).
+ *   [75] filters whose update the innovation gate rejected (eskf_set_innovation_gate; the thresholds of the run that filed
+ *   the records, whatever is set later);   [76 .. 79] reserved (0).
  * Sums over contributing filters only; entries of frozen DOFs, and of pairs that involve one, are 0.  Fixed reduction tree,
  * no atomics: the same records give the same bits.  Plain sums: shards combine them by all-reduce.  The run reserves the
  * row and its partial sums with the records (ESKF_ENOMEM before launch covers them). */
@@ -276,6 +280,37 @@ int eskf_get_group_sums(eskf_t* h, double* stats_sum, double* epoch_sum, double*
  * A run with dropout runs the export instantiation of the persistent kernel. */
 int eskf_set_meas_dropout(eskf_t* h, const double* prob, int64_t n_traj, int64_t n_epochs, int mem);
 
+/* Simulated outlier frames (no reference counterpart): per-filter, per-epoch gross errors of the camera measurement of
+ * eskf_run / eskf_run_epochs, drawn on the device -- relocalisation jumps, tracking snapped to a wrong keyframe.  prob
+ * [n_traj, n_epochs] in `mem` space follows the rules of eskf_set_meas_dropout's table (validated, copied, every later run,
+ * NULL = off, the default; a run with other (n_traj, n_epochs) or with variant 1 is ESKF_EINVAL before launch, handle
+ * unchanged; eskf_propagate / eskf_update ignore it).  std[7] (host memory): the offsets' standard deviations, position (3),
+ * small body rotation (3), notch (1), in the units of cam_noise_std; each finite and >= 0, else ESKF_EINVAL.
+ * Rule: filter g with noise id gid (as for the dropout) has an outlier at global epoch e iff u < prob[trajectory of g, e],
+ * u = (x + 1/2) 2^-32 and x word 0 of Philox4x32-10(key = seed, counter = (e lo, 4 * 16 + 2 + (e hi << 8), gid lo, gid hi));
+ * its offsets are z[0..6] of the normals of kind 4 (the layout of ESKF_NOISE_CAM with kind 4: eskf_noise_dump(kind =
+ * ESKF_NOISE_OUTLIER) reads u and z back).  The offset is added to the measurement as staged, after the camera noise:
+ * position += std[i] z[i]; the quaternion turned by the body rotation std[3 + i] z[3 + i], its norm kept, as the camera
+ * noise does; notch += std[6] z[6].  With noise_free_filter0, noise id 0 is never corrupted, even at prob = 1.  The masks
+ * nest over prob and the offsets do not depend on it.  A dropped frame (eskf_set_meas_dropout decides first) is not
+ * corrupted.  No other draw moves: segments, shards and noise_id_modulus see the outliers of one whole run.  A run with
+ * outliers runs the export instantiation of the persistent kernel. */
+int eskf_set_meas_outliers(eskf_t* h, const double* prob, int64_t n_traj, int64_t n_epochs, const double* std, int mem);
+
+/* Innovation gate (no reference counterpart; Filter.update applies every update whose S it can invert): a chi-square gate in
+ * front of the camera update of eskf_run / eskf_run_epochs.  nis_max in `mem` space: n = 1 threshold for every filter or
+ * n = N, one per filter (as eskf_set_noise; a shard passes its slice); every entry >= 0 and not NaN (+inf: that filter is
+ * never gated), else ESKF_EINVAL and the handle is unchanged.  It applies to every later run until changed; NULL switches it
+ * off (the default).  A run with the gate and variant 1 is ESKF_EINVAL before launch; eskf_propagate / eskf_update ignore it.
+ * Rule: an update whose residual is valid and whose S inverted is REJECTED iff nis > nis_max[f], nis = r^T inv(S) r as
+ * eskf_get_consistency reports it; a NaN nis is never rejected.  A rejected update leaves state and covariance at the prior
+ * (the trace row keeps the propagated state), sets NO status bit (the filter is healthy and stays in stats_sum) and is not
+ * counted in statistics row [9]; the update MSE of the epoch is evaluated as always.  So, for a filter with status 0, the
+ * number of rejected updates = epochs run - dropped frames - row [9]; the per-epoch mask is nis > nis_max on
+ * eskf_get_consistency's output.  Consistency: see eskf_get_consistency and eskf_get_dof_envelope (nis the compared value,
+ * nees of the prior, dof_sum[75] the rejected count).  A run with the gate runs the export instantiation. */
+int eskf_set_innovation_gate(eskf_t* h, const double* nis_max, int64_t n, int mem);
+
 /* blocks until everything queued on the handle's stream has finished */
 int eskf_sync(eskf_t* h);
 
@@ -299,8 +334,9 @@ int eskf_set_variant(eskf_t* h, int variant);
  * kind = ESKF_NOISE_CAM: z[0..2] camera position, z[3..5] small body rotation of the measured quaternion,
  * z[6] notch angle of camera epoch `step`.  The generator uses the device's SFU approximations, so THIS is
  * the definition of the noise a run saw: parity tests feed these samples to the oracle.  kind = ESKF_NOISE_DROP: z[0] is the
- * dropout uniform u of filter id `filter_id0 + f` and epoch `step` (eskf_set_meas_dropout), z[1..7] are 0. */
-enum { ESKF_NOISE_IMU = 1, ESKF_NOISE_CAM = 2, ESKF_NOISE_DROP = 3 };
+ * dropout uniform u of filter id `filter_id0 + f` and epoch `step` (eskf_set_meas_dropout), z[1..7] are 0.
+ * kind = ESKF_NOISE_OUTLIER: z[0] is the outlier uniform u, z[1..7] the seven offset normals (eskf_set_meas_outliers). */
+enum { ESKF_NOISE_IMU = 1, ESKF_NOISE_CAM = 2, ESKF_NOISE_DROP = 3, ESKF_NOISE_OUTLIER = 4 };
 int eskf_noise_dump(int device, void* cuda_stream, uint64_t seed, int64_t filter_id0, int64_t n_filters, int64_t step0,
                     int64_t n_steps, int kind, double* out, int mem);
 
