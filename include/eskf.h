@@ -43,8 +43,10 @@ enum { ESKF_FLAG_ZERO_FROZEN = 1 /* HEAD behaviour, Filter.py:243-245 */ };
 
 /* per-filter status bits (eskf_get_state) */
 enum {
-  ESKF_STATUS_UPDATE_SKIPPED = 1, /* singular / non-finite S: the LinAlgError branch, Filter.py:356-361 */
-  ESKF_STATUS_ASIN_DOMAIN = 2     /* |v| > 1 in Quaternion.angle (math.asin would raise) */
+  ESKF_STATUS_UPDATE_SKIPPED = 1, /* an update was not applied: singular / non-finite S (the LinAlgError branch,
+                                   * Filter.py:356-361) or a residual outside the domain of asin (then with bit 2) */
+  ESKF_STATUS_ASIN_DOMAIN = 2     /* |v| > 1 in Quaternion.angle (math.asin would raise): the update is skipped, so the word
+                                   * reads 3; state and P keep the prior and the gain read back is 0 */
 };
 
 typedef struct {

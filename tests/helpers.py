@@ -22,6 +22,7 @@ from oracle.eskf_oracle import (
     camera_from_arrays,
     camera_gen_rotated,
     quat_normalise,
+    quat_to_matrix,
 )
 
 GOLDEN_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
@@ -104,6 +105,99 @@ def mandala_scenario(golden, n_frames=10, ifv=1, with_notch=False, **cfg_kw):
     cfg = OracleConfig(max_vals=n_frames, interframe_vals=ifv, **cfg_kw)
     notch = golden["notch_notch90"][:n_frames] if with_notch else None
     return Scenario(golden["traj_mandala0_mono"][:n_frames], cfg, notch=notch)
+
+
+def markley_branch(M):
+    """The branch quat_from_matrix (scipy-1.10.1 from_matrix) takes for M: 0, 1, 2 (largest diagonal entry) or 3 (trace)."""
+    dec = [M[0, 0], M[1, 1], M[2, 2], M[0, 0] + M[1, 1] + M[2, 2]]
+    choice = 0
+    for n in range(1, 4):
+        if dec[n] > dec[choice]:
+            choice = n
+    return choice
+
+
+def cube_rotations():
+    """The 24 proper rotations of the cube: signed permutation matrices with determinant +1."""
+    out = []
+    for perm in ((0, 1, 2), (0, 2, 1), (1, 0, 2), (1, 2, 0), (2, 0, 1), (2, 1, 0)):
+        for signs in np.ndindex(2, 2, 2):
+            G = np.zeros((3, 3))
+            for r in range(3):
+                G[r, perm[r]] = -1.0 if signs[r] else 1.0
+            if np.linalg.det(G) > 0:
+                out.append(G)
+    assert len(out) == 24
+    return out
+
+
+def _axis_angle(axis, deg):
+    from scipy.spatial.transform import Rotation
+
+    axis = np.asarray(axis, dtype=float)
+    return Rotation.from_rotvec(np.deg2rad(deg) * axis / np.linalg.norm(axis)).as_matrix()
+
+
+def world_rotations(sc):
+    """The constant world rotations G the rotated scenarios use, by name: the identity (control); 60 deg about -x (the IMU
+    quaternion starts at exactly 180 deg from the identity and crosses w = 0), 150 deg about y and about z (the IMU and camera
+    quaternions on Markley branches 1 and 2); the 24 rotations of the cube; 8 seeded random rotations; and one that puts the
+    camera's roll 0.4 deg short of 180 deg at the middle frame of ``sc``, so the Euler wrap falls inside the run."""
+    from scipy.spatial.transform import Rotation
+
+    out = {"identity": np.eye(3), "x-60": _axis_angle([-1, 0, 0], 60.0), "y150": _axis_angle([0, 1, 0], 150.0),
+           "z150": _axis_angle([0, 0, 1], 150.0)}
+    for i, G in enumerate(cube_rotations()):
+        out[f"cube{i:02d}"] = G
+    for i, G in enumerate(Rotation.random(8, random_state=20261022).as_matrix()):
+        out[f"random{i}"] = G
+    mid = len(sc.cam_meas) // 2
+    Rc = quat_to_matrix(sc.cam_meas[mid, 3:])
+    out["roll-wrap"] = Rotation.from_euler("xyz", [179.6, 25.0, -40.0], degrees=True).as_matrix() @ Rc.T
+    return out
+
+
+class RotatedScenario:
+    """``sc`` in a world turned by the constant rotation G.  The model has no gravity term (oracle/eskf_oracle.py:280), so
+    the body-frame IMU samples, dt and n_prop of ``sc`` stay valid: p, v, p_cam turn by G, q and q_cam become g * q (g the
+    quaternion of G), every camera measurement becomes (G p, g * q_raw with the raw quaternion's norm kept).  The update-MSE
+    references are recomputed from the turned camera measurements and IMU-reference rows with the oracle's Euler function:
+    cam_ref [E,6] = (G p, xyz Euler angles of g * q_raw), imu_ref [E,6] = (G v, xyz Euler angles of g * q_ref) at each epoch's
+    last IMU instant.  The result is not the unrotated run turned by G (Markley's method on the non-orthonormal matrices
+    of the propagation, quirk Q1, breaks the equivariance at 1e-4): the engine is compared with the oracle on THESE inputs."""
+
+    def __init__(self, sc: Scenario, G, name=""):
+        from scipy.spatial.transform import Rotation
+
+        from oracle.eskf_oracle import euler_xyz_deg, quat_mul
+
+        self.name, self.G, self.base = name, np.asarray(G, dtype=float), sc
+        self.g = g = Rotation.from_matrix(self.G).as_quat()
+        self.cfg, self.probe = sc.cfg, sc.probe
+        self.dt, self.om_acc, self.n_prop, self.notch_meas, self.u0 = sc.dt, sc.om_acc, sc.n_prop, sc.notch_meas, sc.u0
+        self.P0, self.Qd, self.Rd, self.sig_om = sc.P0, sc.Qd, sc.Rd, sc.sig_om
+        x = sc.x0.copy()
+        for s in (0, 3, 19):
+            x[s:s + 3] = self.G @ sc.x0[s:s + 3]
+        x[6:10] = quat_mul(g, sc.x0[6:10])
+        x[22:26] = quat_mul(g, sc.x0[22:26])
+        self.x0 = x
+        cam = sc.cam_meas.copy()
+        cam[:, :3] = sc.cam_meas[:, :3] @ self.G.T
+        for e in range(len(cam)):
+            cam[e, 3:] = quat_mul(g, sc.cam_meas[e, 3:]) * np.linalg.norm(sc.cam_meas[e, 3:])
+        self.cam_meas = cam
+        self.cam_ref = np.hstack((cam[:, :3], euler_xyz_deg(cam[:, 3:])))
+        ends = np.cumsum(sc.n_prop) - 1
+        rows = sc.imu_ref_rows[np.maximum(ends, 0)]
+        q_ref = np.array([quat_mul(g, r[[11, 12, 13, 10]]) for r in rows])
+        self.imu_ref = np.hstack((rows[:, 4:7] @ self.G.T, euler_xyz_deg(q_ref)))
+
+    def new_oracle(self, x0=None, cls=None):
+        from oracle.eskf_oracle import OracleFilter
+
+        x = State.from_vector(self.x0 if x0 is None else x0)
+        return (cls or OracleFilter)(self.cfg, x, self.P0, self.u0[:3], self.u0[3:], self.probe)
 
 
 def random_filter_inputs(rng, n, cfg: OracleConfig, frozen=False):
